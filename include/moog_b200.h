@@ -126,6 +126,14 @@ int moog_overlap_pairs(moog_program *p, const moog_state *st, int n_envs, int la
  * frames[N][H][W][3] uint8, row 0 = top. */
 int moog_render(moog_program *p, const moog_state *st, int n_envs, uint8_t *frames, void *stream);
 
+/* RawState.__call__ (moog/observers/raw_state.py:17-19) for N envs: every sprite slot's state as
+ * out[N][S][MOOG_OBS_COLS] float32 (layout and columns: moog_b200_program.h MOOG_OBS_*).  A launch of its
+ * own on `stream`, so call it after moog_env_step to observe the state that call left.  `out` is any
+ * device-accessible address aligned to 16 bytes: HBM, or pinned host memory as for moog_step_io.frames.
+ * MOOG_E_INVAL for a NULL program / state / out, n_envs < 0 or a misaligned out; n_envs == 0 launches
+ * nothing. */
+int moog_observe_sprites(moog_program *p, const moog_state *st, int n_envs, float *out, void *stream);
+
 /* Host-side (CPU) polygon predicates for the HOST Sprite class only: the state
  * initializer's rejection sampling calls Sprite.overlaps_sprite /
  * contains_points (moog/state_initialization/sprite_generators.py:69-105,

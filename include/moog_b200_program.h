@@ -343,6 +343,30 @@ enum {
 };
 #define MOOG_MAX_META 8
 
+/* Sprite observation (RawState, raw_state.py:17-19), written by moog_observe_sprites:
+ * float32 out[N][S][MOOG_OBS_COLS], slots in record order -- layers in state order, the sprites of a
+ * layer in list order (z-order); layer l owns slots [layer_off[l], layer_off[l+1]) and its first
+ * cnt[n][l] are live.  Columns 0-13 follow Sprite.FACTOR_NAMES (sprite.py:237-241) without metadata;
+ * every value is the record's double rounded to nearest float32 (NaN stays NaN, inf stays inf).  A slot
+ * that holds no sprite reads 0 in every column but MOOG_OBS_LAYER, whatever the record keeps there. */
+#define MOOG_OBS_X 0          /* dyn  MOOG_D_X      */
+#define MOOG_OBS_Y 1          /* dyn  MOOG_D_Y      */
+#define MOOG_OBS_SHAPE 2      /* meta MOOG_M_SHAPE: shape id (BatchedEnvironment.shape_names) */
+#define MOOG_OBS_ANGLE 3      /* dyn  MOOG_D_ANG    */
+#define MOOG_OBS_SCALE 4      /* stat MOOG_S_SCALE  */
+#define MOOG_OBS_ASPECT 5     /* stat MOOG_S_ASPECT */
+#define MOOG_OBS_C0 6         /* stat MOOG_S_C0     */
+#define MOOG_OBS_C1 7         /* stat MOOG_S_C1     */
+#define MOOG_OBS_C2 8         /* stat MOOG_S_C2     */
+#define MOOG_OBS_OPACITY 9    /* stat MOOG_S_OPACITY */
+#define MOOG_OBS_X_VEL 10     /* dyn  MOOG_D_VX     */
+#define MOOG_OBS_Y_VEL 11     /* dyn  MOOG_D_VY     */
+#define MOOG_OBS_ANGLE_VEL 12 /* dyn  MOOG_D_ANGVEL */
+#define MOOG_OBS_MASS 13      /* stat MOOG_S_MASS (inf stays inf) */
+#define MOOG_OBS_LAYER 14     /* layer index of the slot, live or not */
+#define MOOG_OBS_ALIVE 15     /* 1 for a live slot, 0 otherwise */
+#define MOOG_OBS_COLS 16
+
 /* step_type values written by the kernels (dm_env.StepType) */
 enum { MOOG_STEP_FIRST = 0, MOOG_STEP_MID = 1, MOOG_STEP_LAST = 2 };
 

@@ -9,6 +9,8 @@ num_envs=N)` works on an unchanged MOOG config -- and the same `reset()` /
     reward      float32[N]   NaN on FIRST steps            (dm_env: None)
     discount    float32[N]   1 mid, 0 last, NaN first
     observation {'image': uint8 [N, H, W, 3]}              (PILRenderer)
+                {key: float32 [N, S, 16]}                 (RawState: every sprite slot, see
+                                                           include/moog_b200_program.h MOOG_OBS_*)
 
 An env whose previous step returned LAST is reset by the next `step()` call and
 ignores that call's action (environment.py:100-101).  Initial states come from
@@ -152,6 +154,9 @@ class Engine(object):
             r = program.render
             self.frames = torch.zeros((self.n, r['height'], r['width'], 3),
                                       dtype=torch.uint8, device=self.device)
+        self.sprites = None
+        if getattr(program, 'state_key', None) is not None:
+            self.sprites = torch.zeros((self.n, program.n_slots, compiler.OBS_COLS), **f32)
         self._calls = 0
         self._pinned_ok = set()
 
@@ -169,6 +174,16 @@ class Engine(object):
 
     def _stream(self):
         return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _check_reachable(self, out, what):
+        """`out` is on this device or in pinned host memory (the kernels store into it)."""
+        if out.device.type == 'cpu':
+            if out.data_ptr() not in self._pinned_ok:
+                if not out.is_pinned():
+                    raise ValueError('host {} must live in pinned memory'.format(what))
+                self._pinned_ok.add(out.data_ptr())
+        elif out.device != self.state.dyn.device:
+            raise ValueError('{} are on {}, the envs on {}'.format(what, out.device, self.state.dyn.device))
 
     def set_pool(self, arrays):
         n = arrays['dyn'].shape[0]
@@ -208,13 +223,7 @@ class Engine(object):
                     or not frames.is_contiguous()):
                 raise ValueError('frames must be a contiguous uint8 tensor of shape {}'.format(
                     tuple(self.frames.shape)))
-            if frames.device.type == 'cpu':
-                if frames.data_ptr() not in self._pinned_ok:
-                    if not frames.is_pinned():
-                        raise ValueError('host frames must live in pinned memory')
-                    self._pinned_ok.add(frames.data_ptr())
-            elif frames.device != self.state.dyn.device:
-                raise ValueError('frames are on {}, the envs on {}'.format(frames.device, self.state.dyn.device))
+            self._check_reachable(frames, 'frames')
         act = self._as_f64(actions, max(p.action_dim, 1)) if actions is not None else None
         nz = self._as_f64(noise, p.K * p.noise_dim) if (noise is not None and p.noise_dim) else None
         rn = self._as_f64(rule_noise, p.rule_noise_dim) if (
@@ -276,6 +285,25 @@ class Engine(object):
                 self.dev_program.handle, ctypes.byref(st), count, dst, self._stream()))
         return out
 
+    def observe_sprites(self, out=None):
+        """`moog_observe_sprites`: RawState (raw_state.py:17-19) of every env as float32 [N, S, 16]
+        (columns: include/moog_b200_program.h MOOG_OBS_*), into `self.sprites` or `out` -- a
+        contiguous tensor of that shape on this device, or in pinned host memory, which the kernel
+        then writes over PCIe.  Enqueued on the current stream behind whatever was enqueued before."""
+        if out is None:
+            if self.sprites is None:
+                raise capi.MoogError('the program has no RawState observer')
+            out = self.sprites
+        shape = (self.n, self.program.n_slots, compiler.OBS_COLS)
+        if out.dtype != torch.float32 or tuple(out.shape) != shape or not out.is_contiguous():
+            raise ValueError('sprites must be a contiguous float32 tensor of shape {}'.format(shape))
+        self._check_reachable(out, 'sprites')
+        st = self.state.struct()
+        with self._on_device():
+            capi.check(capi.lib().moog_observe_sprites(
+                self.dev_program.handle, ctypes.byref(st), self.n, _ptr(out), self._stream()))
+        return out
+
 
 class BatchedEnvironment(object):
     """See module docstring.  Reference: moog/environment.py:28-131."""
@@ -311,6 +339,7 @@ class BatchedEnvironment(object):
         for k, obs in (observers or {}).items():
             if type(obs).__name__ == 'PILRenderer':
                 self._image_key = k
+        self._state_key = self.program.state_key
         self._rng = np.random.RandomState(seed)
         self._started = False
         self._copy_stream = None
@@ -366,11 +395,20 @@ class BatchedEnvironment(object):
                              frames=True if self._image_key is not None else None)
         return self._timestep(rendered=True)
 
+    def shape_names(self):
+        """Shape name of every shape id (meta row 0, column 2 of the RawState observation); an id beyond
+        the list is a shape without a name."""
+        table = self._pool_arrays.get('shape_table')
+        return list(getattr(table, 'names', [])) if table is not None else []
+
     def step_to_host(self, action, host, chunks=4, frames='auto'):
         """`step(action)` whose TimeStep lands in the caller's pinned host buffers:
         `host` is a TimeStep of CPU tensors (step_type int32[N], reward float32[N],
-        discount float32[N] or None, observation {'image': uint8[N,H,W,3]}).  Returns
-        `host` once everything has arrived (the caller owns the TimeStep).
+        discount float32[N] or None, observation {'image': uint8[N,H,W,3]} and, with a RawState
+        observer, its key -> pinned float32[N,S,16]).  Returns `host` once everything has
+        arrived (the caller owns the TimeStep).  The sprite observation travels like the frames:
+        stored by the kernel straight into the pinned tensor with 'mapped', computed in device
+        memory and copied after it otherwise.
 
         frames = 'mapped': the step call draws every env's frame straight into the pinned host
         image (the kernels' stores cross PCIe while other envs are still being stepped; no
@@ -382,6 +420,7 @@ class BatchedEnvironment(object):
         (mapped stores hide behind the step but move fewer bytes per second than the copy
         engines); 'device' when the image is not pinned."""
         img = host.observation[self._image_key] if self._image_key is not None else None
+        spr = host.observation.get(self._state_key) if self._state_key is not None else None
         auto = frames == 'auto'
         if auto:
             frames = self._auto_frames(img)
@@ -395,11 +434,18 @@ class BatchedEnvironment(object):
                 self.reset()
                 if img is not None:
                     img.copy_(e.frames, non_blocking=True)
+                if spr is not None:
+                    spr.copy_(e.sprites, non_blocking=True)
             else:
                 dst = None if img is None else (img if frames == 'mapped' else True)
                 e.env_step(self._flatten_action(action), sample_resets=(self.reset_mode == 'device'), frames=dst)
                 if img is not None and frames == 'device':
                     img.copy_(e.frames, non_blocking=True)
+                if spr is not None:
+                    if frames == 'mapped':
+                        e.observe_sprites(out=spr)
+                    else:
+                        spr.copy_(e.observe_sprites(), non_blocking=True)
             host.step_type.copy_(e.step_type, non_blocking=True)
             host.reward.copy_(e.reward, non_blocking=True)
             if host.discount is not None:
@@ -409,6 +455,8 @@ class BatchedEnvironment(object):
                 self._auto_record(frames, time.perf_counter() - t_begin)
             return host
         self.engine.env_step(self._flatten_action(action), sample_resets=(self.reset_mode == 'device'))
+        if spr is not None:
+            spr.copy_(e.observe_sprites(), non_blocking=True)
         if self._copy_stream is None:
             self._copy_stream = torch.cuda.Stream(device=e.device)
             self._copy_events = [torch.cuda.Event() for _ in range(64)]
@@ -475,12 +523,16 @@ class BatchedEnvironment(object):
         obs = {}
         if self._image_key is not None:
             obs[self._image_key] = self.engine.render()
+        if self._state_key is not None:
+            obs[self._state_key] = self.engine.observe_sprites()
         return obs
 
     def _timestep(self, rendered=False):
         e = self.engine
         if rendered:
             obs = {self._image_key: e.frames} if self._image_key is not None else {}
+            if self._state_key is not None:
+                obs[self._state_key] = e.observe_sprites()
         else:
             obs = self.observation()
         return TimeStep(e.step_type, e.reward, e.discount, obs)
@@ -561,10 +613,11 @@ class HostPipeline(object):
 
     i.e. the policy acts on an observation that is one step old (the usual actor pipeline); with
     depth 1 it is `step_to_host`.  Every submit copies that step's actions host -> device and
-    every collect returns step_type / reward / discount / frames in pinned host memory, valid
-    until `depth` further submits.  frames = 'mapped': the kernels store the frames straight
-    into the slot's pinned image over PCIe as the envs finish; 'device': they are drawn in HBM
-    and copied by a copy engine on a second stream while the next step runs.
+    every collect returns step_type / reward / discount / frames (and the RawState observation
+    when the config has one) in pinned host memory, valid until `depth` further submits.
+    frames = 'mapped': the kernels store the frames and the sprite observation straight into the
+    slot's pinned buffers over PCIe; 'device': they are written to HBM and copied by a copy engine
+    on a second stream while the next step runs.
     Reference protocol: moog/environment.py:98-126 (one `step` per submit, auto-reset included).
     """
 
@@ -581,14 +634,17 @@ class HostPipeline(object):
         pin = lambda *shape, dtype: torch.empty(shape, dtype=dtype).pin_memory()
         self._slots = []
         for _ in range(self.depth):
-            img = None
+            img = spr = None
+            obs = {}
             if env._image_key is not None:  # pylint: disable=protected-access
-                img = pin(*e.frames.shape, dtype=torch.uint8)
+                img = obs[env._image_key] = pin(*e.frames.shape, dtype=torch.uint8)  # pylint: disable=protected-access
+            if env._state_key is not None:  # pylint: disable=protected-access
+                spr = obs[env._state_key] = pin(*e.sprites.shape, dtype=torch.float32)  # pylint: disable=protected-access
             self._slots.append(dict(
-                ts=TimeStep(pin(n, dtype=torch.int32), pin(n, dtype=torch.float32), pin(n, dtype=torch.float32),
-                            {env._image_key: img} if img is not None else {}),  # pylint: disable=protected-access
-                img=img,
+                ts=TimeStep(pin(n, dtype=torch.int32), pin(n, dtype=torch.float32), pin(n, dtype=torch.float32), obs),
+                img=img, spr=spr,
                 dev_frames=(torch.empty_like(e.frames) if (img is not None and frames == 'device') else None),
+                dev_sprites=(torch.empty_like(e.sprites) if (spr is not None and frames == 'device') else None),
                 host_act=pin(n, ad, dtype=torch.float64),
                 dev_act=torch.empty((n, ad), dtype=torch.float64, device=e.device),
                 done=torch.cuda.Event(), stepped=torch.cuda.Event(), busy=False))
@@ -608,6 +664,8 @@ class HostPipeline(object):
                 env.reset()                                   # the first step of a MOOG env is its reset
                 if slot['img'] is not None:
                     slot['img'].copy_(e.frames, non_blocking=True)
+                if slot['spr'] is not None:
+                    slot['spr'].copy_(e.sprites, non_blocking=True)
             else:
                 act = None
                 if action is not None:
@@ -623,15 +681,20 @@ class HostPipeline(object):
                 if slot['img'] is not None:
                     dst = slot['img'] if self.frames == 'mapped' else slot['dev_frames']
                 e.env_step(act, sample_resets=(env.reset_mode == 'device'), frames=dst)
+                if slot['spr'] is not None:
+                    e.observe_sprites(out=slot['spr'] if self.frames == 'mapped' else slot['dev_sprites'])
             ts = slot['ts']
             ts.step_type.copy_(e.step_type, non_blocking=True)
             ts.reward.copy_(e.reward, non_blocking=True)
             ts.discount.copy_(e.discount, non_blocking=True)
-            if self.frames == 'device' and slot['img'] is not None and not was_reset:
+            if self.frames == 'device' and (slot['img'] is not None or slot['spr'] is not None) and not was_reset:
                 slot['stepped'].record(self._main)
                 self._copy.wait_event(slot['stepped'])
                 with torch.cuda.stream(self._copy):
-                    slot['img'].copy_(slot['dev_frames'], non_blocking=True)
+                    if slot['img'] is not None:
+                        slot['img'].copy_(slot['dev_frames'], non_blocking=True)
+                    if slot['spr'] is not None:
+                        slot['spr'].copy_(slot['dev_sprites'], non_blocking=True)
                     slot['done'].record(self._copy)
             else:
                 slot['done'].record(self._main)

@@ -74,6 +74,10 @@ SC_ALL, SC_ANY, SC_COUNT, SC_CONTACT_COUNT, SC_CONTACT_ANY_COUNT, SC_CONST, \
 Z_GENERATE = 192
 Z_N_ATTRS, Z_SHAPE_ATTR = 14, 13
 ZK_CONST, ZK_UNIFORM32, ZK_DISCRETE, ZK_DISCRETE_P = 0, 1, 2, 3
+# columns of the sprite observation (MOOG_OBS_*): float32 [N, n_slots, OBS_COLS]
+(OBS_X, OBS_Y, OBS_SHAPE, OBS_ANGLE, OBS_SCALE, OBS_ASPECT, OBS_C0, OBS_C1, OBS_C2, OBS_OPACITY,
+ OBS_X_VEL, OBS_Y_VEL, OBS_ANGLE_VEL, OBS_MASS, OBS_LAYER, OBS_ALIVE) = range(16)
+OBS_COLS = 16
 
 FL_SYMMETRIC = 1
 FL_UPDATE_ANGLE_VEL = 2
@@ -144,6 +148,7 @@ class Program(object):
         self.layer_vcap = []     # cached-vertex capacity per sprite, per layer
         self.voff = [0]          # first cached vertex of each slot
         self.render = None       # dict or None
+        self.state_key = None    # observers key of the RawState observer, or None
         self.blob = b''
 
     # -- helpers used while building --
@@ -770,13 +775,16 @@ def _compile_rules(prog, rules):
 
 def _compile_render(prog, observers):
     renderer = None
-    for obs in (observers or {}).values():
+    prog.state_key = None
+    for key, obs in (observers or {}).items():
         if _kind(obs) == 'PILRenderer':
             if renderer is not None:
                 raise CompileError('only one PILRenderer observer is supported')
             renderer = obs
         elif _kind(obs) == 'RawState':
-            continue
+            if prog.state_key is not None:
+                raise CompileError('only one RawState observer is supported')
+            prog.state_key = key
         elif callable(obs) and _kind(obs) == 'function':
             continue  # e.g. runtime_benchmark's `lambda _: None`
         else:

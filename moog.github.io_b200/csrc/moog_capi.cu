@@ -542,6 +542,23 @@ static int render_impl(moog_program *p, const moog_state *st, int n_envs, uint8_
   return err == cudaSuccess ? 0 : cuda_fail(err);
 }
 
+int moog_observe_sprites(moog_program *p, const moog_state *st, int n_envs, float *out, void *stream) {
+  if (!p || !valid_state(st) || !out || n_envs < 0 || ((uintptr_t)out & 15)) return MOOG_E_INVAL;
+  if (n_envs == 0) return 0;
+  moog::ObserveArgs a;
+  memset(&a, 0, sizeof(a));
+  a.st = *st;
+  a.out = out;
+  a.n_envs = n_envs;
+  a.S = p->hdr[MOOG_H_N_SLOTS];
+  a.L = p->hdr[MOOG_H_N_LAYERS];
+  memcpy(a.layer_off, &p->hdr[MOOG_H_LAYER_OFF], sizeof(a.layer_off));
+  int launches = 0;
+  cudaError_t err = moog::launch_observe(a, (cudaStream_t)stream, &launches);
+  g_launches += launches;
+  return err == cudaSuccess ? 0 : cuda_fail(err);
+}
+
 const char *moog_strerror(int code) {
   switch (code) {
     case 0: return "ok";

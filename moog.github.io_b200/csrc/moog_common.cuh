@@ -68,6 +68,13 @@ struct RenderArgs {
   int ksize_h, ksize_v;
 };
 
+struct ObserveArgs {
+  moog_state st;
+  float *out;  // [n_envs][S][MOOG_OBS_COLS]
+  int n_envs, S, L;
+  int layer_off[MOOG_MAX_LAYERS + 1];
+};
+
 // Launch options of one program (moog_program_set_option / the MOOG_* environment variables, which
 // are read ONCE, when the program is created).  -1 / 0 = decided by the library.
 struct LaunchOptions {
@@ -109,6 +116,8 @@ int resample_tables(int H, int W, int OH, int OW, std::vector<int> &table, int *
 cudaError_t launch_render(const RenderArgs &a, const int32_t *host_hdr, cudaStream_t stream, int *n_launches,
                           int *done = nullptr, int n_done = 0, int tail_mode = 1,
                           const LaunchOptions &opt = LaunchOptions());
+// moog_observe_sprites (moog_observe.cu): one warp per env
+cudaError_t launch_observe(const ObserveArgs &a, cudaStream_t stream, int *n_launches);
 // ints behind the finished list that launch_render's tail kernels use: a ticket counter and the
 // per-SM count of envs being stepped
 constexpr int kTailExtraInts = 1 + 256;

@@ -17,6 +17,7 @@ from datetime import datetime
 import numpy as np
 import torch
 
+from . import compiler
 from .batched_env import STEP_FIRST, STEP_LAST
 
 
@@ -42,6 +43,10 @@ class VectorGymWrapper(object):
         if r is not None and self._env._image_key is not None:  # pylint: disable=protected-access
             spaces[self._env._image_key] = dict(  # pylint: disable=protected-access
                 low=0, high=255, shape=(r['height'], r['width'], 3), dtype='uint8')
+        key = self._env.program.state_key
+        if key is not None:
+            spaces[key] = dict(low=-np.inf, high=np.inf, shape=(self._env.program.n_slots, compiler.OBS_COLS),
+                               dtype='float32')
         return spaces
 
     @property
@@ -250,10 +255,6 @@ class BatchedLoggingEnvironment(object):
         return parts
 
     # -- serialisation ------------------------------------------------------------
-    def _shape_names(self):
-        table = self._env._pool_arrays.get('shape_table')  # pylint: disable=protected-access
-        return list(getattr(table, 'names', [])) if table is not None else []
-
     def _log(self, ts, action):
         env, prog = self._env, self._env.program
         st = env.engine.state
@@ -265,7 +266,7 @@ class BatchedLoggingEnvironment(object):
             a = env._flatten_action(action)  # pylint: disable=protected-access
             a = a if torch.is_tensor(a) else torch.as_tensor(np.asarray(a))
             act = a.reshape(env.num_envs, -1)[self._idx.to(a.device)].cpu().numpy()
-        names = self._shape_names()
+        names = self._env.shape_names()
         now = time.time()
         for k, n in enumerate(self._envs):
             first = int(step_type[k]) == STEP_FIRST

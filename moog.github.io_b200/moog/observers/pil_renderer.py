@@ -45,7 +45,11 @@ class PILRenderer(AbstractObserver):
 
 
 class RawState(AbstractObserver):
-    """Marker observer: the batched environment exposes its SoA state tensors
-    under this key instead of Python sprite objects (raw_state.py:17-19)."""
+    """Marker observer for the sprites' state (raw_state.py:17-19).  Instead of an OrderedDict of
+    layer -> list of Sprite, the batched environment returns under this key one float32 tensor
+    [num_envs, S, 16] over all S sprite slots of the record, in layer order and, within a layer, in
+    list (z-) order.  Columns: x, y, shape id, angle, scale, aspect_ratio, c0, c1, c2, opacity,
+    x_vel, y_vel, angle_vel, mass, the slot's layer index, alive (1 for a live sprite; every other
+    column of an empty slot is 0).  `BatchedEnvironment.shape_names()` names the shape ids."""
 
     _observation_spec = None
