@@ -126,6 +126,15 @@ int moog_overlap_pairs(moog_program *p, const moog_state *st, int n_envs, int la
  * frames[N][H][W][3] uint8, row 0 = top. */
 int moog_render(moog_program *p, const moog_state *st, int n_envs, uint8_t *frames, void *stream);
 
+/* moog_render for view `view` of a config with several PILRenderer observers (views: moog_b200_program.h
+ * MOOG_H_VIEWS): frames[N][H_view][W_view][3] uint8 with that renderer's settings; view 0 is what
+ * moog_render draws.  A launch of its own on `stream`, like moog_observe_sprites: call it after
+ * moog_env_step (whose io.frames is view 0) to draw the other views of the state that call left.  `frames`
+ * is any device-accessible address aligned to 16 bytes: HBM, or pinned host memory.  MOOG_E_INVAL for a
+ * NULL program / state / frames, n_envs < 0, a misaligned frames, a program without a renderer or a view
+ * outside [0, 1 + hdr[MOOG_H_N_VIEWS]). */
+int moog_render_view(moog_program *p, const moog_state *st, int n_envs, int view, uint8_t *frames, void *stream);
+
 /* RawState.__call__ (moog/observers/raw_state.py:17-19) for N envs: every sprite slot's state as
  * out[N][S][MOOG_OBS_COLS] float32 (layout and columns: moog_b200_program.h MOOG_OBS_*).  A launch of its
  * own on `stream`, so call it after moog_env_step to observe the state that call left.  `out` is any

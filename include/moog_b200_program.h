@@ -128,6 +128,8 @@ enum {
   MOOG_H_N_METAVAR = 57,  /* entries of the env's `meta_state` dict carried in envf (numbers; strings as codes) */
   MOOG_H_METAVAR_OFF = 58,  /* envf offset of the first one */
   MOOG_H_METAVAR_INIT = 59, /* dpool index of their values after meta_state_initializer() (environment.py:86) */
+  MOOG_H_VIEWS = 60,      /* index in ipool of the view table: MOOG_H_N_VIEWS rows of MOOG_VIEW_WORDS */
+  MOOG_H_N_VIEWS = 61,    /* PILRenderer observers after the first (views 1..); 0 = one renderer or none */
   MOOG_H_META_OFF = 56,   /* envf offset of column 0; column k of slot s is envf[off + k * S + s], NaN = no such key.
                              Read as attribute MOOG_AT_META0 + k; travels with the sprite when slots are compacted */
   MOOG_H_CMASK_WORDS = 50 /* 32-bit words of the per-env broad-phase candidate matrices of all
@@ -135,6 +137,30 @@ enum {
                              layer b / 32) words per row).  Derived: moog_program_create fills
                              it in, whatever the blob says. */
 };
+
+/* Views: one per PILRenderer observer, in the order of the config's observers dict.  View 0's settings
+ * are the header words MOOG_H_R_HEIGHT .. MOOG_H_R_ENABLED; view k >= 1 is row k - 1 of the view table,
+ * ipool[hdr[MOOG_H_VIEWS] + MOOG_VIEW_WORDS * (k - 1) ...], whose words are in the same order.  The
+ * renderer reads every view through a pointer to its MOOG_VIEW_WORDS words. */
+#define MOOG_VIEW_WORDS 8
+#define MOOG_MAX_VIEWS 8 /* renderers per program, view 0 included */
+enum {
+  MOOG_V_HEIGHT = 0, MOOG_V_WIDTH, MOOG_V_AA, MOOG_V_BG, MOOG_V_COLORMAP, MOOG_V_MODIFIER, MOOG_V_MOD_LAYER,
+  MOOG_V_ENABLED
+};
+#ifdef __cplusplus
+#define MOOG_STATIC_ASSERT_ static_assert
+#else
+#define MOOG_STATIC_ASSERT_ _Static_assert
+#endif
+MOOG_STATIC_ASSERT_(MOOG_H_R_WIDTH - MOOG_H_R_HEIGHT == MOOG_V_WIDTH && MOOG_H_R_AA - MOOG_H_R_HEIGHT == MOOG_V_AA &&
+                        MOOG_H_R_BG - MOOG_H_R_HEIGHT == MOOG_V_BG &&
+                        MOOG_H_R_COLORMAP - MOOG_H_R_HEIGHT == MOOG_V_COLORMAP &&
+                        MOOG_H_R_MODIFIER - MOOG_H_R_HEIGHT == MOOG_V_MODIFIER &&
+                        MOOG_H_R_MOD_LAYER - MOOG_H_R_HEIGHT == MOOG_V_MOD_LAYER &&
+                        MOOG_H_R_ENABLED - MOOG_H_R_HEIGHT == MOOG_V_ENABLED && MOOG_V_ENABLED + 1 == MOOG_VIEW_WORDS,
+                    "the header's renderer words are a view row");
+#undef MOOG_STATIC_ASSERT_
 
 enum { MOOG_CMAP_NONE = 0, MOOG_CMAP_HSV = 1 };
 enum { MOOG_PMOD_NONE = 0, MOOG_PMOD_FIRST_PERSON = 1, MOOG_PMOD_TORUS = 2 };

@@ -8,7 +8,8 @@ num_envs=N)` works on an unchanged MOOG config -- and the same `reset()` /
     step_type   int32  [N]   0 FIRST, 1 MID, 2 LAST        (dm_env.StepType)
     reward      float32[N]   NaN on FIRST steps            (dm_env: None)
     discount    float32[N]   1 mid, 0 last, NaN first
-    observation {'image': uint8 [N, H, W, 3]}              (PILRenderer)
+    observation {'image': uint8 [N, H, W, 3]}              (PILRenderer; each one of the config's
+                                                           PILRenderers under its own key)
                 {key: float32 [N, S, 16]}                 (RawState: every sprite slot, see
                                                            include/moog_b200_program.h MOOG_OBS_*)
 
@@ -149,11 +150,13 @@ class Engine(object):
         self.step_type = torch.zeros(self.n, dtype=torch.int32, device=self.device)
         self.counters = torch.zeros((self.n, 8), dtype=torch.int64, device=self.device)
         self.stats = torch.zeros(4, dtype=torch.float64, device=self.device)
-        self.frames = None
-        if program.render is not None:
-            r = program.render
-            self.frames = torch.zeros((self.n, r['height'], r['width'], 3),
-                                      dtype=torch.uint8, device=self.device)
+        # view 0 (the first PILRenderer) in `frames`, the further ones in `view_frames`, in view order
+        views = [r for _, r in getattr(program, 'views', ())] or (
+            [program.render] if program.render is not None else [])
+        frames = [torch.zeros((self.n, r['height'], r['width'], 3), dtype=torch.uint8, device=self.device)
+                  for r in views]
+        self.frames = frames[0] if frames else None
+        self.view_frames = frames[1:]
         self.sprites = None
         if getattr(program, 'state_key', None) is not None:
             self.sprites = torch.zeros((self.n, program.n_slots, compiler.OBS_COLS), **f32)
@@ -270,19 +273,43 @@ class Engine(object):
                 self.dev_program.handle, ctypes.byref(st), self.n, la, lb, _ptr(out), self._stream()))
         return out
 
-    def render(self, out=None, first=0, count=None):
-        """Frames of the envs [first, first + count) into out[first:first + count]."""
+    @property
+    def n_views(self):
+        """PILRenderer observers of the program (0 without one)."""
+        return 0 if self.frames is None else 1 + len(self.view_frames)
+
+    def view_buffer(self, view):
+        """This engine's frames of view `view`: `frames` for view 0, else `view_frames[view - 1]`."""
+        if not 0 <= view < self.n_views:
+            raise ValueError('view {} is outside [0, {})'.format(view, self.n_views))
+        return self.frames if view == 0 else self.view_frames[view - 1]
+
+    def render(self, out=None, first=0, count=None, view=0):
+        """Frames of view `view` of the envs [first, first + count) into out[first:first + count]
+        (`out` None: the view's own buffer).  A view other than 0 is drawn by `moog_render_view`
+        into a contiguous uint8 [N, H, W, 3] tensor on this device or in pinned host memory, whose
+        range starts 16-byte aligned."""
         if self.frames is None:
             raise capi.MoogError('the program has no PILRenderer observer')
-        out = self.frames if out is None else out
+        own = self.view_buffer(view)
+        out = own if out is None else out
         count = self.n - first if count is None else count
         if first < 0 or count < 0 or first + count > self.n:
             raise ValueError('env range [{}, {}) is outside [0, {})'.format(first, first + count, self.n))
+        if view != 0:
+            if out.dtype != torch.uint8 or tuple(out.shape) != tuple(own.shape) or not out.is_contiguous():
+                raise ValueError('frames of view {} must be a contiguous uint8 tensor of shape {}'.format(
+                    view, tuple(own.shape)))
+            self._check_reachable(out, 'frames')
         st = self.state.struct(first)
         dst = ctypes.c_void_p(out.data_ptr() + first * out.stride(0) * out.element_size())
         with torch.cuda.device(self.device):
-            capi.check(capi.lib().moog_render(
-                self.dev_program.handle, ctypes.byref(st), count, dst, self._stream()))
+            if view == 0:
+                capi.check(capi.lib().moog_render(
+                    self.dev_program.handle, ctypes.byref(st), count, dst, self._stream()))
+            else:
+                capi.check(capi.lib().moog_render_view(
+                    self.dev_program.handle, ctypes.byref(st), count, view, dst, self._stream()))
         return out
 
     def observe_sprites(self, out=None):
@@ -335,10 +362,9 @@ class BatchedEnvironment(object):
         self.engine.set_pool(self._pool_arrays)
         self.action_space = action_space
         self.observers = observers
-        self._image_key = None
-        for k, obs in (observers or {}).items():
-            if type(obs).__name__ == 'PILRenderer':
-                self._image_key = k
+        # observers keys of the PILRenderers in view order (view 0 first)
+        self._image_keys = [k for k, _ in self.program.views]
+        self._image_key = self._image_keys[0] if self._image_keys else None
         self._state_key = self.program.state_key
         self._rng = np.random.RandomState(seed)
         self._started = False
@@ -404,11 +430,13 @@ class BatchedEnvironment(object):
     def step_to_host(self, action, host, chunks=4, frames='auto'):
         """`step(action)` whose TimeStep lands in the caller's pinned host buffers:
         `host` is a TimeStep of CPU tensors (step_type int32[N], reward float32[N],
-        discount float32[N] or None, observation {'image': uint8[N,H,W,3]} and, with a RawState
-        observer, its key -> pinned float32[N,S,16]).  Returns `host` once everything has
-        arrived (the caller owns the TimeStep).  The sprite observation travels like the frames:
-        stored by the kernel straight into the pinned tensor with 'mapped', computed in device
-        memory and copied after it otherwise.
+        discount float32[N] or None, observation {'image': uint8[N,H,W,3]} -- one such image per
+        PILRenderer, under its key -- and, with a RawState observer, its key -> pinned
+        float32[N,S,16]).  Returns `host` once everything has arrived (the caller owns the
+        TimeStep).  The other views and the sprite observation travel like the frames of view 0:
+        stored by their kernels straight into the pinned tensors with 'mapped', computed in device
+        memory and copied after it otherwise (with 'chunked': range by range, a view whose frame
+        is not a multiple of 16 bytes in one range).
 
         frames = 'mapped': the step call draws every env's frame straight into the pinned host
         image (the kernels' stores cross PCIe while other envs are still being stepped; no
@@ -420,6 +448,7 @@ class BatchedEnvironment(object):
         (mapped stores hide behind the step but move fewer bytes per second than the copy
         engines); 'device' when the image is not pinned."""
         img = host.observation[self._image_key] if self._image_key is not None else None
+        more = [host.observation[k] for k in self._image_keys[1:]]  # views 1..
         spr = host.observation.get(self._state_key) if self._state_key is not None else None
         auto = frames == 'auto'
         if auto:
@@ -434,6 +463,8 @@ class BatchedEnvironment(object):
                 self.reset()
                 if img is not None:
                     img.copy_(e.frames, non_blocking=True)
+                for dst, src in zip(more, e.view_frames):
+                    dst.copy_(src, non_blocking=True)
                 if spr is not None:
                     spr.copy_(e.sprites, non_blocking=True)
             else:
@@ -441,6 +472,11 @@ class BatchedEnvironment(object):
                 e.env_step(self._flatten_action(action), sample_resets=(self.reset_mode == 'device'), frames=dst)
                 if img is not None and frames == 'device':
                     img.copy_(e.frames, non_blocking=True)
+                for v, dst in enumerate(more, 1):
+                    if frames == 'mapped':
+                        e.render(out=dst, view=v)
+                    else:
+                        dst.copy_(e.render(view=v), non_blocking=True)
                 if spr is not None:
                     if frames == 'mapped':
                         e.observe_sprites(out=spr)
@@ -466,7 +502,10 @@ class BatchedEnvironment(object):
         if host.discount is not None:
             host.discount.copy_(e.discount, non_blocking=True)
         if self._image_key is not None:
-            dst = host.observation[self._image_key]
+            dsts = [host.observation[k] for k in self._image_keys]
+            # a range of a view other than 0 must start 16-byte aligned (moog_render_view): a view
+            # whose frame is not a multiple of 16 bytes is drawn and copied whole with the first range
+            ranged = [v == 0 or e.view_buffer(v)[0].numel() % 16 == 0 for v in range(len(dsts))]
             chunks = max(1, min(int(chunks), len(self._copy_events), self.num_envs))
             # equal ranges: measured on B200 / PCIe 5 with 4096 64x64 frames, 4 equal ranges beat
             # 1, 2, 8 or 16 ranges and growing / shrinking ones (each render launch has a fixed
@@ -478,12 +517,18 @@ class BatchedEnvironment(object):
                 count = min(count, self.num_envs - first)
                 if count <= 0:
                     continue
-                e.render(first=first, count=count)
+                spans = []
+                for v in range(len(dsts)):
+                    span = (first, first + count) if ranged[v] else ((0, self.num_envs) if c == 0 else None)
+                    if span is not None:
+                        e.render(first=span[0], count=span[1] - span[0], view=v)
+                        spans.append((v, span))
                 ev = self._copy_events[c]
                 ev.record(main)
                 copy.wait_event(ev)
                 with torch.cuda.stream(copy):
-                    dst[first:first + count].copy_(e.frames[first:first + count], non_blocking=True)
+                    for v, (a, b) in spans:
+                        dsts[v][a:b].copy_(e.view_buffer(v)[a:b], non_blocking=True)
                 first += count
         copy.synchronize()
         main.synchronize()
@@ -521,8 +566,8 @@ class BatchedEnvironment(object):
 
     def observation(self):
         obs = {}
-        if self._image_key is not None:
-            obs[self._image_key] = self.engine.render()
+        for v, key in enumerate(self._image_keys):
+            obs[key] = self.engine.render(view=v)
         if self._state_key is not None:
             obs[self._state_key] = self.engine.observe_sprites()
         return obs
@@ -530,7 +575,10 @@ class BatchedEnvironment(object):
     def _timestep(self, rendered=False):
         e = self.engine
         if rendered:
+            # view 0 came with the step call; the other views are drawn behind it
             obs = {self._image_key: e.frames} if self._image_key is not None else {}
+            for v, key in enumerate(self._image_keys[1:], 1):
+                obs[key] = e.render(view=v)
             if self._state_key is not None:
                 obs[self._state_key] = e.observe_sprites()
         else:
@@ -613,11 +661,11 @@ class HostPipeline(object):
 
     i.e. the policy acts on an observation that is one step old (the usual actor pipeline); with
     depth 1 it is `step_to_host`.  Every submit copies that step's actions host -> device and
-    every collect returns step_type / reward / discount / frames (and the RawState observation
-    when the config has one) in pinned host memory, valid until `depth` further submits.
-    frames = 'mapped': the kernels store the frames and the sprite observation straight into the
-    slot's pinned buffers over PCIe; 'device': they are written to HBM and copied by a copy engine
-    on a second stream while the next step runs.
+    every collect returns step_type / reward / discount / frames of every PILRenderer (and the
+    RawState observation when the config has one) in pinned host memory, valid until `depth`
+    further submits.  frames = 'mapped': the kernels store the frames and the sprite observation
+    straight into the slot's pinned buffers over PCIe; 'device': they are written to HBM and copied
+    by a copy engine on a second stream while the next step runs.
     Reference protocol: moog/environment.py:98-126 (one `step` per submit, auto-reset included).
     """
 
@@ -634,16 +682,18 @@ class HostPipeline(object):
         pin = lambda *shape, dtype: torch.empty(shape, dtype=dtype).pin_memory()
         self._slots = []
         for _ in range(self.depth):
-            img = spr = None
+            spr = None
             obs = {}
-            if env._image_key is not None:  # pylint: disable=protected-access
-                img = obs[env._image_key] = pin(*e.frames.shape, dtype=torch.uint8)  # pylint: disable=protected-access
+            imgs = []  # one pinned image per view, in view order
+            for v, key in enumerate(env._image_keys):  # pylint: disable=protected-access
+                imgs.append(pin(*e.view_buffer(v).shape, dtype=torch.uint8))
+                obs[key] = imgs[-1]
             if env._state_key is not None:  # pylint: disable=protected-access
                 spr = obs[env._state_key] = pin(*e.sprites.shape, dtype=torch.float32)  # pylint: disable=protected-access
             self._slots.append(dict(
                 ts=TimeStep(pin(n, dtype=torch.int32), pin(n, dtype=torch.float32), pin(n, dtype=torch.float32), obs),
-                img=img, spr=spr,
-                dev_frames=(torch.empty_like(e.frames) if (img is not None and frames == 'device') else None),
+                imgs=imgs, spr=spr,
+                dev_imgs=[torch.empty_like(e.view_buffer(v)) for v in range(len(imgs))] if frames == 'device' else None,
                 dev_sprites=(torch.empty_like(e.sprites) if (spr is not None and frames == 'device') else None),
                 host_act=pin(n, ad, dtype=torch.float64),
                 dev_act=torch.empty((n, ad), dtype=torch.float64, device=e.device),
@@ -662,8 +712,8 @@ class HostPipeline(object):
         with torch.cuda.stream(self._main):
             if was_reset:
                 env.reset()                                   # the first step of a MOOG env is its reset
-                if slot['img'] is not None:
-                    slot['img'].copy_(e.frames, non_blocking=True)
+                for v, img in enumerate(slot['imgs']):
+                    img.copy_(e.view_buffer(v), non_blocking=True)
                 if slot['spr'] is not None:
                     slot['spr'].copy_(e.sprites, non_blocking=True)
             else:
@@ -677,22 +727,22 @@ class HostPipeline(object):
                         slot['host_act'].copy_(torch.as_tensor(action).reshape(slot['host_act'].shape))
                         slot['dev_act'].copy_(slot['host_act'], non_blocking=True)
                     act = slot['dev_act']
-                dst = None
-                if slot['img'] is not None:
-                    dst = slot['img'] if self.frames == 'mapped' else slot['dev_frames']
-                e.env_step(act, sample_resets=(env.reset_mode == 'device'), frames=dst)
+                dsts = slot['imgs'] if self.frames == 'mapped' else slot['dev_imgs']
+                e.env_step(act, sample_resets=(env.reset_mode == 'device'), frames=dsts[0] if dsts else None)
+                for v in range(1, len(dsts)):
+                    e.render(out=dsts[v], view=v)
                 if slot['spr'] is not None:
                     e.observe_sprites(out=slot['spr'] if self.frames == 'mapped' else slot['dev_sprites'])
             ts = slot['ts']
             ts.step_type.copy_(e.step_type, non_blocking=True)
             ts.reward.copy_(e.reward, non_blocking=True)
             ts.discount.copy_(e.discount, non_blocking=True)
-            if self.frames == 'device' and (slot['img'] is not None or slot['spr'] is not None) and not was_reset:
+            if self.frames == 'device' and (slot['imgs'] or slot['spr'] is not None) and not was_reset:
                 slot['stepped'].record(self._main)
                 self._copy.wait_event(slot['stepped'])
                 with torch.cuda.stream(self._copy):
-                    if slot['img'] is not None:
-                        slot['img'].copy_(slot['dev_frames'], non_blocking=True)
+                    for img, dev in zip(slot['imgs'], slot['dev_imgs']):
+                        img.copy_(dev, non_blocking=True)
                     if slot['spr'] is not None:
                         slot['spr'].copy_(slot['dev_sprites'], non_blocking=True)
                     slot['done'].record(self._copy)

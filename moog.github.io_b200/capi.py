@@ -41,7 +41,7 @@ SYMBOLS = ('moog_program_create', 'moog_program_destroy',
            'moog_launch_count', 'moog_host_paths_overlap',
            'moog_host_points_in_path', 'moog_step_launch_info',
            'moog_step_draws_frames', 'moog_program_set_option',
-           'moog_program_validate', 'moog_observe_sprites')
+           'moog_program_validate', 'moog_observe_sprites', 'moog_render_view')
 
 
 class MoogError(RuntimeError):
@@ -87,6 +87,8 @@ def lib():
     L.moog_render.restype = ci
     L.moog_observe_sprites.argtypes = [vp, ctypes.POINTER(MoogState), ci, vp, vp]
     L.moog_observe_sprites.restype = ci
+    L.moog_render_view.argtypes = [vp, ctypes.POINTER(MoogState), ci, ci, vp, vp]
+    L.moog_render_view.restype = ci
     L.moog_strerror.argtypes = [ci]
     L.moog_strerror.restype = ctypes.c_char_p
     L.moog_last_cuda_error.argtypes = []

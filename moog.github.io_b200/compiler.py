@@ -56,6 +56,9 @@ H_N_VTX = 49
 H_RESET, H_N_RESET, H_N_DPOOL, H_SHAPE_TAB = 51, 52, 53, 54
 H_N_META, H_META_OFF = 55, 56
 H_N_METAVAR, H_METAVAR_OFF, H_METAVAR_INIT = 57, 58, 59
+H_VIEWS, H_N_VIEWS = 60, 61
+VIEW_WORDS = 8           # MOOG_VIEW_WORDS: a view table row, the words H_R_HEIGHT .. H_R_ENABLED
+MAX_VIEWS = 8            # MOOG_MAX_VIEWS: PILRenderer observers per program
 MAX_META_VARS = 16
 
 F_DRAG, F_KINETIC_FRICTION, F_DOWN_GRAVITY, F_GRAVITY, F_RANDOM, \
@@ -147,7 +150,8 @@ class Program(object):
         self.K = 1
         self.layer_vcap = []     # cached-vertex capacity per sprite, per layer
         self.voff = [0]          # first cached vertex of each slot
-        self.render = None       # dict or None
+        self.render = None       # settings of view 0 (the first PILRenderer), or None
+        self.views = []          # (observers key, render dict) of every PILRenderer, in observers order
         self.state_key = None    # observers key of the RawState observer, or None
         self.blob = b''
 
@@ -238,6 +242,11 @@ class Program(object):
         hdr = np.zeros(HDR_WORDS, dtype='<i4')
         hdr[H_VOFF] = self.add_ints(self.voff)
         hdr[H_N_VTX] = self.voff[-1]
+        if len(self.views) > 1:
+            # views 1..: the view table behind everything else in ipool (a program with one renderer
+            # has no table, and its blob is what it was before views existed)
+            hdr[H_VIEWS] = self.add_ints(w for _, r in self.views[1:] for w in _view_words(r))
+            hdr[H_N_VIEWS] = len(self.views) - 1
         ops = np.zeros(len(self.ops), dtype=OP_DTYPE)
         for k, o in enumerate(self.ops):
             ops[k]['kind'] = o['kind']
@@ -272,16 +281,7 @@ class Program(object):
         hdr[H_NOISE_DIM] = self.noise_dim
         hdr[H_RULE_NOISE_DIM] = self.rule_noise_dim
         if self.render is not None:
-            r = self.render
-            hdr[H_R_ENABLED] = 1
-            hdr[H_R_HEIGHT] = r['height']
-            hdr[H_R_WIDTH] = r['width']
-            hdr[H_R_AA] = r['aa']
-            bg = r['bg']
-            hdr[H_R_BG] = int(bg[0]) | (int(bg[1]) << 8) | (int(bg[2]) << 16)
-            hdr[H_R_COLORMAP] = r['colormap']
-            hdr[H_R_MODIFIER] = r['modifier']
-            hdr[H_R_MOD_LAYER] = r['modifier_layer']
+            hdr[H_R_HEIGHT:H_R_ENABLED + 1] = _view_words(self.render)
         hdr[H_LAYER_OFF:H_LAYER_OFF + len(self.layer_off)] = self.layer_off
         start, count = self.sections.get('reset', (0, 0))
         hdr[H_RESET], hdr[H_N_RESET] = start, count
@@ -773,14 +773,21 @@ def _compile_rules(prog, rules):
 # observers
 # ---------------------------------------------------------------------------
 
+def _view_words(r):
+    """The MOOG_VIEW_WORDS settings of one renderer (header words H_R_HEIGHT .. H_R_ENABLED)."""
+    bg = r['bg']
+    return [r['height'], r['width'], r['aa'], int(bg[0]) | (int(bg[1]) << 8) | (int(bg[2]) << 16),
+            r['colormap'], r['modifier'], r['modifier_layer'], 1]
+
+
 def _compile_render(prog, observers):
-    renderer = None
     prog.state_key = None
+    prog.views = []
     for key, obs in (observers or {}).items():
         if _kind(obs) == 'PILRenderer':
-            if renderer is not None:
-                raise CompileError('only one PILRenderer observer is supported')
-            renderer = obs
+            if len(prog.views) >= MAX_VIEWS:
+                raise CompileError('at most {} PILRenderer observers are supported'.format(MAX_VIEWS))
+            prog.views.append((key, _lower_renderer(prog, obs)))
         elif _kind(obs) == 'RawState':
             if prog.state_key is not None:
                 raise CompileError('only one RawState observer is supported')
@@ -789,9 +796,10 @@ def _compile_render(prog, observers):
             continue  # e.g. runtime_benchmark's `lambda _: None`
         else:
             raise CompileError('unsupported observer {}'.format(_kind(obs)))
-    if renderer is None:
-        prog.render = None
-        return
+    prog.render = prog.views[0][1] if prog.views else None
+
+
+def _lower_renderer(prog, renderer):
     size = tuple(renderer._image_size)
     if len(size) != 2:
         raise CompileError('image_size must be (height, width)')
@@ -825,10 +833,10 @@ def _compile_render(prog, observers):
         raise CompileError('unsupported polygon modifier {}'.format(pk))
     # pil_renderer.py:46,65-66: canvas = (aa*size[0], aa*size[1]) is handed to
     # PIL as (width, height) while the array that comes back is [height, width].
-    prog.render = dict(height=int(size[1]), width=int(size[0]),
-                       aa=int(renderer._anti_aliasing), bg=tuple(bg)[:3],
-                       colormap=cmap, modifier=modifier,
-                       modifier_layer=mod_layer)
+    return dict(height=int(size[1]), width=int(size[0]),
+                aa=int(renderer._anti_aliasing), bg=tuple(bg)[:3],
+                colormap=cmap, modifier=modifier,
+                modifier_layer=mod_layer)
 
 
 # ---------------------------------------------------------------------------

@@ -20,9 +20,13 @@ struct moog_program {
   const void *sched_state;  // the state the costs belong to
   int *done;                // [1 + done_cap]: envs in the order the running step finishes them
   int done_cap;
-  // anti_aliasing > 1: Lanczos coefficient tables (Resample.c), built on first use
-  int *resample;
-  int ksize_h, ksize_v;
+  // views (one per PILRenderer): their settings and where they lie in the blob (int32 words)
+  int n_views;
+  int32_t view[MOOG_MAX_VIEWS][MOOG_VIEW_WORDS];
+  int view_off[MOOG_MAX_VIEWS];
+  // anti_aliasing > 1: Lanczos coefficient tables (Resample.c) per view, built on first use
+  int *resample[MOOG_MAX_VIEWS];
+  int ksize_h[MOOG_MAX_VIEWS], ksize_v[MOOG_MAX_VIEWS];
   // largest outline a slot of each layer can hold (from the blob's voff table)
   int layer_vcap[MOOG_MAX_LAYERS];
   // cached vertex -> (slot << 8 | index within the slot's outline), [VT]: the Euler pass of the step
@@ -255,6 +259,23 @@ int moog_program_validate(const void *blob, size_t nbytes) {
       return MOOG_E_INVAL;
     if (hdr[MOOG_H_R_MODIFIER] == MOOG_PMOD_FIRST_PERSON && !layer_ok(hdr[MOOG_H_R_MOD_LAYER])) return MOOG_E_INVAL;
   }
+  // views 1..: rows of the view table, each a renderer next to view 0
+  const int nv = hdr[MOOG_H_N_VIEWS], vt = hdr[MOOG_H_VIEWS];
+  if (nv < 0 || nv >= MOOG_MAX_VIEWS) return MOOG_E_INVAL;
+  if (nv > 0) {
+    if (!hdr[MOOG_H_R_ENABLED] || vt < 0 || (long long)vt + (long long)MOOG_VIEW_WORDS * nv > NI) return MOOG_E_INVAL;
+    for (int k = 0; k < nv; ++k) {
+      const int32_t *v = pv.ipool + vt + MOOG_VIEW_WORDS * k;
+      if (v[MOOG_V_ENABLED] != 1 || v[MOOG_V_HEIGHT] < 1 || v[MOOG_V_WIDTH] < 1 || v[MOOG_V_AA] < 1 ||
+          v[MOOG_V_HEIGHT] > 8192 || v[MOOG_V_WIDTH] > 8192 || v[MOOG_V_AA] > 16)
+        return MOOG_E_INVAL;
+      if (v[MOOG_V_COLORMAP] != MOOG_CMAP_NONE && v[MOOG_V_COLORMAP] != MOOG_CMAP_HSV) return MOOG_E_INVAL;
+      if (v[MOOG_V_MODIFIER] != MOOG_PMOD_NONE && v[MOOG_V_MODIFIER] != MOOG_PMOD_FIRST_PERSON &&
+          v[MOOG_V_MODIFIER] != MOOG_PMOD_TORUS)
+        return MOOG_E_INVAL;
+      if (v[MOOG_V_MODIFIER] == MOOG_PMOD_FIRST_PERSON && !layer_ok(v[MOOG_V_MOD_LAYER])) return MOOG_E_INVAL;
+    }
+  }
   return 0;
 }
 
@@ -274,6 +295,14 @@ int moog_program_create(const void *blob, size_t nbytes, moog_program **out) {
     for (int l = 0; l < hdr[MOOG_H_N_LAYERS]; ++l) {
       const int a = hdr[MOOG_H_LAYER_OFF + l], b = hdr[MOOG_H_LAYER_OFF + l + 1];
       p->layer_vcap[l] = b > a ? pv.voff[a + 1] - pv.voff[a] : 0;
+    }
+    if (hdr[MOOG_H_R_ENABLED]) {
+      p->n_views = 1 + hdr[MOOG_H_N_VIEWS];
+      for (int k = 0; k < p->n_views; ++k) {
+        const int32_t *v = k == 0 ? hdr + MOOG_H_R_HEIGHT : pv.ipool + hdr[MOOG_H_VIEWS] + MOOG_VIEW_WORDS * (k - 1);
+        memcpy(p->view[k], v, sizeof(p->view[k]));
+        p->view_off[k] = (int)(v - hdr);
+      }
     }
   }
   if (moog::env_smem_bytes(p->hdr) > 220 * 1024 || p->hdr[MOOG_H_CMASK_WORDS] > 2048) {
@@ -314,7 +343,8 @@ void moog_program_destroy(moog_program *p) {
   if (p->dev_vmap) cudaFree(p->dev_vmap);
   if (p->sched) cudaFree(p->sched);
   if (p->done) cudaFree(p->done);
-  if (p->resample) cudaFree(p->resample);
+  for (int k = 0; k < MOOG_MAX_VIEWS; ++k)
+    if (p->resample[k]) cudaFree(p->resample[k]);
   free(p);
 }
 
@@ -376,7 +406,7 @@ int moog_step_draws_frames(const moog_program *p, int n_envs) {
   return moog::plan_step(p->hdr, resident, helper, frames_mode(n_envs), p->opt).fuse ? 1 : 0;
 }
 
-static int render_impl(moog_program *p, const moog_state *st, int n_envs, uint8_t *frames, void *stream,
+static int render_impl(moog_program *p, const moog_state *st, int n_envs, int view, uint8_t *frames, void *stream,
                        int *done, int tail_mode, long long *trace = nullptr);
 
 static int run_step(moog_program *p, const moog_state *st, int n_envs, int mode, const moog_step_io *io,
@@ -465,7 +495,7 @@ static int run_step(moog_program *p, const moog_state *st, int n_envs, int mode,
   g_launches += launches;
   if (err != cudaSuccess) return cuda_fail(err);
   if (a.io.frames && !fused)
-    return render_impl(p, st, n_envs, a.io.frames, stream, tail ? p->done : nullptr, tail_mode,
+    return render_impl(p, st, n_envs, 0, a.io.frames, stream, tail ? p->done : nullptr, tail_mode,
                        a.trace ? (long long *)a.io.counters : nullptr);
   return 0;
 }
@@ -503,41 +533,49 @@ int moog_overlap_pairs(moog_program *p, const moog_state *st, int n_envs, int la
 }
 
 int moog_render(moog_program *p, const moog_state *st, int n_envs, uint8_t *frames, void *stream) {
-  return render_impl(p, st, n_envs, frames, stream, nullptr, 0);
+  return render_impl(p, st, n_envs, 0, frames, stream, nullptr, 0);
 }
 
-static int render_impl(moog_program *p, const moog_state *st, int n_envs, uint8_t *frames, void *stream,
+int moog_render_view(moog_program *p, const moog_state *st, int n_envs, int view, uint8_t *frames, void *stream) {
+  if (!p || !frames || ((uintptr_t)frames & 15) || view < 0 || view >= p->n_views) return MOOG_E_INVAL;
+  return render_impl(p, st, n_envs, view, frames, stream, nullptr, 0);
+}
+
+static int render_impl(moog_program *p, const moog_state *st, int n_envs, int view, uint8_t *frames, void *stream,
                        int *done, int tail_mode, long long *trace) {
   if (!p || !valid_state(st) || !frames || n_envs < 0) return MOOG_E_INVAL;
   if (!p->hdr[MOOG_H_R_ENABLED]) return MOOG_E_INVAL;
-  if (p->hdr[MOOG_H_R_AA] < 1) return MOOG_E_UNSUPPORTED;
+  const int32_t *v = p->view[view];
+  if (v[MOOG_V_AA] < 1) return MOOG_E_UNSUPPORTED;
   moog::RenderArgs a;
   memset(&a, 0, sizeof(a));
   a.blob = p->dev_blob;
+  a.view_off = p->view_off[view];
   a.st = *st;
   a.n_envs = n_envs;
   a.frames = frames;
   a.trace = trace;
-  if (p->hdr[MOOG_H_R_AA] > 1) {
-    if (!p->resample) {
-      const int OH = p->hdr[MOOG_H_R_HEIGHT], OW = p->hdr[MOOG_H_R_WIDTH], aa = p->hdr[MOOG_H_R_AA];
+  if (v[MOOG_V_AA] > 1) {
+    if (!p->resample[view]) {
+      const int OH = v[MOOG_V_HEIGHT], OW = v[MOOG_V_WIDTH], aa = v[MOOG_V_AA];
       std::vector<int> table;
-      int n = moog::resample_tables(aa * OH, aa * OW, OH, OW, table, &p->ksize_h, &p->ksize_v);
-      cudaError_t err = cudaMalloc((void **)&p->resample, sizeof(int) * (size_t)n);
+      int n = moog::resample_tables(aa * OH, aa * OW, OH, OW, table, &p->ksize_h[view], &p->ksize_v[view]);
+      cudaError_t err = cudaMalloc((void **)&p->resample[view], sizeof(int) * (size_t)n);
       if (err == cudaSuccess)
-        err = cudaMemcpy(p->resample, table.data(), sizeof(int) * (size_t)n, cudaMemcpyHostToDevice);
+        err = cudaMemcpy(p->resample[view], table.data(), sizeof(int) * (size_t)n, cudaMemcpyHostToDevice);
       if (err != cudaSuccess) {  // never keep a table that was not filled
-        if (p->resample) cudaFree(p->resample);
-        p->resample = nullptr;
+        if (p->resample[view]) cudaFree(p->resample[view]);
+        p->resample[view] = nullptr;
         return cuda_fail(err);
       }
     }
-    a.resample = p->resample;
-    a.ksize_h = p->ksize_h;
-    a.ksize_v = p->ksize_v;
+    a.resample = p->resample[view];
+    a.ksize_h = p->ksize_h[view];
+    a.ksize_v = p->ksize_v[view];
   }
   int launches = 0;
-  cudaError_t err = moog::launch_render(a, p->hdr, (cudaStream_t)stream, &launches, done, n_envs, tail_mode, p->opt);
+  cudaError_t err =
+      moog::launch_render(a, p->hdr, v, (cudaStream_t)stream, &launches, done, n_envs, tail_mode, p->opt);
   g_launches += launches;
   return err == cudaSuccess ? 0 : cuda_fail(err);
 }

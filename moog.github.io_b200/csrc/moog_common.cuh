@@ -60,6 +60,7 @@ struct StepArgs {
 
 struct RenderArgs {
   const void *blob;
+  int view_off;         // int32 word of the blob where the view's MOOG_VIEW_WORDS settings start
   moog_state st;
   int n_envs;
   uint8_t *frames;
@@ -112,9 +113,10 @@ cudaError_t launch_order(const int *cost, int *order, int n, cudaStream_t stream
 int resample_tables(int H, int W, int OH, int OW, std::vector<int> &table, int *ksize_h, int *ksize_v);
 // done: nullptr, or the finished-env list of the step kernel launched just before on `stream`
 // (StepArgs::done): the render kernel is then launched with programmatic stream serialization,
-// starts while the last envs are still being stepped and draws the envs in finishing order
-cudaError_t launch_render(const RenderArgs &a, const int32_t *host_hdr, cudaStream_t stream, int *n_launches,
-                          int *done = nullptr, int n_done = 0, int tail_mode = 1,
+// starts while the last envs are still being stepped and draws the envs in finishing order.
+// host_view: the host copy of the words at a.view_off (the view's settings)
+cudaError_t launch_render(const RenderArgs &a, const int32_t *host_hdr, const int32_t *host_view, cudaStream_t stream,
+                          int *n_launches, int *done = nullptr, int n_done = 0, int tail_mode = 1,
                           const LaunchOptions &opt = LaunchOptions());
 // moog_observe_sprites (moog_observe.cu): one warp per env
 cudaError_t launch_observe(const ObserveArgs &a, cudaStream_t stream, int *n_launches);

@@ -25,12 +25,13 @@ __global__ void moog_render_kernel(RenderArgs a, int T, int envs_per_block, int 
   extern __shared__ __align__(16) unsigned char smem_raw[];
   ProgramView pv = view_of(a.blob);
   const int32_t *hdr = pv.hdr;
+  const int32_t *view = hdr + a.view_off;
   const int S = hdr[MOOG_H_N_SLOTS], VT = hdr[MOOG_H_N_VTX];
-  const int OH = hdr[MOOG_H_R_HEIGHT], OW = hdr[MOOG_H_R_WIDTH], aa = hdr[MOOG_H_R_AA];
+  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
   const int g = threadIdx.x / T, t = threadIdx.x - g * T;
   const int n = blockIdx.x * envs_per_block + g;
   const bool live = n < a.n_envs;
-  const int C = hdr[MOOG_H_R_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
+  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
   const RenderLayout lay = render_layout(band > 0 ? band : aa * OH, aa * OW, S * C, (VT > 0 ? VT : 1) * C, OW);
   const size_t row = live ? (size_t)n : 0;
   RenderSrc src;
@@ -41,6 +42,7 @@ __global__ void moog_render_kernel(RenderArgs a, int T, int envs_per_block, int 
   src.vtx = (const double2 *)(a.st.vtx + row * 2 * VT);
   src.hdr = hdr;
   src.voff = pv.voff;
+  src.view = view;
   render_env(src, lay, smem_raw + (size_t)g * lay.total, nullptr, t, T, P, live,
              a.frames + row * OH * OW * 3, a.resample, a.ksize_h, a.ksize_v, [] { __syncthreads(); }, band);
 }
@@ -68,9 +70,10 @@ __global__ void moog_render_tail_kernel(RenderArgs a, int T, int P, const int *d
   const int n = s_env;
   ProgramView pv = view_of(a.blob);
   const int32_t *hdr = pv.hdr;
+  const int32_t *view = hdr + a.view_off;
   const int S = hdr[MOOG_H_N_SLOTS], VT = hdr[MOOG_H_N_VTX];
-  const int OH = hdr[MOOG_H_R_HEIGHT], OW = hdr[MOOG_H_R_WIDTH], aa = hdr[MOOG_H_R_AA];
-  const int C = hdr[MOOG_H_R_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
+  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
+  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
   const RenderLayout lay = render_layout(band > 0 ? band : aa * OH, aa * OW, S * C, (VT > 0 ? VT : 1) * C, OW);
   const size_t row = (size_t)n;
   RenderSrc src;
@@ -81,6 +84,7 @@ __global__ void moog_render_tail_kernel(RenderArgs a, int T, int P, const int *d
   src.vtx = (const double2 *)(a.st.vtx + row * 2 * VT);
   src.hdr = hdr;
   src.voff = pv.voff;
+  src.view = view;
   unsigned long long tr0 = 0;
   if (a.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tr0));
   render_env(src, lay, smem_raw, nullptr, (int)threadIdx.x, T, P, true, a.frames + row * OH * OW * 3, a.resample,
@@ -110,9 +114,10 @@ __global__ void moog_render_tail_persistent_kernel(RenderArgs a, int T, int P, i
   asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
   ProgramView pv = view_of(a.blob);
   const int32_t *hdr = pv.hdr;
+  const int32_t *view = hdr + a.view_off;
   const int S = hdr[MOOG_H_N_SLOTS], VT = hdr[MOOG_H_N_VTX];
-  const int OH = hdr[MOOG_H_R_HEIGHT], OW = hdr[MOOG_H_R_WIDTH], aa = hdr[MOOG_H_R_AA];
-  const int C = hdr[MOOG_H_R_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
+  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
+  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
   const RenderLayout lay = render_layout(band > 0 ? band : aa * OH, aa * OW, S * C, (VT > 0 ? VT : 1) * C, OW);
   bool last = false;
   for (;;) {
@@ -154,6 +159,7 @@ __global__ void moog_render_tail_persistent_kernel(RenderArgs a, int T, int P, i
     src.vtx = (const double2 *)(a.st.vtx + row * 2 * VT);
     src.hdr = hdr;
     src.voff = pv.voff;
+    src.view = view;
     unsigned long long tr0 = 0;
     if (a.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tr0));
     render_env(src, lay, smem_raw, nullptr, (int)threadIdx.x, T, P, true, a.frames + row * OH * OW * 3, a.resample,
@@ -225,12 +231,12 @@ int resample_tables(int H, int W, int OH, int OW, std::vector<int> &table, int *
   return (int)table.size();
 }
 
-cudaError_t launch_render(const RenderArgs &a, const int32_t *hdr, cudaStream_t stream, int *n_launches,
-                          int *done, int n_done, int tail_mode, const LaunchOptions &opt) {
+cudaError_t launch_render(const RenderArgs &a, const int32_t *hdr, const int32_t *view, cudaStream_t stream,
+                          int *n_launches, int *done, int n_done, int tail_mode, const LaunchOptions &opt) {
   if (a.n_envs <= 0) return cudaSuccess;
-  const int OH = hdr[MOOG_H_R_HEIGHT], OW = hdr[MOOG_H_R_WIDTH], aa = hdr[MOOG_H_R_AA];
+  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
   const int H = aa * OH, W = aa * OW, S = hdr[MOOG_H_N_SLOTS], VT = hdr[MOOG_H_N_VTX];
-  const int C = hdr[MOOG_H_R_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;  // TorusGeometry: 9 copies per sprite
+  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;  // TorusGeometry: 9 copies per sprite
   // A canvas that does not fit next to the edge lists in one CTA's shared memory is drawn in bands
   // of `band` rows (render_env): the largest band, a multiple of 8 rows, whose layout leaves room
   // for two CTAs per SM.  Anti-aliased canvases are not banded (the Lanczos resize reads across rows).

@@ -305,6 +305,7 @@ struct RenderSrc {
   const int32_t *meta, *cnt;
   const double2 *vtx;
   const int32_t *hdr, *voff;  // program header, slot -> first cached vertex
+  const int32_t *view;        // the view's MOOG_VIEW_WORDS settings (view 0: hdr + MOOG_H_R_HEIGHT)
 };
 
 // PILRenderer.__call__ for ONE env by the T threads t = 0..T-1 of a CTA (every thread of the
@@ -320,13 +321,13 @@ template <class Sync>
 __device__ __forceinline__ void render_env(const RenderSrc &src, const RenderLayout &lay, unsigned char *base,
                                            unsigned *ext_items, int t, int T, int P, bool live, unsigned char *out,
                                            const int *resample, int ksize_h, int ksize_v, Sync sync, int HB = 0) {
-  const int32_t *hdr = src.hdr;
+  const int32_t *hdr = src.hdr, *view = src.view;
   const int S = hdr[MOOG_H_N_SLOTS], L = hdr[MOOG_H_N_LAYERS], VT = hdr[MOOG_H_N_VTX];
   // pil_renderer.py:65-66: the canvas is anti_aliasing x the image size
-  const int OH = hdr[MOOG_H_R_HEIGHT], OW = hdr[MOOG_H_R_WIDTH], aa = hdr[MOOG_H_R_AA];
+  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
   const int H = aa * OH, W = aa * OW;
-  const unsigned bgc = (unsigned)hdr[MOOG_H_R_BG] & 0xffffffu;
-  const int cmap = hdr[MOOG_H_R_COLORMAP], pmod = hdr[MOOG_H_R_MODIFIER], pml = hdr[MOOG_H_R_MOD_LAYER];
+  const unsigned bgc = (unsigned)view[MOOG_V_BG] & 0xffffffu;
+  const int cmap = view[MOOG_V_COLORMAP], pmod = view[MOOG_V_MODIFIER], pml = view[MOOG_V_MOD_LAYER];
   // polygon_modifiers.py:88-96 TorusGeometry: every sprite is drawn as 9 copies shifted by
   // (i, j), i outer / j inner over (-1, 0, 1); copy c of slot s is the virtual slot s * C + c
   // and its vertices live at c * VT + voff[s]

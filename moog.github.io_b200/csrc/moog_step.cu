@@ -3771,7 +3771,7 @@ __global__ void __launch_bounds__(64) moog_step_kernel(const StepArgs a) {
     const RenderLayout lay = render_layout(OH, OW, a.S * C, VTr * C, OW, 16 * VTr);
     RenderSrc src;
     src.dyn = e.dyn; src.stat = e.stat; src.meta = e.meta; src.cnt = e.cnt;
-    src.vtx = e.vtx; src.hdr = e.hdr; src.voff = e.voff;
+    src.vtx = e.vtx; src.hdr = e.hdr; src.voff = e.voff; src.view = e.hdr + MOOG_H_R_HEIGHT;
     const int T = (int)blockDim.x;
     const int P = (OH * 2 <= T) ? 2 : 1;
     render_env(src, lay, smem_raw + a.render_off, (unsigned *)e.vtx, (int)threadIdx.x, T, P, true,

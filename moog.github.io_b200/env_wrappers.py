@@ -39,10 +39,8 @@ class VectorGymWrapper(object):
     def observation_space(self):
         """{key: dict(low, high, shape, dtype)} per env (gym_wrapper.py:66-78)."""
         spaces = {}
-        r = self._env.program.render
-        if r is not None and self._env._image_key is not None:  # pylint: disable=protected-access
-            spaces[self._env._image_key] = dict(  # pylint: disable=protected-access
-                low=0, high=255, shape=(r['height'], r['width'], 3), dtype='uint8')
+        for key, r in self._env.program.views:
+            spaces[key] = dict(low=0, high=255, shape=(r['height'], r['width'], 3), dtype='uint8')
         key = self._env.program.state_key
         if key is not None:
             spaces[key] = dict(low=-np.inf, high=np.inf, shape=(self._env.program.n_slots, compiler.OBS_COLS),
