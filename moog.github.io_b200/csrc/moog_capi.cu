@@ -455,8 +455,7 @@ static int run_step(moog_program *p, const moog_state *st, int n_envs, int mode,
   // others than alone (profiles/README.md): with the envs dispatched longest-first, capping
   // the envs resident per SM at about n_envs / (5.5 .. 7 x SMs) finishes the step sooner than filling
   // the SMs (4096 envs on 148 SMs: 5 per SM; measured with the frames drawn behind the step, step
-  // + render per 4096 envs: 3: 5.33 ms, 4: 4.66 ms, 5: 4.46 ms -- the most the 39 KB records of the
-  // helper mode allow -- and 5.6 ms at 12 with one warp per env).
+  // + render per 4096 envs: 3: 5.33 ms, 4: 4.66 ms, 5: 4.46 ms, and 5.6 ms at 12 with one warp per env).
   // In that regime the SMs have registers to spare, and every env gets a helper warp that
   // computes one of the two directions of _get_collision_vectors (MOOG_HELPER=0/1 overrides).
   int resident = 0;

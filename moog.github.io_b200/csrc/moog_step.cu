@@ -28,6 +28,7 @@
 #include <stdlib.h>
 
 #include "moog_common.cuh"
+#include "moog_dcv_argmin.cuh"
 #include "moog_render_dev.cuh"
 
 namespace moog {
@@ -59,7 +60,7 @@ namespace moog {
 enum { KIND_WEAK = 0, KIND_F32 = 1, KIND_F64 = 2 };
 
 struct SmemLayout {
-  int rec, dyn, stat, aabb, aabb0, nskin, tmp, vtx, envf, ctr, meta, sflag, voff, cnt, envi, cmoff, cmask, nearp, hdr, scratch, xchg, mbar, plist, kscr, kscr_bytes, tile, vmap, total;
+  int rec, dyn, stat, aabb, aabb0, nskin, tmp, vtx, envf, ctr, meta, sflag, voff, cnt, envi, cmoff, cmask, nearp, hdr, scratch, xchg, mbar, plist, win_a, win_e, tile, vmap, total;
 };
 
 #define MOOG_MAX_FORCE_OPS 32
@@ -84,7 +85,6 @@ __host__ __device__ inline SmemLayout smem_layout(int S, int VT, int NF, int CMW
   L.stat = o;  o += 8 * MOOG_STAT_FIELDS * S;
   L.aabb = o;  o += 8 * 4 * S;
   L.vtx = o;   o += 16 * VT;     // 16-byte aligned: everything before it is a multiple of 16
-  L.tmp = -1;  // tether scratch (3 fields) / per-slot translations of the Euler pass: placed below
   L.envf = o;  o += 8 * NF;
   L.ctr = o;   o += 8 * 12;
   L.meta = o;  o += 4 * MOOG_META_FIELDS * S;
@@ -104,17 +104,11 @@ __host__ __device__ inline SmemLayout smem_layout(int S, int VT, int NF, int CMW
   L.mbar = o;  o += 16;                   // mbarrier of the bulk (TMA) loads of the record
   L.tile = tile;
   L.plist = o; o += CMW > 0 ? 2 * 32 * tile * warps : 8;  // crossing (vertex, edge) pairs, per warp
-  L.kscr_bytes = CMW > 0 ? 8 * 32 * tile : 8;
-  L.kscr = o;  o += L.kscr_bytes * warps;
-  // the tether / Euler-pass scratch is never live together with a directed search: it shares the
-  // owner's key tile when it fits there
-  if (8 * 3 * S <= L.kscr_bytes) {
-    L.tmp = L.kscr;
-  } else {
-    o = (o + 15) & ~15;
-    L.tmp = o;
-    o += 8 * 3 * S;
-  }
+  o = (o + 15) & ~15;
+  // per warp, the directed search's winner of each contained vertex (up to 32): its edge's cross_a and the edge
+  L.win_a = o; o += CMW > 0 ? 8 * 32 * warps : 0;
+  L.win_e = o; o += CMW > 0 ? 32 * warps : 0;
+  L.tmp = o;   o += 8 * 3 * S;  // (16-byte aligned) tether scratch (3 fields) / per-slot translations of the Euler pass
   L.vmap = o;  o += VT;  // cached vertex -> slot (integrate_all)
   L.total = (o + 15) & ~15;
   return L;
@@ -147,7 +141,8 @@ struct Env {
   int *meta, *sflag, *voff, *cnt, *envi, *cmoff;
   unsigned *cmask, *nearp;
   unsigned char *scratch;
-  unsigned long long *kscr;
+  double *win_a;
+  unsigned char *win_e;
   unsigned char *xchg;
   unsigned short *plist;
   int dcv_tile;
@@ -213,7 +208,8 @@ __device__ __forceinline__ Env env_view() {
   e.hdr = (const int32_t *)(base + r->lay.hdr);
   const int warp = threadIdx.x >> 5;
   e.scratch = base + r->lay.scratch + 64 * warp;
-  e.kscr = (unsigned long long *)(base + r->lay.kscr + r->lay.kscr_bytes * warp);
+  e.win_a = (double *)(base + r->lay.win_a) + 32 * warp;
+  e.win_e = base + r->lay.win_e + 32 * warp;
   e.xchg = base + r->lay.xchg;
   e.plist = (unsigned short *)(base + r->lay.plist) + 32 * r->lay.tile * warp;
   e.dcv_tile = r->lay.tile;
@@ -851,18 +847,16 @@ __device__ __forceinline__ void directed_collision_vectors_impl(const Env &e, in
   double2 q2 = P1[eact ? ((ej + 1 == n1) ? 0 : ej + 1) : 0];
   double d1x = q2.x - q1.x, d1y = q2.y - q1.y;
 
-  // Stage A (lane = (vertex, edge of s1); no cross-lane traffic, so consecutive
-  // passes overlap in the pipeline): the argmin key of every (vertex, edge) goes
-  // to a shared-memory tile.
-  // Stage B (lane = vertex): each lane scans its row of the tile for np.argmin
-  // (first index on ties), recomputes the winning edge's coefficient -- the same
-  // IEEE operations, hence the same bits -- and the penetration length.
+  // Stage A1 (lane = (vertex, edge of s1); no cross-lane traffic but the compaction, so
+  // consecutive trips overlap in the pipeline): the crossing pairs go to a list.
+  // Stage A2 (lane = crossing pair): cross_a and its np.argmin key, in registers.
+  // Stage B: np.argmin per vertex (first edge on ties) by a segmented scan over the pair lanes;
+  // lane = vertex gets the winning edge and its cross_a from A2, and the penetration length.
   // Stage C: np.argmax over the vertices by two warp maxima.
   bool my_cross = false;
   bool have = false;
   double b_dist = 0, b_cpx = 0, b_cpy = 0, b_dfx = 0, b_dfy = 0, b_a = 0;
   int b_edge = 0;
-  unsigned long long *keys = e.kscr;
   // contained vertex indices, ascending, in the scratch bytes
   const int n_in = __popc(mask);
   wsync();
@@ -876,12 +870,14 @@ __device__ __forceinline__ void directed_collision_vectors_impl(const Env &e, in
     const int cnt = min(TILE, n_in - vbase);
 #ifdef MOOG_PROFILE_DCV
     long long tp1 = clock64();
+    long long tb = 0;
 #endif
     // Stage A1 (no division): which (vertex, edge) pairs cross, i.e. 0 <= cross_b <= 1
     // (sprite.py:171-175).  A line meets a convex outline in two edges, so only a couple
-    // of pairs per vertex do; they are compacted into a list, every other pair's key is
-    // |1 - (-inf)| = +inf.  Two passes per iteration for instruction-level parallelism.
-    const unsigned long long KEY_INF = (unsigned long long)__double_as_longlong(INFINITY) + 1ull;
+    // of pairs per vertex do; they are compacted into a list in ascending (vertex, edge)
+    // order (ballots in lane order, later trips hold later vertices), so the pairs of one
+    // vertex are one contiguous segment of it.  Every other pair's key is |1 - (-inf)| = +inf.
+    // Two passes per iteration for instruction-level parallelism.
     const unsigned lt = (1u << e.lane) - 1u;
     int n_pairs = 0;
     for (int t0 = 0; t0 < cnt; t0 += DCV_U * V) {
@@ -908,7 +904,6 @@ __device__ __forceinline__ void directed_collision_vectors_impl(const Env &e, in
         inexact |= !exact;
         cr[u] = on && in_unit;
         nB2[u] = nB; den2[u] = den; on2[u] = on;
-        if (on) keys[t * 32 + ej] = KEY_INF;
       }
       if (__any_sync(FULL, inexact)) {  // out-of-range operands somewhere in the warp: divide
 #pragma unroll
@@ -925,10 +920,16 @@ __device__ __forceinline__ void directed_collision_vectors_impl(const Env &e, in
       }
     }
     my_cross |= n_pairs > 0;
+    // a vertex without a crossing pair: np.argmin of an all-inf row is edge 0, whose cross_a is -inf
+    if (e.lane < cnt) { e.win_a[e.lane] = -INFINITY; e.win_e[e.lane] = 0; }
     wsync();
-    // Stage A2: cross_a of the crossing pairs, 32 pairs per pass -- the same IEEE operations
-    // on the same operands as above and as the reference, hence the same bits
+    // Stages A2 + B, 32 pairs per pass.  A pass ends after 32 pairs wherever that is, so the
+    // running winner of its last vertex is carried into the next pass, where that vertex's
+    // segment may go on.
+    DcvCarry carry;
     for (int base = 0; base < n_pairs; base += 32) {
+      // Stage A2: cross_a of the crossing pairs -- the same IEEE operations on the same operands
+      // as above and as the reference, hence the same bits
       const int k = base + e.lane;
       const bool act2 = k < n_pairs;
       const unsigned ent = e.plist[act2 ? k : 0];
@@ -942,57 +943,37 @@ __device__ __forceinline__ void directed_collision_vectors_impl(const Env &e, in
       const double e1x = w2.x - w1.x, e1y = w2.y - w1.y;
       const double den = act2 ? (d0x * e1y - d0y * e1x) + EPS_INTERP : 1.0;
       const double qx = w1.x - sx, qy = w1.y - sy;
+#ifdef MOOG_PROFILE_DCV
+      const double A = shfl_d((act2 ? (qx * e1y - qy * e1x) : 1.0) / den, e.lane);  // waits for A2: the clock splits A2 from B
+      const long long tb0 = clock64();
+#else
       const double A = (act2 ? (qx * e1y - qy * e1x) : 1.0) / den;
-      const double ab = fabs(1.0 - A);
-      // np.argmin order: a NaN beats everything, then the smaller value (ab >= 0, so
-      // its bit pattern orders like the value), then the smaller index
-      if (act2) keys[t * 32 + ed] = isnan(ab) ? 0ull : (unsigned long long)__double_as_longlong(ab) + 1ull;
+#endif
+      // Stage B (moog_dcv_argmin.cuh)
+      const int t_after = base + 32 < n_pairs ? (int)(e.plist[base + 32] >> 8) : 255;  // first vertex of the next pass
+      int w_ed;
+      double w_a;
+      if (dcv_argmin_pass(act2, t, ed, A, t_after, e.lane, carry, w_ed, w_a)) {
+        e.win_a[t] = w_a;
+        e.win_e[t] = (unsigned char)w_ed;
+      }
+#ifdef MOOG_PROFILE_DCV
+      tb += clock64() - tb0;
+#endif
     }
     wsync();
 #ifdef MOOG_PROFILE_DCV
     long long tp2 = clock64();
-    ctr_add(e, CT_CYC_NARROW, tp2 - tp1);
+    ctr_add(e, CT_CYC_NARROW, tp2 - tp1 - tb);
 #endif
-    // stage B (lane = edge of s1): np.argmin of every vertex's row of keys by two warp
-    // minima (high word, then low word among the lanes that hold the minimum high word) and
-    // the first such lane; the rows are independent, so the reductions pipeline.  Lane v
-    // keeps the winner of vertex v.
     const bool vact = e.lane < cnt;
-    int idx = 0;
+    const int idx = e.win_e[vact ? e.lane : 0];
+    double A = e.win_a[vact ? e.lane : 0], cpx = 0, cpy = 0, dfx = 0, dfy = 0, dist = 0;
     {
-      const bool kact = e.lane < n1;
-#pragma unroll 1
-      for (int v = 0; v < cnt; ++v) {
-        const unsigned long long k = kact ? keys[v * 32 + e.lane] : ~0ull;
-        const unsigned hi = (unsigned)(k >> 32), lo = (unsigned)k;
-        const unsigned mhi = __reduce_min_sync(FULL, hi);
-        const bool th = kact && hi == mhi;
-        const unsigned mlo = __reduce_min_sync(FULL, th ? lo : 0xffffffffu);
-        const int win = __ffs(__ballot_sync(FULL, th && lo == mlo)) - 1;
-        if (e.lane == v) idx = win;
-      }
-    }
-    double A = 0, cpx = 0, cpy = 0, dfx = 0, dfy = 0, dist = 0;
-    {
-      // the winning edge's coefficient again -- the same IEEE operations, hence the same bits
       const double2 ev = P0[e.scratch[vbase + (vact ? e.lane : 0)]];
       const double ex = ev.x, ey = ev.y;
       const double sx = M.m0 * ex + M.m1 * ey + M.m2;
       const double sy = M.m3 * ex + M.m4 * ey + M.m5;
-      const double d0x = ex - sx, d0y = ey - sy;
-      const double2 w1 = P1[idx], w2 = P1[(idx + 1 == n1) ? 0 : idx + 1];
-      const double e1x = w2.x - w1.x, e1y = w2.y - w1.y;
-      const double den = vact ? (d0x * e1y - d0y * e1x) + EPS_INTERP : 1.0;
-      const double qx = w1.x - sx, qy = w1.y - sy;
-      const double nB = vact ? (qx * d0y - qy * d0x) : 1.0;
-      bool exact;
-      bool in_unit = unit_ratio(nB, den, exact);
-      if (__any_sync(FULL, !exact)) {
-        const double Bc = nB / den;
-        in_unit = (Bc >= 0) && (Bc <= 1);
-      }
-      A = (vact ? (qx * e1y - qy * e1x) : 1.0) / den;
-      if (!in_unit) A = -INFINITY;
       cpx = sx + A * (ex - sx);
       cpy = sy + A * (ey - sy);
       dfx = ex - cpx;
@@ -1019,7 +1000,7 @@ __device__ __forceinline__ void directed_collision_vectors_impl(const Env &e, in
     }
     wsync();
 #ifdef MOOG_PROFILE_DCV
-    ctr_add(e, CT_CYC_RESOLVE, clock64() - tp2);
+    ctr_add(e, CT_CYC_RESOLVE, clock64() - tp2 + tb);
 #endif
   }
   const bool any_cross = __any_sync(FULL, my_cross) != 0;
