@@ -135,6 +135,16 @@ int moog_render(moog_program *p, const moog_state *st, int n_envs, uint8_t *fram
  * outside [0, 1 + hdr[MOOG_H_N_VIEWS]). */
 int moog_render_view(moog_program *p, const moog_state *st, int n_envs, int view, uint8_t *frames, void *stream);
 
+/* How the render kernel draws view `view` of a program blob, without touching the GPU (like
+ * moog_program_validate, which it runs first).  The canvas (anti_aliasing x the image size) is drawn
+ * *chunk_rows rows at a time: the whole canvas, a band (anti_aliasing 1) or a chunk streamed through
+ * the Lanczos resize (anti_aliasing > 1); *smem_bytes of shared memory per env.  Either pointer may
+ * be NULL.  0; MOOG_E_INVAL for a malformed blob, a program without a renderer or a view outside
+ * [0, 1 + hdr[MOOG_H_N_VIEWS]); MOOG_E_UNSUPPORTED for a view no chunk size can hold in one CTA's
+ * shared memory (moog_render, moog_render_view and moog_env_step with io.frames refuse it the same way,
+ * before launching anything). */
+int moog_render_plan(const void *blob, size_t nbytes, int view, int *chunk_rows, int *smem_bytes);
+
 /* RawState.__call__ (moog/observers/raw_state.py:17-19) for N envs: every sprite slot's state as
  * out[N][S][MOOG_OBS_COLS] float32 (layout and columns: moog_b200_program.h MOOG_OBS_*).  A launch of its
  * own on `stream`, so call it after moog_env_step to observe the state that call left.  `out` is any

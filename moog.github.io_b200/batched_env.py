@@ -139,6 +139,7 @@ class Engine(object):
             raise capi.MoogError('device must be a CUDA device')
         self.n = int(num_envs)
         self.seed = int(seed)
+        self._check_views(program)
         with torch.cuda.device(self.device):
             self.dev_program = capi.DeviceProgram(program.blob)
         self.dev_program.set_option('seed', self.seed & 0x7fffffff)
@@ -164,6 +165,22 @@ class Engine(object):
         self._pinned_ok = set()
 
     # -- helpers -----------------------------------------------------------
+    @staticmethod
+    def _check_views(program):
+        """Every renderer must be drawable by the render kernel (moog_render_plan): a view that no
+        chunk of its canvas fits one CTA's shared memory is refused here, before anything is
+        allocated or launched."""
+        views = list(getattr(program, 'views', ())) or (
+            [('image', program.render)] if program.render is not None else [])
+        for v, (key, r) in enumerate(views):
+            code, _, _ = capi.render_plan(program.blob, v)
+            if code == capi.E_UNSUPPORTED:
+                raise capi.MoogError(
+                    'observer {!r}: PILRenderer(image_size=({}, {}), anti_aliasing={}) draws a {} x {} canvas, '
+                    'and no chunk of it fits the shared memory of one CTA'.format(
+                        key, r['width'], r['height'], r['aa'], r['aa'] * r['width'], r['aa'] * r['height']))
+            capi.check(code)
+
     def call_seed(self):
         """io.seed of the next env_step call (a different Philox key every call)."""
         return (self.seed * 0x9E3779B97F4A7C15 + self._calls) & 0xFFFFFFFFFFFFFFFF

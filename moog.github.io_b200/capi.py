@@ -41,7 +41,12 @@ SYMBOLS = ('moog_program_create', 'moog_program_destroy',
            'moog_launch_count', 'moog_host_paths_overlap',
            'moog_host_points_in_path', 'moog_step_launch_info',
            'moog_step_draws_frames', 'moog_program_set_option',
-           'moog_program_validate', 'moog_observe_sprites', 'moog_render_view')
+           'moog_program_validate', 'moog_observe_sprites', 'moog_render_view',
+           'moog_render_plan')
+
+
+# include/moog_b200.h return codes
+E_INVAL, E_CUDA, E_TOO_BIG, E_UNSUPPORTED = -1, -2, -3, -4
 
 
 class MoogError(RuntimeError):
@@ -105,6 +110,8 @@ def lib():
     L.moog_program_set_option.restype = ci
     L.moog_program_validate.argtypes = [vp, ctypes.c_size_t]
     L.moog_program_validate.restype = ci
+    L.moog_render_plan.argtypes = [vp, ctypes.c_size_t, ci, ctypes.POINTER(ci), ctypes.POINTER(ci)]
+    L.moog_render_plan.restype = ci
     L.moog_launch_count.argtypes = []
     L.moog_launch_count.restype = ctypes.c_int64
     _lib = L
@@ -115,13 +122,23 @@ def check(code):
     if code != 0:
         L = lib()
         msg = L.moog_strerror(code).decode()
-        if code == -2:
+        if code == E_CUDA:
             msg += ': ' + L.moog_last_cuda_error().decode()
         raise MoogError('libmoog_b200: {} ({})'.format(msg, code))
 
 
 def launch_count():
     return int(lib().moog_launch_count())
+
+
+def render_plan(blob, view=0):
+    """How the render kernel draws view `view` of a program blob, without a device
+    (include/moog_b200.h moog_render_plan): (code, chunk_rows, smem_bytes); code 0, or
+    E_UNSUPPORTED for a view no chunk size can hold, or E_INVAL."""
+    buf = ctypes.create_string_buffer(bytes(blob), len(blob))
+    rows, smem = ctypes.c_int(), ctypes.c_int()
+    code = int(lib().moog_render_plan(buf, len(blob), int(view), ctypes.byref(rows), ctypes.byref(smem)))
+    return code, rows.value, smem.value
 
 
 class DeviceProgram(object):

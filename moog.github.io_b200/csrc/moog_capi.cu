@@ -26,6 +26,7 @@ struct moog_program {
   int view_off[MOOG_MAX_VIEWS];
   // anti_aliasing > 1: Lanczos coefficient tables (Resample.c) per view, built on first use
   int *resample[MOOG_MAX_VIEWS];
+  moog::RenderPlan plan[MOOG_MAX_VIEWS];  // how the render kernels draw each view (render_plan)
   int ksize_h[MOOG_MAX_VIEWS], ksize_v[MOOG_MAX_VIEWS];
   // largest outline a slot of each layer can hold (from the blob's voff table)
   int layer_vcap[MOOG_MAX_LAYERS];
@@ -279,6 +280,20 @@ int moog_program_validate(const void *blob, size_t nbytes) {
   return 0;
 }
 
+int moog_render_plan(const void *blob, size_t nbytes, int view, int *chunk_rows, int *smem_bytes) {
+  const int bad = moog_program_validate(blob, nbytes);
+  if (bad) return bad;
+  const int32_t *hdr = (const int32_t *)blob;
+  if (!hdr[MOOG_H_R_ENABLED] || view < 0 || view > hdr[MOOG_H_N_VIEWS]) return MOOG_E_INVAL;
+  const int32_t *v = view == 0 ? hdr + MOOG_H_R_HEIGHT
+                               : moog::view_of(blob).ipool + hdr[MOOG_H_VIEWS] + MOOG_VIEW_WORDS * (view - 1);
+  const moog::RenderPlan plan = moog::render_plan(hdr, v);
+  if (!plan.ok) return MOOG_E_UNSUPPORTED;
+  if (chunk_rows) *chunk_rows = plan.rows;
+  if (smem_bytes) *smem_bytes = plan.env_bytes;
+  return 0;
+}
+
 int moog_program_create(const void *blob, size_t nbytes, moog_program **out) {
   if (!out) return MOOG_E_INVAL;
   const int bad = moog_program_validate(blob, nbytes);
@@ -302,6 +317,7 @@ int moog_program_create(const void *blob, size_t nbytes, moog_program **out) {
         const int32_t *v = k == 0 ? hdr + MOOG_H_R_HEIGHT : pv.ipool + hdr[MOOG_H_VIEWS] + MOOG_VIEW_WORDS * (k - 1);
         memcpy(p->view[k], v, sizeof(p->view[k]));
         p->view_off[k] = (int)(v - hdr);
+        p->plan[k] = moog::render_plan(p->hdr, p->view[k]);
       }
     }
   }
@@ -464,6 +480,8 @@ static int run_step(moog_program *p, const moog_state *st, int n_envs, int mode,
   bool fused = false;
   if (a.io.frames && (mode != moog::MODE_ENV_STEP || !p->hdr[MOOG_H_R_ENABLED] || p->hdr[MOOG_H_R_AA] < 1))
     return MOOG_E_INVAL;
+  // a view no chunk size can hold is refused before anything is launched
+  if (a.io.frames && !p->plan[0].ok) return MOOG_E_UNSUPPORTED;
   const int fmode = a.io.frames ? frames_mode(n_envs) : 0;
   // Frames of a large batch: the step ends when its longest-running env does, and long before
   // that most SMs have no env left to step.  The render kernel is launched behind the step kernel
@@ -545,7 +563,7 @@ static int render_impl(moog_program *p, const moog_state *st, int n_envs, int vi
   if (!p || !valid_state(st) || !frames || n_envs < 0) return MOOG_E_INVAL;
   if (!p->hdr[MOOG_H_R_ENABLED]) return MOOG_E_INVAL;
   const int32_t *v = p->view[view];
-  if (v[MOOG_V_AA] < 1) return MOOG_E_UNSUPPORTED;
+  if (v[MOOG_V_AA] < 1 || !p->plan[view].ok) return MOOG_E_UNSUPPORTED;
   moog::RenderArgs a;
   memset(&a, 0, sizeof(a));
   a.blob = p->dev_blob;
@@ -574,7 +592,7 @@ static int render_impl(moog_program *p, const moog_state *st, int n_envs, int vi
   }
   int launches = 0;
   cudaError_t err =
-      moog::launch_render(a, p->hdr, v, (cudaStream_t)stream, &launches, done, n_envs, tail_mode, p->opt);
+      moog::launch_render(a, p->plan[view], v, (cudaStream_t)stream, &launches, done, n_envs, tail_mode, p->opt);
   g_launches += launches;
   return err == cudaSuccess ? 0 : cuda_fail(err);
 }

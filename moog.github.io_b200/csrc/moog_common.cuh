@@ -111,11 +111,20 @@ cudaError_t launch_step(const StepArgs &a, const int32_t *host_hdr, cudaStream_t
                         int frames_mode = 0, bool *fused = nullptr, const LaunchOptions &opt = LaunchOptions());
 cudaError_t launch_order(const int *cost, int *order, int n, cudaStream_t stream, int *n_launches);
 int resample_tables(int H, int W, int OH, int OW, std::vector<int> &table, int *ksize_h, int *ksize_v);
+int lanczos_ksize(int in_size, int out_size);
+// How the render kernels draw a view (the one place that decides it; moog_render_plan exposes it).
+// rows: canvas rows drawn at once -- the whole canvas, a band (anti_aliasing 1) or a chunk
+// (anti_aliasing > 1, streamed through the Lanczos resize); ring: rows of the horizontally resampled
+// ring (anti_aliasing > 1); P threads per canvas row, T per env; env_bytes: shared memory per env.
+// ok == false: no band / chunk fits one CTA's shared memory.
+struct RenderPlan { bool ok; int rows, ring, P, T, env_bytes; };
+RenderPlan render_plan(const int32_t *host_hdr, const int32_t *host_view);
 // done: nullptr, or the finished-env list of the step kernel launched just before on `stream`
 // (StepArgs::done): the render kernel is then launched with programmatic stream serialization,
 // starts while the last envs are still being stepped and draws the envs in finishing order.
-// host_view: the host copy of the words at a.view_off (the view's settings)
-cudaError_t launch_render(const RenderArgs &a, const int32_t *host_hdr, const int32_t *host_view, cudaStream_t stream,
+// plan: render_plan of the view (the program keeps one per view); host_view: the host copy of the
+// words at a.view_off (the view's settings)
+cudaError_t launch_render(const RenderArgs &a, const RenderPlan &plan, const int32_t *host_view, cudaStream_t stream,
                           int *n_launches, int *done = nullptr, int n_done = 0, int tail_mode = 1,
                           const LaunchOptions &opt = LaunchOptions());
 // moog_observe_sprites (moog_observe.cu): one warp per env

@@ -20,31 +20,47 @@
 
 namespace moog {
 
-// blockDim.x = envs_per_block * T, T = threads of one env (>= H, multiple of 32)
-__global__ void moog_render_kernel(RenderArgs a, int T, int envs_per_block, int P, int band) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  ProgramView pv = view_of(a.blob);
-  const int32_t *hdr = pv.hdr;
-  const int32_t *view = hdr + a.view_off;
-  const int S = hdr[MOOG_H_N_SLOTS], VT = hdr[MOOG_H_N_VTX];
-  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
-  const int g = threadIdx.x / T, t = threadIdx.x - g * T;
-  const int n = blockIdx.x * envs_per_block + g;
-  const bool live = n < a.n_envs;
-  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
-  const RenderLayout lay = render_layout(band > 0 ? band : aa * OH, aa * OW, S * C, (VT > 0 ? VT : 1) * C, OW);
-  const size_t row = live ? (size_t)n : 0;
+// One env's frame: render_env (anti_aliasing 1, `rows` rows per band) or render_env_aa (chunks of
+// `rows` canvas rows, a ring of `ring` resampled rows), as render_plan chose for the view.
+template <bool AA>
+__device__ __forceinline__ void draw_env(const RenderArgs &a, const RenderSrc &src, unsigned char *base, int t, int T,
+                                         int P, bool live, uint8_t *out, int rows, int ring) {
+  const RenderLayout lay = view_layout(src.hdr, src.view, rows, AA ? ring : 0);
+  if (AA)
+    render_env_aa(src, lay, base, nullptr, t, T, P, live, out, a.resample, a.ksize_h, a.ksize_v,
+                  [] { __syncthreads(); }, rows, ring);
+  else
+    render_env(src, lay, base, nullptr, t, T, P, live, out, [] { __syncthreads(); }, rows);
+}
+
+__device__ __forceinline__ RenderSrc env_src(const RenderArgs &a, const ProgramView &pv, const int32_t *view, size_t row) {
+  const int S = pv.hdr[MOOG_H_N_SLOTS], VT = pv.hdr[MOOG_H_N_VTX];
   RenderSrc src;
   src.dyn = a.st.dyn + row * MOOG_DYN_FIELDS * S;
   src.stat = a.st.stat + row * MOOG_STAT_FIELDS * S;
   src.meta = a.st.meta + row * MOOG_META_FIELDS * S;
   src.cnt = a.st.cnt + row * MOOG_MAX_LAYERS;
   src.vtx = (const double2 *)(a.st.vtx + row * 2 * VT);
-  src.hdr = hdr;
+  src.hdr = pv.hdr;
   src.voff = pv.voff;
   src.view = view;
-  render_env(src, lay, smem_raw + (size_t)g * lay.total, nullptr, t, T, P, live,
-             a.frames + row * OH * OW * 3, a.resample, a.ksize_h, a.ksize_v, [] { __syncthreads(); }, band);
+  return src;
+}
+
+// blockDim.x = envs_per_block * T, T = threads of one env (render_plan)
+template <bool AA>
+__global__ void moog_render_kernel(RenderArgs a, int T, int envs_per_block, int P, int rows, int ring) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  ProgramView pv = view_of(a.blob);
+  const int32_t *view = pv.hdr + a.view_off;
+  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH];
+  const int g = threadIdx.x / T, t = threadIdx.x - g * T;
+  const int n = blockIdx.x * envs_per_block + g;
+  const bool live = n < a.n_envs;
+  const size_t row = live ? (size_t)n : 0;
+  const RenderSrc src = env_src(a, pv, view, row);
+  const int env_bytes = view_layout(pv.hdr, view, rows, AA ? ring : 0).total;
+  draw_env<AA>(a, src, smem_raw + (size_t)g * env_bytes, t, T, P, live, a.frames + row * OH * OW * 3, rows, ring);
 }
 
 // The same for the envs of a step kernel that is still running (launched behind it with
@@ -53,7 +69,8 @@ __global__ void moog_render_kernel(RenderArgs a, int T, int envs_per_block, int 
 // thread 0 waits for entry b of the step kernel's finished list (acquire; the step kernel releases
 // it after the env's record is in HBM).  Every env it could wait for is running or done, so the
 // wait is bounded by the step itself; the poll limit only turns a broken launch into an error.
-__global__ void moog_render_tail_kernel(RenderArgs a, int T, int P, const int *done, int band) {
+template <bool AA>
+__global__ void moog_render_tail_kernel(RenderArgs a, int T, int P, const int *done, int rows, int ring) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ int s_env;
   if (threadIdx.x == 0) {
@@ -69,26 +86,13 @@ __global__ void moog_render_tail_kernel(RenderArgs a, int T, int P, const int *d
   __syncthreads();
   const int n = s_env;
   ProgramView pv = view_of(a.blob);
-  const int32_t *hdr = pv.hdr;
-  const int32_t *view = hdr + a.view_off;
-  const int S = hdr[MOOG_H_N_SLOTS], VT = hdr[MOOG_H_N_VTX];
-  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
-  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
-  const RenderLayout lay = render_layout(band > 0 ? band : aa * OH, aa * OW, S * C, (VT > 0 ? VT : 1) * C, OW);
+  const int32_t *view = pv.hdr + a.view_off;
+  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH];
   const size_t row = (size_t)n;
-  RenderSrc src;
-  src.dyn = a.st.dyn + row * MOOG_DYN_FIELDS * S;
-  src.stat = a.st.stat + row * MOOG_STAT_FIELDS * S;
-  src.meta = a.st.meta + row * MOOG_META_FIELDS * S;
-  src.cnt = a.st.cnt + row * MOOG_MAX_LAYERS;
-  src.vtx = (const double2 *)(a.st.vtx + row * 2 * VT);
-  src.hdr = hdr;
-  src.voff = pv.voff;
-  src.view = view;
+  const RenderSrc src = env_src(a, pv, view, row);
   unsigned long long tr0 = 0;
   if (a.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tr0));
-  render_env(src, lay, smem_raw, nullptr, (int)threadIdx.x, T, P, true, a.frames + row * OH * OW * 3, a.resample,
-             a.ksize_h, a.ksize_v, [] { __syncthreads(); }, band);
+  draw_env<AA>(a, src, smem_raw, (int)threadIdx.x, T, P, true, a.frames + row * OH * OW * 3, rows, ring);
   if (a.trace && threadIdx.x == 0) {
     unsigned long long tr1;
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tr1));
@@ -104,8 +108,9 @@ __global__ void moog_render_tail_kernel(RenderArgs a, int T, int P, const int *d
 // CTA takes none while its own SM is still stepping envs (sm_active, kept by the step kernel) -- a
 // renderer next to a long-running env slows down exactly the env the whole step is waiting for.
 // The frames are drawn on the SMs the step has left, the last env's by whichever CTA is free.
+template <bool AA>
 __global__ void moog_render_tail_persistent_kernel(RenderArgs a, int T, int P, int *done, int n_done, int busy_thr,
-                                                   int band) {
+                                                   int rows, int ring) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ int s_env;
   int *ticket = done + 1 + n_done;
@@ -113,12 +118,8 @@ __global__ void moog_render_tail_persistent_kernel(RenderArgs a, int T, int P, i
   unsigned smid;
   asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
   ProgramView pv = view_of(a.blob);
-  const int32_t *hdr = pv.hdr;
-  const int32_t *view = hdr + a.view_off;
-  const int S = hdr[MOOG_H_N_SLOTS], VT = hdr[MOOG_H_N_VTX];
-  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
-  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
-  const RenderLayout lay = render_layout(band > 0 ? band : aa * OH, aa * OW, S * C, (VT > 0 ? VT : 1) * C, OW);
+  const int32_t *view = pv.hdr + a.view_off;
+  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH];
   bool last = false;
   for (;;) {
     if (threadIdx.x == 0) {
@@ -151,19 +152,10 @@ __global__ void moog_render_tail_persistent_kernel(RenderArgs a, int T, int P, i
     last = last || (n & 0x40000000) != 0;
     n &= 0x3fffffff;
     const size_t row = (size_t)n;
-    RenderSrc src;
-    src.dyn = a.st.dyn + row * MOOG_DYN_FIELDS * S;
-    src.stat = a.st.stat + row * MOOG_STAT_FIELDS * S;
-    src.meta = a.st.meta + row * MOOG_META_FIELDS * S;
-    src.cnt = a.st.cnt + row * MOOG_MAX_LAYERS;
-    src.vtx = (const double2 *)(a.st.vtx + row * 2 * VT);
-    src.hdr = hdr;
-    src.voff = pv.voff;
-    src.view = view;
+    const RenderSrc src = env_src(a, pv, view, row);
     unsigned long long tr0 = 0;
     if (a.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tr0));
-    render_env(src, lay, smem_raw, nullptr, (int)threadIdx.x, T, P, true, a.frames + row * OH * OW * 3, a.resample,
-               a.ksize_h, a.ksize_v, [] { __syncthreads(); }, band);
+    draw_env<AA>(a, src, smem_raw, (int)threadIdx.x, T, P, true, a.frames + row * OH * OW * 3, rows, ring);
     __syncthreads();
     if (a.trace && threadIdx.x == 0) {
       unsigned long long tr1;
@@ -191,10 +183,16 @@ static double lanczos_weight(double x) {
   return sinc(x) * sinc(x / 3);
 }
 
+// Resample.c precompute_coeffs: taps per output pixel, the longest window an output pixel reads
+int lanczos_ksize(int in_size, int out_size) {
+  double scale = (double)in_size / out_size, filterscale = scale < 1.0 ? 1.0 : scale;
+  return (int)ceil(3.0 * filterscale) * 2 + 1;
+}
+
 static int resample_axis(int in_size, int out_size, std::vector<int> &bounds, std::vector<int> &coeffs) {
   double scale = (double)in_size / out_size, filterscale = scale < 1.0 ? 1.0 : scale;
   double support = 3.0 * filterscale;
-  int ksize = (int)ceil(support) * 2 + 1;
+  int ksize = lanczos_ksize(in_size, out_size);
   bounds.assign(2 * (size_t)out_size, 0);
   coeffs.assign((size_t)out_size * ksize, 0);
   std::vector<double> k(ksize);
@@ -231,62 +229,93 @@ int resample_tables(int H, int W, int OH, int OW, std::vector<int> &table, int *
   return (int)table.size();
 }
 
-cudaError_t launch_render(const RenderArgs &a, const int32_t *hdr, const int32_t *view, cudaStream_t stream,
-                          int *n_launches, int *done, int n_done, int tail_mode, const LaunchOptions &opt) {
-  if (a.n_envs <= 0) return cudaSuccess;
+// How a view is drawn (see RenderPlan in moog_common.cuh).  anti_aliasing 1: a canvas that does not
+// fit next to the edge lists in one CTA's shared memory is drawn in bands: the largest band, a
+// multiple of 8 rows, whose layout leaves room for two CTAs per SM.  anti_aliasing > 1: the largest
+// chunk (at most 512 rows) whose canvas, edge lists and ring of chunk + ksize_v resampled rows
+// leave room for two CTAs per SM, else the largest that fits one CTA; then the chunks are evened out.
+RenderPlan render_plan(const int32_t *hdr, const int32_t *view) {
+  RenderPlan p;
+  memset(&p, 0, sizeof(p));
   const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
-  const int H = aa * OH, W = aa * OW, S = hdr[MOOG_H_N_SLOTS], VT = hdr[MOOG_H_N_VTX];
-  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;  // TorusGeometry: 9 copies per sprite
-  // A canvas that does not fit next to the edge lists in one CTA's shared memory is drawn in bands
-  // of `band` rows (render_env): the largest band, a multiple of 8 rows, whose layout leaves room
-  // for two CTAs per SM.  Anti-aliased canvases are not banded (the Lanczos resize reads across rows).
-  int band = 0;
-  if (aa == 1 && render_layout(H, W, S * C, (VT > 0 ? VT : 1) * C, OW).total > 110 * 1024) {
-    band = H & ~7;
-    while (band > 8 && render_layout(band, W, S * C, (VT > 0 ? VT : 1) * C, OW).total > 110 * 1024) band -= 8;
+  if (OH < 1 || OW < 1 || aa < 1 || OH > 8192 || OW > 8192 || aa > 16) return p;
+  const int H = aa * OH, W = aa * OW;
+  const int kBudget2 = 110 * 1024, kBudget1 = 224 * 1024;
+  if (4LL * (W + 1) > kBudget1) return p;  // not even one canvas row fits
+  if (aa == 1) {
+    int band = 0;
+    if (view_layout(hdr, view, H, 0).total > kBudget2) {
+      band = H & ~7;
+      while (band > 8 && view_layout(hdr, view, band, 0).total > kBudget2) band -= 8;
+    }
+    p.rows = band > 0 ? band : H;
+    p.P = (p.rows <= 128) ? 2 : 1;  // threads per canvas row (they split its columns)
+  } else {
+    const int ks = lanczos_ksize(H, OH);
+    for (int budget : {kBudget2, kBudget1}) {
+      for (int hc = H < 512 ? H : 512; hc >= 1 && p.rows == 0; --hc) {
+        const int ring = hc + ks < H ? hc + ks : H;
+        if (view_layout(hdr, view, hc, ring).total <= budget) {
+          p.rows = hc;
+          p.ring = ring;
+        }
+      }
+      if (p.rows > 0) break;
+    }
+    if (p.rows == 0) return p;
+    if (p.rows < H) {  // the same number of chunks, of even height: no short last chunk
+      const int n = (H + p.rows - 1) / p.rows;
+      p.rows = (H + n - 1) / n;
+      p.ring = p.rows + ks < H ? p.rows + ks : H;
+    }
+    p.P = p.rows <= 128 ? 2 : 1;
+    if (p.rows * p.P < 256) p.P = 256 / p.rows;  // short chunks: more threads share a row
+    if (p.P > W / 16) p.P = W / 16 > 1 ? W / 16 : 1;
   }
-  const int HB = band > 0 ? band : H;
-  const int P = (HB <= 128) ? 2 : 1;  // threads per canvas row (they split its columns)
-  const int T = (HB * P + 31) & ~31;
-  RenderLayout lay = render_layout(HB, W, S * C, (VT > 0 ? VT : 1) * C, OW);
+  p.T = (p.rows * p.P + 31) & ~31;
+  p.env_bytes = view_layout(hdr, view, p.rows, p.ring).total;
+  p.ok = p.env_bytes <= kBudget1 && p.T <= 1024;
+  return p;
+}
+
+template <class K>
+static cudaError_t allow_smem(K kernel, size_t smem, size_t &configured) {
+  if (smem <= 48 * 1024 || smem <= configured) return cudaSuccess;
+  cudaError_t err = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (err == cudaSuccess) configured = smem;
+  return err;
+}
+
+template <bool AA>
+static cudaError_t launch_render_t(const RenderArgs &a, const RenderPlan &plan, cudaStream_t stream, int *n_launches,
+                                   int *done, int n_done, int tail_mode, const LaunchOptions &opt) {
+  const int T = plan.T, P = plan.P, rows = plan.rows, ring = plan.ring;
+  const size_t env_bytes = (size_t)plan.env_bytes;
   // envs per CTA: the split that keeps the most envs resident per SM (228 KB of shared
   // memory, 1 KB of it reserved per CTA); ties go to the larger CTA
   int epb = 1;
   {
     int best = 0;
     for (int c = 1; c * T <= 256 || c == 1; ++c) {
-      const size_t per_cta = (size_t)lay.total * c + 1024;
+      const size_t per_cta = env_bytes * c + 1024;
       if (per_cta > 228 * 1024) break;
       const int envs = (int)(233472 / per_cta) * c;
       if (envs >= best) { best = envs; epb = c; }
     }
     if (opt.render_epb > 0) epb = opt.render_epb;
   }
-  size_t smem = (size_t)lay.total * epb;
-  if (smem > 224 * 1024 || T > 1024) return cudaErrorInvalidConfiguration;
+  size_t smem = env_bytes * epb;
+  if (smem > 224 * 1024) return cudaErrorInvalidConfiguration;
   static size_t configured = 0;
-  if (smem > 48 * 1024 && smem > configured) {
-    cudaError_t err = cudaFuncSetAttribute(moog_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (err != cudaSuccess) return err;
-    configured = smem;
-  }
+  cudaError_t err = allow_smem(moog_render_kernel<AA>, smem, configured);
+  if (err != cudaSuccess) return err;
   if (done) {
     // one env per CTA, in finishing order, overlapping the tail of the step kernel
-    smem = (size_t)lay.total;
-    static size_t configured_tail = 0;
-    if (smem > 48 * 1024 && smem > configured_tail) {
-      cudaError_t err =
-          cudaFuncSetAttribute(moog_render_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (err != cudaSuccess) return err;
-      configured_tail = smem;
-    }
-    static size_t configured_pers = 0;
-    if (tail_mode == 2 && smem > 48 * 1024 && smem > configured_pers) {
-      cudaError_t err = cudaFuncSetAttribute(moog_render_tail_persistent_kernel,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (err != cudaSuccess) return err;
-      configured_pers = smem;
-    }
+    smem = env_bytes;
+    static size_t configured_tail = 0, configured_pers = 0;
+    err = tail_mode == 2 ? allow_smem(moog_render_tail_persistent_kernel<AA>, smem, configured_pers)
+                         : allow_smem(moog_render_tail_kernel<AA>, smem, configured_tail);
+    if (err != cudaSuccess) return err;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cfg.gridDim = dim3((unsigned)a.n_envs);
@@ -298,7 +327,6 @@ cudaError_t launch_render(const RenderArgs &a, const int32_t *hdr, const int32_t
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t err;
     if (tail_mode == 2) {
       int dev = 0, sms = 0;
       cudaGetDevice(&dev);
@@ -312,17 +340,26 @@ cudaError_t launch_render(const RenderArgs &a, const int32_t *hdr, const int32_t
       if (grid > n_done) grid = n_done;
       cfg.gridDim = dim3((unsigned)grid);
       const int busy_thr = opt.tail_busy_thr > 0 ? opt.tail_busy_thr : 1;  // envs being stepped on an SM from which its render CTAs stand back
-      err = cudaLaunchKernelEx(&cfg, moog_render_tail_persistent_kernel, a, T, P, done, n_done, busy_thr, band);
+      err = cudaLaunchKernelEx(&cfg, moog_render_tail_persistent_kernel<AA>, a, T, P, done, n_done, busy_thr, rows,
+                               ring);
     } else {
-      err = cudaLaunchKernelEx(&cfg, moog_render_tail_kernel, a, T, P, (const int *)done, band);
+      err = cudaLaunchKernelEx(&cfg, moog_render_tail_kernel<AA>, a, T, P, (const int *)done, rows, ring);
     }
     if (n_launches) *n_launches += 1;
     return err;
   }
   int blocks = (a.n_envs + epb - 1) / epb;
-  moog_render_kernel<<<blocks, epb * T, smem, stream>>>(a, T, epb, P, band);
+  moog_render_kernel<AA><<<blocks, epb * T, smem, stream>>>(a, T, epb, P, rows, ring);
   if (n_launches) *n_launches += 1;
   return cudaGetLastError();
+}
+
+cudaError_t launch_render(const RenderArgs &a, const RenderPlan &plan, const int32_t *view, cudaStream_t stream,
+                          int *n_launches, int *done, int n_done, int tail_mode, const LaunchOptions &opt) {
+  if (a.n_envs <= 0) return cudaSuccess;
+  if (!plan.ok) return cudaErrorInvalidConfiguration;  // render_impl refuses such a view before
+  return view[MOOG_V_AA] > 1 ? launch_render_t<true>(a, plan, stream, n_launches, done, n_done, tail_mode, opt)
+                             : launch_render_t<false>(a, plan, stream, n_launches, done, n_done, tail_mode, opt);
 }
 
 }  // namespace moog

@@ -258,11 +258,12 @@ __device__ inline unsigned color_to_ink(int cmap, double c0, double c1, double c
 /* (sprite, row) items whose spans are precomputed, per env: 512, more for scenes with many
    sprites (a pacman maze has ~180), the rest is scan-converted by the row threads directly */
 __host__ __device__ inline int item_cap(int S) { return S * 8 < 512 ? 512 : (S * 8 > 2048 ? 2048 : S * 8); }
-struct RenderLayout { int canvas, ivtx, erec, items, ink, ymin, ymax, horiz, nedge, ibase, tmp, cap, total; };
+struct RenderLayout { int canvas, ivtx, erec, items, ink, ymin, ymax, horiz, nedge, ibase, ring, cap, total; };
 
-// H, W: canvas size (anti_aliasing x image size); OW: image width.  ext_items: bytes of a
-// buffer outside this layout that may hold the item spans (the step kernel's vertex cache, dead
-// once the int vertices exist); when they fit there, L.items = -1
+// H, W: rows and width of the canvas held at once (a band / chunk of the anti_aliasing x image
+// size canvas); OW: image width.  ext_items: bytes of a buffer outside this layout that may hold the
+// item spans (the step kernel's vertex cache, dead once the int vertices exist); when they fit
+// there, L.items = -1.  L.ring: see view_layout.
 __host__ __device__ inline RenderLayout render_layout(int H, int W, int S, int VT, int OW, int ext_items = 0) {
   RenderLayout L;
   int o = 0;
@@ -287,17 +288,29 @@ __host__ __device__ inline RenderLayout render_layout(int H, int W, int S, int V
   L.horiz = o;  o += 4 * S;
   L.nedge = o;  o += 4 * S;
   L.ibase = o;  o += 4 * (S + 1);
-  // anti_aliasing > 1: the horizontally resampled image [H][OW] reuses everything
-  // after the canvas (dead by then); the final image reuses the canvas
-  L.tmp = L.erec;
-  if (OW != W) {
-    int end = L.tmp + 4 * H * OW;
-    if (end > o) o = end;
-  }
+  L.ring = -1;
   L.total = (o + 15) & ~15;
   return L;
 }
 
+
+// The layout of a view's canvas drawn `rows` rows at a time (render_plan picks them), with
+// `ring_rows` rows of OW horizontally resampled RGBX words (anti_aliasing > 1) at L.ring.  While
+// chunks follow each other the ring lives behind everything else, like the edge lists; when one chunk
+// is the whole canvas, the edge lists and item spans are dead once it is drawn, and the ring reuses
+// their space.
+__host__ __device__ inline RenderLayout view_layout(const int32_t *hdr, const int32_t *view, int rows, int ring_rows) {
+  const int S = hdr[MOOG_H_N_SLOTS], VT = hdr[MOOG_H_N_VTX];
+  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;  // TorusGeometry: 9 copies per sprite
+  const int OW = view[MOOG_V_WIDTH];
+  RenderLayout L = render_layout(rows, view[MOOG_V_AA] * OW, S * C, (VT > 0 ? VT : 1) * C, OW);
+  if (ring_rows > 0) {
+    L.ring = rows >= view[MOOG_V_AA] * view[MOOG_V_HEIGHT] ? L.erec : L.total;
+    const int end = (L.ring + 4 * ring_rows * OW + 15) & ~15;
+    if (end > L.total) L.total = end;
+  }
+  return L;
+}
 
 // what render_env reads of one env: the SoA record (global or shared memory) and the program
 struct RenderSrc {
@@ -308,43 +321,33 @@ struct RenderSrc {
   const int32_t *view;        // the view's MOOG_VIEW_WORDS settings (view 0: hdr + MOOG_H_R_HEIGHT)
 };
 
-// PILRenderer.__call__ for ONE env by the T threads t = 0..T-1 of a CTA (every thread of the
-// CTA group that shares `base` calls it with the same arguments; `sync` is a barrier over exactly
-// those threads).  base: lay.total bytes of shared memory; ext_items: where the item spans go when
-// lay.items < 0.  P threads share a canvas row.  out: [OH][OW][3] bytes of this env's frame.
-// HB (0 = the whole canvas): rows per band.  A canvas that does not fit one CTA's shared memory
-// (the shipped pacman draws 256 x 256, tests/runtime_benchmark.py up to 1024 x 1024) is drawn in
-// bands of HB rows: `lay` is then the layout of an HB-row canvas, the edge lists are built once and
-// every band scan-converts, fills and writes out its own rows (anti_aliasing 1 only: the Lanczos
-// resize needs the rows around a band).
+// The parts of PILRenderer.__call__ for ONE env that render_env (anti_aliasing 1) and
+// render_env_aa share.  Every thread t = 0..T-1 of the CTA group that shares `base` calls them with
+// the same arguments; `sync` is a barrier over exactly those threads.
+//
+// render_prepare: int-truncated canvas vertices, ink, and Pillow's edge list and row extent of every
+// (virtual) slot, built once per env; they stay live while the canvas is drawn in bands / chunks.
 template <class Sync>
-__device__ __forceinline__ void render_env(const RenderSrc &src, const RenderLayout &lay, unsigned char *base,
-                                           unsigned *ext_items, int t, int T, int P, bool live, unsigned char *out,
-                                           const int *resample, int ksize_h, int ksize_v, Sync sync, int HB = 0) {
+__device__ __forceinline__ void render_prepare(const RenderSrc &src, const RenderLayout &lay, unsigned char *base,
+                                               int t, int T, bool live, Sync sync) {
   const int32_t *hdr = src.hdr, *view = src.view;
   const int S = hdr[MOOG_H_N_SLOTS], L = hdr[MOOG_H_N_LAYERS], VT = hdr[MOOG_H_N_VTX];
   // pil_renderer.py:65-66: the canvas is anti_aliasing x the image size
-  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
-  const int H = aa * OH, W = aa * OW;
-  const unsigned bgc = (unsigned)view[MOOG_V_BG] & 0xffffffu;
+  const int aa = view[MOOG_V_AA], H = aa * view[MOOG_V_HEIGHT], W = aa * view[MOOG_V_WIDTH];
   const int cmap = view[MOOG_V_COLORMAP], pmod = view[MOOG_V_MODIFIER], pml = view[MOOG_V_MOD_LAYER];
   // polygon_modifiers.py:88-96 TorusGeometry: every sprite is drawn as 9 copies shifted by
   // (i, j), i outer / j inner over (-1, 0, 1); copy c of slot s is the virtual slot s * C + c
   // and its vertices live at c * VT + voff[s]
   const int C = pmod == MOOG_PMOD_TORUS ? 9 : 1;
-  unsigned *canvas = (unsigned *)(base + lay.canvas);
   int2 *ivtx = (int2 *)(base + lay.ivtx);
   unsigned *ink = (unsigned *)(base + lay.ink);
   int *symin = (int *)(base + lay.ymin), *symax = (int *)(base + lay.ymax), *shoriz = (int *)(base + lay.horiz);
-  int *snedge = (int *)(base + lay.nedge), *sibase = (int *)(base + lay.ibase);
+  int *snedge = (int *)(base + lay.nedge);
   ERec *erec = (ERec *)(base + lay.erec);
-  unsigned *items = lay.items >= 0 ? (unsigned *)(base + lay.items) : ext_items;
-  const int stride = W + 1;
   const double *dyn = src.dyn, *stat = src.stat;
   const int32_t *meta = src.meta, *cnt = src.cnt;
   const double2 *vtx = src.vtx;
 
-  if (HB <= 0 || HB > H || aa > 1) HB = H;
   if (live) {
     double ox = 0, oy = 0;
     if (pmod == MOOG_PMOD_FIRST_PERSON) {  // polygon_modifiers.py:54-63
@@ -391,9 +394,27 @@ __device__ __forceinline__ void render_env(const RenderSrc &src, const RenderLay
     }
   }
   sync();  // the scan below reads every slot's extents
-#pragma unroll 1
-  for (int y0 = 0; y0 < H; y0 += HB) {
-  const int y1 = min(H, y0 + HB);  // this band: canvas rows [y0, y1)
+}
+
+// render_draw_rows: the canvas rows [y0, y1) into the layout's canvas (its row 0 = canvas row y0):
+// background, (sprite, row) item spans, then P threads per row fill the sprites in z-order.
+// Returns after a barrier: the canvas rows are complete.
+template <class Sync>
+__device__ __forceinline__ void render_draw_rows(const RenderSrc &src, const RenderLayout &lay, unsigned char *base,
+                                                 unsigned *ext_items, int t, int T, int P, bool live, int y0, int y1,
+                                                 Sync sync) {
+  const int32_t *view = src.view;
+  const int S = src.hdr[MOOG_H_N_SLOTS], VT = src.hdr[MOOG_H_N_VTX];
+  const int aa = view[MOOG_V_AA], H = aa * view[MOOG_V_HEIGHT], W = aa * view[MOOG_V_WIDTH];
+  const unsigned bgc = (unsigned)view[MOOG_V_BG] & 0xffffffu;
+  const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
+  unsigned *canvas = (unsigned *)(base + lay.canvas);
+  unsigned *ink = (unsigned *)(base + lay.ink);
+  int *symin = (int *)(base + lay.ymin), *symax = (int *)(base + lay.ymax), *shoriz = (int *)(base + lay.horiz);
+  int *snedge = (int *)(base + lay.nedge), *sibase = (int *)(base + lay.ibase);
+  ERec *erec = (ERec *)(base + lay.erec);
+  unsigned *items = lay.items >= 0 ? (unsigned *)(base + lay.items) : ext_items;
+  const int stride = W + 1;
   if (live)
     for (int i = t; i < (y1 - y0) * stride; i += T) canvas[i] = bgc;
   // (sprite, row) item ranges: exclusive prefix sum of the visible rows per slot by the first
@@ -504,87 +525,172 @@ __device__ __forceinline__ void render_env(const RenderSrc &src, const RenderLay
     }
   }
   sync();
-  const unsigned *img = canvas;  // the image to write out: [OH][img_stride] RGBX words
-  int img_stride = stride;
-  if (aa > 1) {
-    // Image.resize(LANCZOS) (Resample.c, 8 bpc): horizontal pass into an 8-bit
-    // intermediate, then vertical pass; fixed-point coefficients from the host
-    const int *bh = resample, *kh = bh + 2 * OW;
-    const int *bv = kh + OW * ksize_h, *kv = bv + 2 * OH;
-    unsigned *tmp = (unsigned *)(base + lay.tmp);
-    if (live) {
+}
+
+// render_store_rows: pil_renderer.py:118-120, np.flipud -> output row j is image row OH-1-j.  img
+// holds the image rows [r0, r1) ([r1 - r0][img_stride] RGBX words); they are the output rows
+// [OH - r1, OH - r0) of out ([OH][OW][3] bytes).
+__device__ __forceinline__ void render_store_rows(const unsigned *img, int img_stride, unsigned char *out, int OH,
+                                                  int OW, int r0, int r1, int t, int T) {
+  if ((OW & 15) == 0) {
+    // consecutive threads store consecutive 16-byte chunks of the frame (a row is OW * 3 / 16
+    // of them); packed word m = 3u + r of a row holds bytes r.. of pixel 4u + r and the first
+    // bytes of the next pixel
+    uint4 *out4 = (uint4 *)out;
+    const int cpr = (OW * 3) >> 4;
+    for (int q0 = t; q0 < (r1 - r0) * cpr; q0 += T) {
+      const int q = q0 + (OH - r1) * cpr;
+      const int j = q / cpr, c = q - j * cpr;
+      const unsigned *srcp = img + (OH - 1 - j - r0) * img_stride;
+      unsigned w[4];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int m = 4 * c + i, u = m / 3, r = m - 3 * u;
+        const unsigned lo = srcp[4 * u + r] & 0xffffffu, hi = srcp[4 * u + r + 1] & 0xffffffu;
+        w[i] = (lo >> (8 * r)) | (hi << (24 - 8 * r));
+      }
+      out4[q] = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+  } else {
+    const int nbytes = (r1 - r0) * OW * 3;
+    for (int b0 = t; b0 < nbytes; b0 += T) {
+      const int b = b0 + (OH - r1) * OW * 3;
+      int p = b / 3, ch = b - 3 * p;
+      int j = p / OW, col = p - j * OW;
+      out[b] = (unsigned char)((img[(OH - 1 - j - r0) * img_stride + col] >> (8 * ch)) & 255u);
+    }
+  }
+}
+
+// PILRenderer.__call__ with anti_aliasing 1, for ONE env by the T threads t = 0..T-1 of a CTA (every
+// thread of the CTA group that shares `base` calls it with the same arguments; `sync` is a barrier
+// over exactly those threads).  base: lay.total bytes of shared memory; ext_items: where the item
+// spans go when lay.items < 0.  P threads share a canvas row.  out: [OH][OW][3] bytes of this env's
+// frame.  HB (0 = the whole canvas): rows per band.  A canvas that does not fit one CTA's shared
+// memory (the shipped pacman draws 256 x 256, tests/runtime_benchmark.py up to 1024 x 1024) is drawn
+// in bands of HB rows: `lay` is then the layout of an HB-row canvas, the edge lists are built once
+// and every band scan-converts, fills and writes out its own rows.
+template <class Sync>
+__device__ __forceinline__ void render_env(const RenderSrc &src, const RenderLayout &lay, unsigned char *base,
+                                           unsigned *ext_items, int t, int T, int P, bool live, unsigned char *out,
+                                           Sync sync, int HB = 0) {
+  const int OH = src.view[MOOG_V_HEIGHT], OW = src.view[MOOG_V_WIDTH];
+  const int H = src.view[MOOG_V_AA] * OH;  // == OH (anti_aliasing 1)
+  if (HB <= 0 || HB > H) HB = H;
+  render_prepare(src, lay, base, t, T, live, sync);
+#pragma unroll 1
+  for (int y0 = 0; y0 < H; y0 += HB) {
+    const int y1 = min(H, y0 + HB);  // this band: canvas rows [y0, y1)
+    render_draw_rows(src, lay, base, ext_items, t, T, P, live, y0, y1, sync);
+    if (live) render_store_rows((const unsigned *)(base + lay.canvas), OW + 1, out, OH, OW, y0, y1, t, T);
+    if (y0 + HB < H) sync();  // the next band reuses the canvas and the item spans
+  }
+}
+
+// Resample.c's inner loop over n taps of 8-bit RGBX pixels p[0], p[step], ... with the fixed-point
+// coefficients k, into the channel sums r / g / b (which start at 1 << 21, the rounding term)
+__device__ __forceinline__ void lanczos_taps(const unsigned *p, int step, const int *k, int n, int &r, int &g, int &b) {
+  for (int y = 0; y < n; ++y) {
+    const unsigned px = p[y * step];
+    const int c = k[y];
+    r += (int)(px & 255u) * c;
+    g += (int)((px >> 8) & 255u) * c;
+    b += (int)((px >> 16) & 255u) * c;
+  }
+}
+
+__device__ __forceinline__ unsigned pack_clip8(int r, int g, int b) { return clip8(r) | (clip8(g) << 8) | (clip8(b) << 16); }
+
+// output pixel xx of the horizontal pass over one canvas row
+__device__ __forceinline__ unsigned resample_h(const unsigned *row, const int *bh, const int *kh, int ksize_h, int xx) {
+  int r = 1 << 21, g = 1 << 21, b = 1 << 21;
+  lanczos_taps(row + bh[2 * xx], 1, kh + xx * ksize_h, bh[2 * xx + 1], r, g, b);
+  return pack_clip8(r, g, b);
+}
+
+// PILRenderer.__call__ with anti_aliasing > 1: Image.resize(LANCZOS) of the aa x canvas (Resample.c,
+// 8 bpc: a horizontal pass into an 8-bit intermediate, then a vertical pass, with the fixed-point
+// coefficients of resample_tables on the host), streamed so that the canvas never exists whole.
+// The canvas is drawn in chunks of HC rows (render_draw_rows, every row exactly once); each chunk is
+// resampled horizontally into a ring of R rows of OW RGBX words (lay.ring; canvas row y in ring row
+// y % R), after which the next chunk reuses the canvas.  Output row yy needs the intermediate rows
+// [bv[2yy], bv[2yy] + bv[2yy+1]); it is resampled vertically into the dead canvas and written out as
+// soon as its last row is in the ring.  The windows are monotone in yy and at most ksize_v rows
+// long, so R = HC + ksize_v rows keep every row a pending output row still reads.  A canvas that is
+// one chunk (HC == H, R == H: the ring is the whole intermediate) takes the straight single pass
+// instead, without ring arithmetic.  Same arguments as render_env; `lay` is the layout of an HC-row
+// canvas with R ring rows.
+template <class Sync>
+__device__ __forceinline__ void render_env_aa(const RenderSrc &src, const RenderLayout &lay, unsigned char *base,
+                                              unsigned *ext_items, int t, int T, int P, bool live, unsigned char *out,
+                                              const int *resample, int ksize_h, int ksize_v, Sync sync, int HC, int R) {
+  const int32_t *view = src.view;
+  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH], aa = view[MOOG_V_AA];
+  const int H = aa * OH, W = aa * OW, stride = W + 1;
+  const int *bh = resample, *kh = bh + 2 * OW;
+  const int *bv = kh + OW * ksize_h, *kv = bv + 2 * OH;
+  unsigned *canvas = (unsigned *)(base + lay.canvas);
+  unsigned *ring = (unsigned *)(base + lay.ring);
+  render_prepare(src, lay, base, t, T, live, sync);
+  if (HC >= H) {  // one chunk
+    render_draw_rows(src, lay, base, ext_items, t, T, P, live, 0, H, sync);
+    if (live)
       for (int i = t; i < H * OW; i += T) {
         const int yy = i / OW, xx = i - yy * OW;
-        const int xmin = bh[2 * xx], xmax = bh[2 * xx + 1];
-        const int *k = kh + xx * ksize_h;
-        const unsigned *srcp = canvas + yy * stride + xmin;
-        int r = 1 << 21, gch = 1 << 21, b = 1 << 21;
-        for (int x = 0; x < xmax; ++x) {
-          const unsigned px = srcp[x];
-          const int c = k[x];
-          r += (int)(px & 255u) * c;
-          gch += (int)((px >> 8) & 255u) * c;
-          b += (int)((px >> 16) & 255u) * c;
-        }
-        tmp[i] = clip8(r) | (clip8(gch) << 8) | (clip8(b) << 16);
+        ring[i] = resample_h(canvas + yy * stride, bh, kh, ksize_h, xx);
       }
-    }
     sync();
-    if (live) {
-      unsigned *small = canvas;  // the canvas is dead
+    if (live)
       for (int i = t; i < OH * OW; i += T) {
         const int yy = i / OW, xx = i - yy * OW;
-        const int ymin = bv[2 * yy], ymax = bv[2 * yy + 1];
-        const int *k = kv + yy * ksize_v;
-        int r = 1 << 21, gch = 1 << 21, b = 1 << 21;
-        for (int y = 0; y < ymax; ++y) {
-          const unsigned px = tmp[(y + ymin) * OW + xx];
-          const int c = k[y];
-          r += (int)(px & 255u) * c;
-          gch += (int)((px >> 8) & 255u) * c;
-          b += (int)((px >> 16) & 255u) * c;
-        }
-        small[i] = clip8(r) | (clip8(gch) << 8) | (clip8(b) << 16);
+        int r = 1 << 21, g = 1 << 21, b = 1 << 21;
+        lanczos_taps(ring + bv[2 * yy] * OW + xx, OW, kv + yy * ksize_v, bv[2 * yy + 1], r, g, b);
+        canvas[i] = pack_clip8(r, g, b);  // the canvas is dead
       }
-    }
     sync();
-    img_stride = OW;
+    if (live) render_store_rows(canvas, OW, out, OH, OW, 0, OH, t, T);
+    return;
   }
-  if (live) {
-    // pil_renderer.py:118-120: np.flipud -> output row j is image row OH-1-j
-    // (a band holds the image rows [y0, y1), i.e. the output rows [OH - y1, OH - y0); with
-    // anti-aliasing there is one band and the resized image starts at row 0)
-    const int r0 = aa > 1 ? 0 : y0, r1 = aa > 1 ? OH : y1;
-    if ((OW & 15) == 0) {
-      // consecutive threads store consecutive 16-byte chunks of the frame (a row is OW * 3 / 16
-      // of them); packed word m = 3u + r of a row holds bytes r.. of pixel 4u + r and the first
-      // bytes of the next pixel
-      uint4 *out4 = (uint4 *)out;
-      const int cpr = (OW * 3) >> 4;
-      for (int q0 = t; q0 < (r1 - r0) * cpr; q0 += T) {
-        const int q = q0 + (OH - r1) * cpr;
-        const int j = q / cpr, c = q - j * cpr;
-        const unsigned *srcp = img + (OH - 1 - j - r0) * img_stride;
-        unsigned w[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const int m = 4 * c + i, u = m / 3, r = m - 3 * u;
-          const unsigned lo = srcp[4 * u + r] & 0xffffffu, hi = srcp[4 * u + r + 1] & 0xffffffu;
-          w[i] = (lo >> (8 * r)) | (hi << (24 - 8 * r));
+  // output rows resampled per pass: as many as the dead canvas holds
+  const int stage_rows = max(1, (HC * stride) / OW);
+  int next = 0;  // first output row not yet written
+  int rb = 0;    // ring row of canvas row y0 (y0 % R)
+#pragma unroll 1
+  for (int y0 = 0; y0 < H; y0 += HC) {
+    const int y1 = min(H, y0 + HC);  // this chunk: canvas rows [y0, y1)
+    render_draw_rows(src, lay, base, ext_items, t, T, P, live, y0, y1, sync);
+    if (live)
+      for (int i = t; i < (y1 - y0) * OW; i += T) {
+        const int yr = i / OW, xx = i - yr * OW;
+        const int q = rb + yr;  // yr < HC <= R
+        ring[(q < R ? q : q - R) * OW + xx] = resample_h(canvas + yr * stride, bh, kh, ksize_h, xx);
+      }
+    rb += y1 - y0;
+    if (rb >= R) rb -= R;
+    sync();  // the chunk's intermediate rows are in the ring; the canvas is dead
+    // output rows [next, last) have their whole window in the ring (every row after the last chunk)
+    int last = y1 == H ? OH : next;
+    while (last < OH && bv[2 * last] + bv[2 * last + 1] <= y1) ++last;
+#pragma unroll 1
+    for (int r0 = next; r0 < last; r0 += stage_rows) {
+      const int r1 = min(last, r0 + stage_rows);
+      if (live)
+        for (int i = t; i < (r1 - r0) * OW; i += T) {
+          const int yr = i / OW, xx = i - yr * OW, yy = r0 + yr;
+          const int ymin = bv[2 * yy], ymax = bv[2 * yy + 1];
+          const int *k = kv + yy * ksize_v;
+          // the window is ring rows [q, q + ymax) up to the ring's end, then from ring row 0 on
+          const int q = ymin % R, n1 = min(ymax, R - q);
+          int r = 1 << 21, g = 1 << 21, b = 1 << 21;
+          lanczos_taps(ring + q * OW + xx, OW, k, n1, r, g, b);
+          lanczos_taps(ring + xx, OW, k + n1, ymax - n1, r, g, b);
+          canvas[i] = pack_clip8(r, g, b);
         }
-        out4[q] = make_uint4(w[0], w[1], w[2], w[3]);
-      }
-    } else {
-      const int nbytes = (r1 - r0) * OW * 3;
-      for (int b0 = t; b0 < nbytes; b0 += T) {
-        const int b = b0 + (OH - r1) * OW * 3;
-        int p = b / 3, ch = b - 3 * p;
-        int j = p / OW, col = p - j * OW;
-        out[b] = (unsigned char)((img[(OH - 1 - j - r0) * img_stride + col] >> (8 * ch)) & 255u);
-      }
+      sync();
+      if (live) render_store_rows(canvas, OW, out, OH, OW, r0, r1, t, T);
+      if (r1 < OH) sync();  // the canvas is the next pass's (or chunk's) again
     }
-  }
-  if (y0 + HB < H) sync();  // the next band reuses the canvas and the item spans
+    next = last;
   }
 }
 

@@ -3756,7 +3756,7 @@ __global__ void __launch_bounds__(64) moog_step_kernel(const StepArgs a) {
     const int T = (int)blockDim.x;
     const int P = (OH * 2 <= T) ? 2 : 1;
     render_env(src, lay, smem_raw + a.render_off, (unsigned *)e.vtx, (int)threadIdx.x, T, P, true,
-               a.frames + (size_t)e.env_id * OH * OW * 3, nullptr, 0, 0, [] { __syncthreads(); });
+               a.frames + (size_t)e.env_id * OH * OW * 3, [] { __syncthreads(); });
   }
 #endif
 }

@@ -5,7 +5,8 @@ out = subprocess.run(['cuobjdump', '-elf', sys.argv[1]], capture_output=True, te
 pat = sys.argv[2] if len(sys.argv) > 2 else ''
 counts = {}
 # symbol table rows: index, value, size, info (0x2 / 0x12 = local / global function), other, section, name
-for m in re.finditer(r'^\s*0x[0-9a-f]+\s+0x[0-9a-f]+\s+(0x[0-9a-f]+)\s+0x1?2\s+\S+\s+\S+\s+(\S+)\s*$', out, re.M):
+# (the value of a kernel's own symbol prints as a bare 0)
+for m in re.finditer(r'^\s*0x[0-9a-f]+\s+(?:0x[0-9a-f]+|0)\s+(0x[0-9a-f]+)\s+0x1?2\s+\S+\s+\S+\s+(\S+)\s*$', out, re.M):
     name = m.group(2)  # out-of-line functions read $<kernel>$<function>
     if pat in name:
         counts[name] = counts.get(name, 0) + int(m.group(1), 16) // 16
