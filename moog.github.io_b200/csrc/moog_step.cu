@@ -30,6 +30,7 @@
 #include "moog_common.cuh"
 #include "moog_dcv_argmin.cuh"
 #include "moog_render_dev.cuh"
+#include "moog_seg_cross.cuh"
 
 namespace moog {
 
@@ -557,16 +558,40 @@ __device__ __noinline__ bool segments_parallel_case(double x1, double y1, double
   return false;
 }
 
-__device__ inline bool segments_intersect(double x1, double y1, double x2, double y2, double x3, double y3,
-                                          double x4, double y4) {
-  double den = ((y4 - y3) * (x2 - x1)) - ((x4 - x3) * (y2 - y1));
-  if (isclose_(den, 0.0)) return segments_parallel_case(x1, y1, x2, y2, x3, y3, x4, y4);
-  double n1 = ((x4 - x3) * (y1 - y3)) - ((y4 - y3) * (x1 - x3));
-  double n2 = ((x2 - x1) * (y1 - y3)) - ((y2 - y1) * (x1 - x3));
+// (fmin(a, b), fmax(a, b)) for finite a, b: one compare and selects instead of fmin / fmax's NaN handling
+__device__ __forceinline__ void minmax_finite(double a, double b, double &lo, double &hi) {
+  const bool s = a < b;
+  lo = s ? a : b;
+  hi = s ? b : a;
+}
+
+// the range tests of segments_intersect by division, for the operands seg_param_in_unit leaves
+// undecided (rare: kept out of the callers' instruction stream)
+__device__ __noinline__ bool segments_params_divide(double n1, double n2, double den) {
   double u1 = n1 / den;
   double u2 = n2 / den;
   return ((u1 > 0.0 || isclose_(u1, 0.0)) && (u1 < 1.0 || isclose_(u1, 1.0)) &&
           (u2 > 0.0 || isclose_(u2, 0.0)) && (u2 < 1.0 || isclose_(u2, 1.0)));
+}
+
+// src/_path.h segments_intersect, called by every lane of the warp together; a lane with `act`
+// false returns false.  The range tests on u1 = n1 / den and u2 = n2 / den are decided without
+// dividing (moog_seg_cross.cuh); when some lane's operands are outside that decision's regime,
+// those lanes divide, behind a warp-uniform branch.
+__device__ __forceinline__ bool segments_intersect(bool act, double x1, double y1, double x2, double y2, double x3,
+                                                   double y3, double x4, double y4) {
+  const double den = ((y4 - y3) * (x2 - x1)) - ((x4 - x3) * (y2 - y1));
+  const double n1 = ((x4 - x3) * (y1 - y3)) - ((y4 - y3) * (x1 - x3));
+  const double n2 = ((x2 - x1) * (y1 - y3)) - ((y2 - y1) * (x1 - x3));
+  const bool par = isclose_(den, 0.0);
+  bool e1, e2;
+  bool r = seg_param_in_unit(n1, den, e1) & seg_param_in_unit(n2, den, e2);
+  const bool divide = act && !par && !(e1 && e2);
+  if (__any_sync(FULL, divide)) {
+    if (divide) r = segments_params_divide(n1, n2, den);
+  }
+  if (act && par) r = segments_parallel_case(x1, y1, x2, y2, x3, y3, x4, y4);
+  return act && r;
 }
 
 // point_in_path_impl for one point against the closed outline Q[0..n-1]
@@ -590,7 +615,7 @@ __device__ inline bool point_in_poly(double tx, double ty, const double2 *Q, int
 
 // serial restatement of path_intersects_path for outlines with degenerate
 // (nearly zero-length) edges, where matplotlib merges consecutive points.
-// All lanes run it redundantly; it is never on the hot path.
+// All lanes run it redundantly (together); it is never on the hot path.
 __device__ __noinline__ bool path_intersects_path_serial(const double2 *A, int nA, const double2 *B, int nB) {
   int na = nA + 1, nb = nB + 1;
   if (na < 2 || nb < 2) return false;
@@ -604,7 +629,7 @@ __device__ __noinline__ bool path_intersects_path_serial(const double2 *A, int n
       double2 pb = B[j == nB ? 0 : j];
       double x22 = pb.x, y22 = pb.y;
       if (isclose_((x21 - x22) * (x21 - x22) + (y21 - y22) * (y21 - y22), 0.0)) continue;
-      if (segments_intersect(x11, y11, x12, y12, x21, y21, x22, y22)) return true;
+      if (segments_intersect(true, x11, y11, x12, y12, x21, y21, x22, y22)) return true;
       x21 = x22;
       y21 = y22;
     }
@@ -634,6 +659,13 @@ __device__ __noinline__ bool containment_fallback(int a, int b, bool try_b_in_a,
   return false;
 }
 
+// floor(2^16 / n) + 1 for n = 1..32: (t * PAIR_DIV_MAGIC[n]) >> 16 == t / n for t < 2^16 / n, which
+// covers the pair indices t < 32 n of path_intersects_filled_impl (with 2^16 + k = n PAIR_DIV_MAGIC[n],
+// 0 < k <= n: t / n + t k / (n 2^16) < floor(t / n) + (n - 1) / n + t / 2^16)
+__constant__ unsigned PAIR_DIV_MAGIC[33] = {
+    0,    65537, 32769, 21846, 16385, 13108, 10923, 9363, 8193, 7282, 6554, 5958, 5462, 5042, 4682, 4370, 4097,
+    3856, 3641,  3450,  3277,  3121,  2979,  2850,  2731, 2622, 2521, 2428, 2341, 2260, 2185, 2115, 2049};
+
 // Path.intersects_path(a, b, filled=True) as MOOG calls it (sprite.py:482-483)
 __device__ __forceinline__ bool path_intersects_filled_impl(const Env &e, int a, int b) {
   const double2 *A = e.vtx + e.voff[a];
@@ -653,7 +685,9 @@ __device__ __forceinline__ bool path_intersects_filled_impl(const Env &e, int a,
     // edges of P whose (padded) box meets Q's box and edges of Q whose box meets
     // P's padded box.  The surviving (P edge, Q edge) pairs -- a handful for two
     // touching outlines -- are then tested all at once, one pair per lane.
-    // Argument order of segments_intersect is kept.
+    // Argument order of segments_intersect is kept.  Every coordinate here is finite (SLF_NONFINITE
+    // takes the serial path), so fmin / fmax reduce to a compare and selects, and a bound on
+    // fmax(u, v) (fmin) to the same bound on both u and v.
     bool lanesA = nA >= nB;
     const double2 *P = lanesA ? A : B;
     const double2 *Q = lanesA ? B : A;
@@ -662,18 +696,19 @@ __device__ __forceinline__ bool path_intersects_filled_impl(const Env &e, int a,
     bool act = e.lane < nP;
     double2 p1 = P[act ? e.lane : 0];
     double2 p2 = P[act ? ((e.lane + 1 == nP) ? 0 : e.lane + 1) : 0];
-    double pxmin = fmin(p1.x, p2.x) - AABB_PAD, pxmax = fmax(p1.x, p2.x) + AABB_PAD;
-    double pymin = fmin(p1.y, p2.y) - AABB_PAD, pymax = fmax(p1.y, p2.y) + AABB_PAD;
-    act = act && !(pxmax < BOX(e, 0, qslot) || pxmin > BOX(e, 2, qslot) || pymax < BOX(e, 1, qslot) ||
-                   pymin > BOX(e, 3, qslot));
+    double pxmin, pxmax, pymin, pymax;
+    minmax_finite(p1.x, p2.x, pxmin, pxmax);
+    minmax_finite(p1.y, p2.y, pymin, pymax);
+    act = act && !(pxmax + AABB_PAD < BOX(e, 0, qslot) || pxmin - AABB_PAD > BOX(e, 2, qslot) ||
+                   pymax + AABB_PAD < BOX(e, 1, qslot) || pymin - AABB_PAD > BOX(e, 3, qslot));
     bool qact = e.lane < nQ;
     {
       double2 q1 = Q[qact ? e.lane : 0];
       double2 q2 = Q[qact ? ((e.lane + 1 == nQ) ? 0 : e.lane + 1) : 0];
       double Pxmin = BOX(e, 0, pslot) - AABB_PAD, Pymin = BOX(e, 1, pslot) - AABB_PAD;
       double Pxmax = BOX(e, 2, pslot), Pymax = BOX(e, 3, pslot);
-      qact = qact && !(fmax(q1.x, q2.x) < Pxmin || fmin(q1.x, q2.x) > Pxmax || fmax(q1.y, q2.y) < Pymin ||
-                       fmin(q1.y, q2.y) > Pymax);
+      qact = qact && !((q1.x < Pxmin && q2.x < Pxmin) || (q1.x > Pxmax && q2.x > Pxmax) ||
+                       (q1.y < Pymin && q2.y < Pymin) || (q1.y > Pymax && q2.y > Pymax));
     }
     const unsigned pm = __ballot_sync(FULL, act), qm = __ballot_sync(FULL, qact);
     if (pm && qm) {
@@ -684,23 +719,24 @@ __device__ __forceinline__ bool path_intersects_filled_impl(const Env &e, int a,
       if (qact) e.scratch[32 + __popc(qm & lt)] = (unsigned char)e.lane;
       wsync();
       const int total = np_ * nq_;
+      const unsigned qmagic = PAIR_DIV_MAGIC[nq_];
       for (int base = 0; base < total; base += 32) {
         int t = base + e.lane;
         bool v = t < total;
-        int pi = v ? t / nq_ : 0;
+        int pi = v ? (int)(((unsigned)t * qmagic) >> 16) : 0;  // t / nq_
         int qi = v ? t - pi * nq_ : 0;
         int pl = e.scratch[pi], ql = e.scratch[32 + qi];
         double2 a1 = P[pl], a2 = P[(pl + 1 == nP) ? 0 : pl + 1];
         double2 b1 = Q[ql], b2 = Q[(ql + 1 == nQ) ? 0 : ql + 1];
-        double axmin = fmin(a1.x, a2.x) - AABB_PAD, axmax = fmax(a1.x, a2.x) + AABB_PAD;
-        double aymin = fmin(a1.y, a2.y) - AABB_PAD, aymax = fmax(a1.y, a2.y) + AABB_PAD;
-        bool h = false;
-        if (v && !(fmax(b1.x, b2.x) < axmin || fmin(b1.x, b2.x) > axmax || fmax(b1.y, b2.y) < aymin ||
-                   fmin(b1.y, b2.y) > aymax)) {
-          const double2 f1 = lanesA ? a1 : b1, f2 = lanesA ? a2 : b2;
-          const double2 g1 = lanesA ? b1 : a1, g2 = lanesA ? b2 : a2;
-          h = segments_intersect(f1.x, f1.y, f2.x, f2.y, g1.x, g1.y, g2.x, g2.y);
-        }
+        double axmin, axmax, aymin, aymax;
+        minmax_finite(a1.x, a2.x, axmin, axmax);
+        minmax_finite(a1.y, a2.y, aymin, aymax);
+        axmin -= AABB_PAD, axmax += AABB_PAD, aymin -= AABB_PAD, aymax += AABB_PAD;
+        const bool test = v && !((b1.x < axmin && b2.x < axmin) || (b1.x > axmax && b2.x > axmax) ||
+                                 (b1.y < aymin && b2.y < aymin) || (b1.y > aymax && b2.y > aymax));
+        const double2 f1 = lanesA ? a1 : b1, f2 = lanesA ? a2 : b2;
+        const double2 g1 = lanesA ? b1 : a1, g2 = lanesA ? b2 : a2;
+        const bool h = segments_intersect(test, f1.x, f1.y, f2.x, f2.y, g1.x, g1.y, g2.x, g2.y);
         if (__any_sync(FULL, h)) return true;
       }
     }
@@ -749,23 +785,6 @@ __device__ inline bool overlaps(const Env &e, int a, int b) {
 // ---------------------------------------------------------------------------
 // collisions.py
 // ---------------------------------------------------------------------------
-// (fl(n / d) >= 0 && fl(n / d) <= 1) without the division, for the crossing test of
-// sprite.py:171-175.  Rounding to nearest is monotone and 0 and 1 are representable, so for
-// finite operands whose quotient neither overflows nor underflows
-//   fl(n/d) <= 1  <=>  n/d <= 1   (the smallest quotient above 1, (d + ulp)/d, is > 1 + 2^-53
-//                                  and rounds to 1 + 2^-52)
-//   fl(n/d) >= 0  <=>  n/d >= 0 or n == -0.0  (-0.0 >= 0 is true)
-// and d == 0 gives +-inf or NaN, false either way.  `exact` is false when the operands are
-// outside that regime; the caller then divides.
-__device__ __forceinline__ bool unit_ratio(double n, double d, bool &exact) {
-  // the regime test on the exponent fields (high words): |n| in [2^-959, 2^961) or n == 0, and
-  // |d| in [2^-959, 2^33) or d == 0 -- inside [1e-290, 1e290] and [1e-290, 1e10]; NaN / inf fail
-  const unsigned hn = (unsigned)__double2hiint(n) & 0x7fffffffu, hd = (unsigned)__double2hiint(d) & 0x7fffffffu;
-  exact = ((hn - (64u << 20)) < ((1984u - 64u) << 20) || n == 0.0) &&
-          ((hd - (64u << 20)) < ((1056u - 64u) << 20) || d == 0.0);
-  return d > 0.0 ? (n >= 0.0 && n <= d) : (d < 0.0 && n <= 0.0 && n >= d);
-}
-
 enum { HELPER_EXIT = 0, HELPER_DCV = 1 };
 // named barrier over the owner and helper warps of the CTA (also orders their shared-memory traffic)
 // (the warp reconverges first: `bar.sync` is the .aligned form, which every lane of a warp must execute together --
