@@ -178,12 +178,12 @@ int moog_step_launch_info(const moog_program *p, int n_envs, int *resident_envs_
 int moog_step_draws_frames(const moog_program *p, int n_envs);
 
 /* Launch options of a program (tuning / tests; the reference has no counterpart).  The MOOG_*
- * environment variables of the same names (MOOG_HELPER, MOOG_CTAS_PER_SM, MOOG_SMEM_PAD,
- * MOOG_FUSED_RENDER, MOOG_TAIL_RENDER, MOOG_TAIL_CTAS_PER_SM, MOOG_TAIL_BUSY_THR, MOOG_RENDER_EPB,
- * MOOG_TRACE_TIMES) are read once, when the program is created; this call changes one option of a
- * live program: name in {"helper", "ctas_per_sm", "smem_pad", "fused_render", "tail_render",
- * "tail_ctas_per_sm", "tail_busy_thr", "render_epb", "trace_times", "seed"}; value -1 (helper,
- * fused_render) or 0 (the counts) hands the decision back to the library.  None of the launch options
+ * environment variables of the same names (MOOG_HELPER, MOOG_CTAS_PER_SM, MOOG_TRACE_TIMES) are
+ * read once, when the program is created; this call changes one option of a live program: name in
+ * {"helper", "ctas_per_sm", "trace_times", "seed"}, any other name is MOOG_E_INVAL.  "helper" 0 / 1:
+ * the helper warp off / on, "ctas_per_sm": envs resident per SM for the step kernel; value -1
+ * (helper) or 0 (ctas_per_sm) hands the decision back to the library.  "trace_times" 1: globaltimer
+ * stamps of every env's step and render in io->counters (diagnostic).  None of the launch options
  * changes results; "seed" is the io.seed that moog_env_post_reset (which takes no moog_step_io) keys
  * the draws of its rules pass with (CreateSprites, random conditions). */
 int moog_program_set_option(moog_program *p, const char *name, int value);

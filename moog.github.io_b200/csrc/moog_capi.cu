@@ -54,10 +54,7 @@ namespace moog {
 LaunchOptions launch_options_from_env() {
   LaunchOptions o;
   static const struct { const char *env, *name; } kVars[] = {
-      {"MOOG_HELPER", "helper"}, {"MOOG_CTAS_PER_SM", "ctas_per_sm"}, {"MOOG_SMEM_PAD", "smem_pad"},
-      {"MOOG_FUSED_RENDER", "fused_render"}, {"MOOG_TAIL_RENDER", "tail_render"},
-      {"MOOG_TAIL_CTAS_PER_SM", "tail_ctas_per_sm"}, {"MOOG_TAIL_BUSY_THR", "tail_busy_thr"},
-      {"MOOG_RENDER_EPB", "render_epb"}, {"MOOG_TRACE_TIMES", "trace_times"}};
+      {"MOOG_HELPER", "helper"}, {"MOOG_CTAS_PER_SM", "ctas_per_sm"}, {"MOOG_TRACE_TIMES", "trace_times"}};
   for (const auto &v : kVars) {
     const char *t = getenv(v.env);
     if (t && *t) set_launch_option(o, v.name, atoi(t));
@@ -69,12 +66,6 @@ bool set_launch_option(LaunchOptions &o, const char *name, int value) {
   const std::string n(name);
   if (n == "helper") o.helper = value;
   else if (n == "ctas_per_sm") o.ctas_per_sm = value;
-  else if (n == "smem_pad") o.smem_pad = value;
-  else if (n == "fused_render") o.fused_render = value;
-  else if (n == "tail_render") o.tail_render = value;
-  else if (n == "tail_ctas_per_sm") o.tail_ctas_per_sm = value;
-  else if (n == "tail_busy_thr") o.tail_busy_thr = value;
-  else if (n == "render_epb") o.render_epb = value;
   else if (n == "trace_times") o.trace_times = value;
   else if (n == "seed") o.seed = value;
   else return false;
@@ -366,25 +357,16 @@ void moog_program_destroy(moog_program *p) {
 
 int moog_program_env_smem_bytes(const moog_program *p) { return p ? moog::env_smem_bytes(p->hdr) : MOOG_E_INVAL; }
 
-// envs resident per SM / helper warp for a batch of n_envs (see the comment in run_step)
-static void launch_policy(const moog::LaunchOptions &opt, int n_envs, bool ordered, int *resident, bool *helper) {
-  *resident = 0;
-  *helper = false;
+static int sm_count() {
   int dev = 0, sms = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (sms > 0) {
-    *resident = (n_envs + 7 * sms / 2) / (7 * sms);  // n_envs / (7 x SMs), rounded
-    // helper-warp regime (few envs per SM): one more env per SM pays once the frames are drawn
-    // behind the step (4096 envs: 4 -> 5 per SM, 4.66 -> 4.46 ms); larger batches keep 7 waves
-    // (8192 / 32768 envs measured slower at 10 / 40 per SM than at 8 / 32)
-    if (*resident <= 4) *resident = (2 * n_envs + 11 * sms / 2) / (11 * sms);
-    if (*resident < 2) *resident = 2;
-    *helper = *resident <= 6;
-  }
-  if (!ordered) *resident = 0;
-  if (opt.helper >= 0) *helper = opt.helper != 0;
-  if (opt.ctas_per_sm > 0) *resident = opt.ctas_per_sm;
+  return sms;
+}
+
+// what moog_env_step with frames does with a batch of n_envs on the current device
+static moog::StepPlan env_step_plan(const moog_program *p, int n_envs) {
+  return moog::plan_step(p->hdr, moog::MODE_ENV_STEP, n_envs, true, sm_count(), p->opt);
 }
 
 int moog_program_set_option(moog_program *p, const char *name, int value) {
@@ -395,35 +377,20 @@ int moog_program_set_option(moog_program *p, const char *name, int value) {
 int moog_step_launch_info(const moog_program *p, int n_envs, int *resident_envs_per_sm, int *warps_per_env,
                           int *smem_bytes_per_env) {
   if (!p || n_envs < 0) return MOOG_E_INVAL;
-  int resident = 0;
-  bool helper = false;
-  launch_policy(p->opt, n_envs, n_envs >= 1024, &resident, &helper);
-  if (resident_envs_per_sm) *resident_envs_per_sm = resident;
-  if (warps_per_env) *warps_per_env = helper ? 2 : 1;
-  if (smem_bytes_per_env) *smem_bytes_per_env = moog::env_smem_bytes(p->hdr, helper);
+  const moog::StepPlan plan = env_step_plan(p, n_envs);
+  if (resident_envs_per_sm) *resident_envs_per_sm = plan.resident;
+  if (warps_per_env) *warps_per_env = plan.helper ? 2 : 1;
+  if (smem_bytes_per_env) *smem_bytes_per_env = moog::env_smem_bytes(p->hdr, plan.helper);
   return 0;
-}
-
-// How moog_env_step produces io->frames for a batch of n_envs: 2 = inside the step kernel when one
-// CTA can hold the canvas (small batches: every env has an SM to itself, one launch and no second
-// pass over the state), 1 = by the render kernel.
-static int frames_mode(int n_envs) {
-  int dev = 0, sms = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  return n_envs <= 2 * sms ? 2 : 1;
 }
 
 int moog_step_draws_frames(const moog_program *p, int n_envs) {
   if (!p || n_envs < 0) return MOOG_E_INVAL;
-  int resident = 0;
-  bool helper = false;
-  launch_policy(p->opt, n_envs, n_envs >= 1024, &resident, &helper);
-  return moog::plan_step(p->hdr, resident, helper, frames_mode(n_envs), p->opt).fuse ? 1 : 0;
+  return env_step_plan(p, n_envs).fuse ? 1 : 0;
 }
 
 static int render_impl(moog_program *p, const moog_state *st, int n_envs, int view, uint8_t *frames, void *stream,
-                       int *done, int tail_mode, long long *trace = nullptr);
+                       int *done, long long *trace = nullptr);
 
 static int run_step(moog_program *p, const moog_state *st, int n_envs, int mode, const moog_step_io *io,
                     int layer_a, int layer_b, uint8_t *overlap_out, void *stream) {
@@ -443,10 +410,14 @@ static int run_step(moog_program *p, const moog_state *st, int n_envs, int mode,
   a.layer_a = layer_a;
   a.layer_b = layer_b;
   a.overlap_out = overlap_out;
+  if (a.io.frames && (mode != moog::MODE_ENV_STEP || !p->hdr[MOOG_H_R_ENABLED] || p->hdr[MOOG_H_R_AA] < 1))
+    return MOOG_E_INVAL;
+  // a view no chunk size can hold is refused before anything is launched
+  if (a.io.frames && !p->plan[0].ok) return MOOG_E_UNSUPPORTED;
+  const moog::StepPlan plan = moog::plan_step(p->hdr, mode, n_envs, a.io.frames != nullptr, sm_count(), p->opt);
   int launches = 0;
   cudaError_t err = cudaSuccess;
-  if ((mode == moog::MODE_ENV_STEP || mode == moog::MODE_PHYSICS) && n_envs >= 1024) {
-    // longest-processing-time-first dispatch from the costs of the previous call
+  if (plan.ordered) {
     if (p->sched_cap < n_envs) {
       if (p->sched) cudaFree(p->sched);
       p->sched = nullptr;
@@ -467,32 +438,7 @@ static int run_step(moog_program *p, const moog_state *st, int n_envs, int mode,
     a.order = order;
     a.cost = cost;
   }
-  // The step ends when its longest-running env does, and a warp runs ~2.4x slower next to 11
-  // others than alone (profiles/README.md): with the envs dispatched longest-first, capping
-  // the envs resident per SM at about n_envs / (5.5 .. 7 x SMs) finishes the step sooner than filling
-  // the SMs (4096 envs on 148 SMs: 5 per SM; measured with the frames drawn behind the step, step
-  // + render per 4096 envs: 3: 5.33 ms, 4: 4.66 ms, 5: 4.46 ms, and 5.6 ms at 12 with one warp per env).
-  // In that regime the SMs have registers to spare, and every env gets a helper warp that
-  // computes one of the two directions of _get_collision_vectors (MOOG_HELPER=0/1 overrides).
-  int resident = 0;
-  bool helper = false;
-  launch_policy(p->opt, n_envs, a.order != nullptr, &resident, &helper);
-  bool fused = false;
-  if (a.io.frames && (mode != moog::MODE_ENV_STEP || !p->hdr[MOOG_H_R_ENABLED] || p->hdr[MOOG_H_R_AA] < 1))
-    return MOOG_E_INVAL;
-  // a view no chunk size can hold is refused before anything is launched
-  if (a.io.frames && !p->plan[0].ok) return MOOG_E_UNSUPPORTED;
-  const int fmode = a.io.frames ? frames_mode(n_envs) : 0;
-  // Frames of a large batch: the step ends when its longest-running env does, and long before
-  // that most SMs have no env left to step.  The render kernel is launched behind the step kernel
-  // with programmatic stream serialization, starts as soon as the last env has got an SM, and
-  // draws the envs in the order they finish (the `done` list) on the SMs the step left idle
-  // (MOOG_TAIL_RENDER=0: the render kernel waits for the whole step instead).
-  bool tail = a.io.frames && a.order != nullptr &&
-              !moog::plan_step(p->hdr, resident, helper, fmode, p->opt).fuse;
-  const int tail_mode = p->opt.tail_render;
-  if (tail_mode <= 0) tail = false;
-  if (tail) {
+  if (plan.tail) {
     if (p->done_cap < n_envs) {
       if (p->done) cudaFree(p->done);
       p->done = nullptr;
@@ -505,15 +451,14 @@ static int run_step(moog_program *p, const moog_state *st, int n_envs, int mode,
     err = cudaMemsetAsync(p->done, 0, sizeof(int) * (1 + (size_t)n_envs + moog::kTailExtraInts), (cudaStream_t)stream);
     if (err != cudaSuccess) return cuda_fail(err);
     a.done = p->done;
-    if (tail_mode == 2) a.sm_active = p->done + 1 + n_envs + 1;
+    a.sm_active = p->done + 1 + n_envs + 1;
   }
   a.trace = (p->opt.trace_times != 0 && a.io.counters) ? 1 : 0;  // diagnostic: per-env timeline in io.counters
-  err = moog::launch_step(a, p->hdr, (cudaStream_t)stream, &launches, 0, -1, resident, helper, fmode, &fused, p->opt);
+  err = moog::launch_step(a, p->hdr, plan, (cudaStream_t)stream, &launches);
   g_launches += launches;
   if (err != cudaSuccess) return cuda_fail(err);
-  if (a.io.frames && !fused)
-    return render_impl(p, st, n_envs, 0, a.io.frames, stream, tail ? p->done : nullptr, tail_mode,
-                       a.trace ? (long long *)a.io.counters : nullptr);
+  if (a.io.frames && !plan.fuse)
+    return render_impl(p, st, n_envs, 0, a.io.frames, stream, a.done, a.trace ? (long long *)a.io.counters : nullptr);
   return 0;
 }
 
@@ -550,16 +495,16 @@ int moog_overlap_pairs(moog_program *p, const moog_state *st, int n_envs, int la
 }
 
 int moog_render(moog_program *p, const moog_state *st, int n_envs, uint8_t *frames, void *stream) {
-  return render_impl(p, st, n_envs, 0, frames, stream, nullptr, 0);
+  return render_impl(p, st, n_envs, 0, frames, stream, nullptr);
 }
 
 int moog_render_view(moog_program *p, const moog_state *st, int n_envs, int view, uint8_t *frames, void *stream) {
   if (!p || !frames || ((uintptr_t)frames & 15) || view < 0 || view >= p->n_views) return MOOG_E_INVAL;
-  return render_impl(p, st, n_envs, view, frames, stream, nullptr, 0);
+  return render_impl(p, st, n_envs, view, frames, stream, nullptr);
 }
 
 static int render_impl(moog_program *p, const moog_state *st, int n_envs, int view, uint8_t *frames, void *stream,
-                       int *done, int tail_mode, long long *trace) {
+                       int *done, long long *trace) {
   if (!p || !valid_state(st) || !frames || n_envs < 0) return MOOG_E_INVAL;
   if (!p->hdr[MOOG_H_R_ENABLED]) return MOOG_E_INVAL;
   const int32_t *v = p->view[view];
@@ -591,8 +536,7 @@ static int render_impl(moog_program *p, const moog_state *st, int n_envs, int vi
     a.ksize_v = p->ksize_v[view];
   }
   int launches = 0;
-  cudaError_t err =
-      moog::launch_render(a, p->plan[view], v, (cudaStream_t)stream, &launches, done, n_envs, tail_mode, p->opt);
+  cudaError_t err = moog::launch_render(a, p->plan[view], v, (cudaStream_t)stream, &launches, done, n_envs);
   g_launches += launches;
   return err == cudaSuccess ? 0 : cuda_fail(err);
 }

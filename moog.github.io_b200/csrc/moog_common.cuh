@@ -42,16 +42,15 @@ struct StepArgs {
   int S, L, K, VT, NF, CMW;  // program dimensions (filled in by launch_step from the header)
   int dcv_tile;              // contained vertices per pass of the directed search (launch_step)
   const int *order;          // [n_envs] env handled by CTA i, or nullptr = identity
-  int first, count;          // this launch covers dispatch positions [first, first + count)
   int *cost;                 // [n_envs] SM cycles >> 6 this call cost each env, or nullptr
   int *done;                 // nullptr or [1 + n_envs], zeroed: count, then env + 1 in finishing order
   int *sm_active;            // nullptr or [256], zeroed: envs being stepped on each SM right now
   int trace;                 // MOOG_TRACE_TIMES=1: io.counters[n][6..7] = globaltimer at start / finish
   moog_step_io io;
-  // io.frames, drawn by the step kernel itself (launch_step decides): shared-memory offset of
-  // the renderer's buffers behind the part of the env record it reads
-  int fused_render, render_off;
+  // io.frames when the step kernel draws them itself (StepPlan::fuse), else nullptr, and the
+  // shared-memory offset of the renderer's buffers behind the part of the env record it reads
   uint8_t *frames;
+  int render_off;
   moog_state pool;  // valid iff io.pool != nullptr
   // MODE_OVERLAP
   int layer_a, layer_b;
@@ -81,12 +80,6 @@ struct ObserveArgs {
 struct LaunchOptions {
   int helper = -1;            // "helper": second warp per env for one direction of _get_collision_vectors
   int ctas_per_sm = 0;        // "ctas_per_sm": envs resident per SM (the shared-memory request is padded to cap it)
-  int smem_pad = 0;           // "smem_pad": bytes added to the request instead
-  int fused_render = -1;      // "fused_render": the step CTAs draw their env's frame themselves
-  int tail_render = 2;        // "tail_render": 0 render after the step, 1 / 2 behind it (programmatic launch; 2 persistent)
-  int tail_ctas_per_sm = 0;   // "tail_ctas_per_sm"
-  int tail_busy_thr = 1;      // "tail_busy_thr": envs stepped on an SM from which its render CTAs stand back
-  int render_epb = 0;         // "render_epb": envs per CTA of the stand-alone render kernel
   int trace_times = 0;        // "trace_times": per-env globaltimer stamps in io.counters (diagnostic)
   int seed = 0;               // "seed": the draws of moog_env_post_reset (which has no io.seed of its own)
 };
@@ -97,18 +90,20 @@ bool set_launch_option(LaunchOptions &o, const char *name, int value);
 constexpr int kMaxForceOps = 32;
 int env_smem_bytes(const int32_t *hdr, bool helper = true);
 int candidate_matrix_words(const void *host_blob);
-// [first, first + count): dispatch positions covered by this launch (count < 0: all);
-// resident_envs_per_sm > 0 pads the shared-memory request so that at most that many envs
-// share an SM; helper: every env's CTA gets a second warp that runs one direction of
-// _get_collision_vectors next to its owner
-struct StepPlan { size_t smem; bool fuse; int render_off; };
-// frames_mode: 0 no frames, 1 frames (fused only when MOOG_FUSED_RENDER=1), 2 frames, fused preferred
-StepPlan plan_step(const int32_t *host_hdr, int resident_envs_per_sm, bool helper, int frames_mode,
-                   const LaunchOptions &opt = LaunchOptions());
-// *fused (optional): whether the kernel also drew a.io.frames (else the caller runs launch_render)
-cudaError_t launch_step(const StepArgs &a, const int32_t *host_hdr, cudaStream_t stream, int *n_launches,
-                        int first = 0, int count = -1, int resident_envs_per_sm = 0, bool helper = false,
-                        int frames_mode = 0, bool *fused = nullptr, const LaunchOptions &opt = LaunchOptions());
+// How a step call launches its batch (plan_step is the one place that decides it).
+struct StepPlan {
+  bool ordered;    // envs dispatched longest-first by the costs of the previous call (launch_order)
+  int resident;    // envs resident per SM the shared-memory request is padded to (0: as many as fit)
+  bool helper;     // every env's CTA gets a second warp for one direction of _get_collision_vectors
+  size_t smem;     // dynamic shared memory of one step CTA
+  bool fuse;       // the step kernel draws io.frames itself, its canvas at render_off
+  int render_off;
+  bool tail;       // io.frames drawn by the persistent tail render kernel behind the step (StepArgs::done)
+};
+// mode: StepMode; frames: io.frames wanted (MODE_ENV_STEP); sms: multiprocessors of the device
+StepPlan plan_step(const int32_t *host_hdr, int mode, int n_envs, bool frames, int sms, const LaunchOptions &opt);
+cudaError_t launch_step(const StepArgs &a, const int32_t *host_hdr, const StepPlan &plan, cudaStream_t stream,
+                        int *n_launches);
 cudaError_t launch_order(const int *cost, int *order, int n, cudaStream_t stream, int *n_launches);
 int resample_tables(int H, int W, int OH, int OW, std::vector<int> &table, int *ksize_h, int *ksize_v);
 int lanczos_ksize(int in_size, int out_size);
@@ -120,16 +115,16 @@ int lanczos_ksize(int in_size, int out_size);
 struct RenderPlan { bool ok; int rows, ring, P, T, env_bytes; };
 RenderPlan render_plan(const int32_t *host_hdr, const int32_t *host_view);
 // done: nullptr, or the finished-env list of the step kernel launched just before on `stream`
-// (StepArgs::done): the render kernel is then launched with programmatic stream serialization,
-// starts while the last envs are still being stepped and draws the envs in finishing order.
+// (StepArgs::done, with StepArgs::sm_active behind it): the persistent tail render kernel is then
+// launched with programmatic stream serialization, starts while the last envs are still being
+// stepped and draws the envs in finishing order.
 // plan: render_plan of the view (the program keeps one per view); host_view: the host copy of the
 // words at a.view_off (the view's settings)
 cudaError_t launch_render(const RenderArgs &a, const RenderPlan &plan, const int32_t *host_view, cudaStream_t stream,
-                          int *n_launches, int *done = nullptr, int n_done = 0, int tail_mode = 1,
-                          const LaunchOptions &opt = LaunchOptions());
+                          int *n_launches, int *done = nullptr, int n_done = 0);
 // moog_observe_sprites (moog_observe.cu): one warp per env
 cudaError_t launch_observe(const ObserveArgs &a, cudaStream_t stream, int *n_launches);
-// ints behind the finished list that launch_render's tail kernels use: a ticket counter and the
+// ints behind the finished list that launch_render's tail kernel uses: a ticket counter and the
 // per-SM count of envs being stepped
 constexpr int kTailExtraInts = 1 + 256;
 

@@ -65,49 +65,14 @@ __global__ void moog_render_kernel(RenderArgs a, int T, int envs_per_block, int 
 
 // The same for the envs of a step kernel that is still running (launched behind it with
 // programmatic stream serialization: this grid starts once every step CTA is resident or done, so
-// its CTAs land on the SMs the step has no more envs for).  CTA b draws the b-th env to finish:
-// thread 0 waits for entry b of the step kernel's finished list (acquire; the step kernel releases
-// it after the env's record is in HBM).  Every env it could wait for is running or done, so the
-// wait is bounded by the step itself; the poll limit only turns a broken launch into an error.
-template <bool AA>
-__global__ void moog_render_tail_kernel(RenderArgs a, int T, int P, const int *done, int rows, int ring) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  __shared__ int s_env;
-  if (threadIdx.x == 0) {
-    int v = 0;
-    for (unsigned polls = 0;; ++polls) {
-      asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(done + 1 + blockIdx.x) : "memory");
-      if (v != 0) break;
-      if (polls > (1u << 24)) __trap();
-      __nanosleep(200);
-    }
-    s_env = v - 1;
-  }
-  __syncthreads();
-  const int n = s_env;
-  ProgramView pv = view_of(a.blob);
-  const int32_t *view = pv.hdr + a.view_off;
-  const int OH = view[MOOG_V_HEIGHT], OW = view[MOOG_V_WIDTH];
-  const size_t row = (size_t)n;
-  const RenderSrc src = env_src(a, pv, view, row);
-  unsigned long long tr0 = 0;
-  if (a.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tr0));
-  draw_env<AA>(a, src, smem_raw, (int)threadIdx.x, T, P, true, a.frames + row * OH * OW * 3, rows, ring);
-  if (a.trace && threadIdx.x == 0) {
-    unsigned long long tr1;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tr1));
-    a.trace[MOOG_N_COUNTERS * row + 4] = (long long)tr0;
-    a.trace[MOOG_N_COUNTERS * row + 5] = (long long)tr1;
-  }
-  // this grid must not complete before the step grid has (what follows on the stream waits for
-  // this grid only): the CTA that drew the last env to finish waits for the step grid's completion
-  if (blockIdx.x == gridDim.x - 1) asm volatile("griddepcontrol.wait;" ::: "memory");
-}
-
-// Persistent variant: a few CTAs per SM take tickets for the entries of the finished list, and a
-// CTA takes none while its own SM is still stepping envs (sm_active, kept by the step kernel) -- a
-// renderer next to a long-running env slows down exactly the env the whole step is waiting for.
-// The frames are drawn on the SMs the step has left, the last env's by whichever CTA is free.
+// its CTAs land on the SMs the step has no more envs for).  A few CTAs per SM take tickets for the
+// entries of the finished list, and a CTA takes none while its own SM is still stepping an env
+// (sm_active, kept by the step kernel) -- a renderer next to a long-running env slows down exactly
+// the env the whole step is waiting for.  The frames are drawn on the SMs the step has left, the
+// last env's by whichever CTA is free.  A ticket's CTA waits for its entry of the finished list
+// (acquire; the step kernel releases it after the env's record is in HBM).  Every env it could wait
+// for is running or done, so the wait is bounded by the step itself; the poll limit only turns a
+// broken launch into an error.
 template <bool AA>
 __global__ void moog_render_tail_persistent_kernel(RenderArgs a, int T, int P, int *done, int n_done, int busy_thr,
                                                    int rows, int ring) {
@@ -164,7 +129,9 @@ __global__ void moog_render_tail_persistent_kernel(RenderArgs a, int T, int P, i
       a.trace[MOOG_N_COUNTERS * row + 5] = (long long)tr1;
     }
   }
-  if (last) asm volatile("griddepcontrol.wait;" ::: "memory");  // see moog_render_tail_kernel
+  // this grid must not complete before the step grid has (what follows on the stream waits for
+  // this grid only): the CTA that drew the last env to finish waits for the step grid's completion
+  if (last) asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
 // ---------------------------------------------------------------------------
@@ -288,7 +255,7 @@ static cudaError_t allow_smem(K kernel, size_t smem, size_t &configured) {
 
 template <bool AA>
 static cudaError_t launch_render_t(const RenderArgs &a, const RenderPlan &plan, cudaStream_t stream, int *n_launches,
-                                   int *done, int n_done, int tail_mode, const LaunchOptions &opt) {
+                                   int *done, int n_done) {
   const int T = plan.T, P = plan.P, rows = plan.rows, ring = plan.ring;
   const size_t env_bytes = (size_t)plan.env_bytes;
   // envs per CTA: the split that keeps the most envs resident per SM (228 KB of shared
@@ -302,7 +269,6 @@ static cudaError_t launch_render_t(const RenderArgs &a, const RenderPlan &plan, 
       const int envs = (int)(233472 / per_cta) * c;
       if (envs >= best) { best = envs; epb = c; }
     }
-    if (opt.render_epb > 0) epb = opt.render_epb;
   }
   size_t smem = env_bytes * epb;
   if (smem > 224 * 1024) return cudaErrorInvalidConfiguration;
@@ -310,15 +276,23 @@ static cudaError_t launch_render_t(const RenderArgs &a, const RenderPlan &plan, 
   cudaError_t err = allow_smem(moog_render_kernel<AA>, smem, configured);
   if (err != cudaSuccess) return err;
   if (done) {
-    // one env per CTA, in finishing order, overlapping the tail of the step kernel
+    // one env per CTA at a time, in finishing order, overlapping the tail of the step kernel
     smem = env_bytes;
-    static size_t configured_tail = 0, configured_pers = 0;
-    err = tail_mode == 2 ? allow_smem(moog_render_tail_persistent_kernel<AA>, smem, configured_pers)
-                         : allow_smem(moog_render_tail_kernel<AA>, smem, configured_tail);
+    static size_t configured_tail = 0;
+    err = allow_smem(moog_render_tail_persistent_kernel<AA>, smem, configured_tail);
     if (err != cudaSuccess) return err;
+    // as many CTAs per SM as its shared memory and threads hold, no more than there are envs
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    int per_sm = (int)(233472 / (smem + 1024));
+    const int by_threads = 2048 / T;
+    if (per_sm > by_threads) per_sm = by_threads;
+    if (per_sm < 1) per_sm = 1;
+    const int grid = sms * per_sm < n_done ? sms * per_sm : n_done;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3((unsigned)a.n_envs);
+    cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3((unsigned)T);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = stream;
@@ -327,24 +301,9 @@ static cudaError_t launch_render_t(const RenderArgs &a, const RenderPlan &plan, 
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (tail_mode == 2) {
-      int dev = 0, sms = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-      int per_sm = (int)(233472 / (smem + 1024));
-      const int by_threads = 2048 / T;
-      if (per_sm > by_threads) per_sm = by_threads;
-      if (per_sm < 1) per_sm = 1;
-      if (opt.tail_ctas_per_sm > 0 && opt.tail_ctas_per_sm < per_sm) per_sm = opt.tail_ctas_per_sm;
-      int grid = sms * per_sm;
-      if (grid > n_done) grid = n_done;
-      cfg.gridDim = dim3((unsigned)grid);
-      const int busy_thr = opt.tail_busy_thr > 0 ? opt.tail_busy_thr : 1;  // envs being stepped on an SM from which its render CTAs stand back
-      err = cudaLaunchKernelEx(&cfg, moog_render_tail_persistent_kernel<AA>, a, T, P, done, n_done, busy_thr, rows,
-                               ring);
-    } else {
-      err = cudaLaunchKernelEx(&cfg, moog_render_tail_kernel<AA>, a, T, P, (const int *)done, rows, ring);
-    }
+    // busy_thr = 1: no ticket while the SM steps any env (an argument: as a constant in the kernel it
+    // costs the anti-aliased variant two registers)
+    err = cudaLaunchKernelEx(&cfg, moog_render_tail_persistent_kernel<AA>, a, T, P, done, n_done, 1, rows, ring);
     if (n_launches) *n_launches += 1;
     return err;
   }
@@ -355,11 +314,11 @@ static cudaError_t launch_render_t(const RenderArgs &a, const RenderPlan &plan, 
 }
 
 cudaError_t launch_render(const RenderArgs &a, const RenderPlan &plan, const int32_t *view, cudaStream_t stream,
-                          int *n_launches, int *done, int n_done, int tail_mode, const LaunchOptions &opt) {
+                          int *n_launches, int *done, int n_done) {
   if (a.n_envs <= 0) return cudaSuccess;
   if (!plan.ok) return cudaErrorInvalidConfiguration;  // render_impl refuses such a view before
-  return view[MOOG_V_AA] > 1 ? launch_render_t<true>(a, plan, stream, n_launches, done, n_done, tail_mode, opt)
-                             : launch_render_t<false>(a, plan, stream, n_launches, done, n_done, tail_mode, opt);
+  return view[MOOG_V_AA] > 1 ? launch_render_t<true>(a, plan, stream, n_launches, done, n_done)
+                             : launch_render_t<false>(a, plan, stream, n_launches, done, n_done);
 }
 
 }  // namespace moog

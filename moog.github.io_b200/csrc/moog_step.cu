@@ -68,13 +68,9 @@ struct SmemLayout {
 /* contained vertices per pass of _directed_collision_vectors: one pass covers any outline when the
    step is bound by its longest env (few envs per SM, shared memory to spare); the small tile keeps
    the record small when the batch is large and residency is what counts */
-#ifndef DCV_TILE_MAX
 #define DCV_TILE_MAX 32
-#endif
 #define DCV_TILE_MIN 8
-#ifndef DCV_U
 #define DCV_U 2 /* vertices (x edges) per trip of stage A1 of the directed search */
-#endif
 #define NEAR_SKIN 0.02
 #define NEAR_CAP 512  /* near-list entries; more near pairs than this -> every pair is tested */
 
@@ -1561,11 +1557,7 @@ __device__ inline void collision_op(const Env &e, const moog_op *op, int f, int 
         ctr_add(e, CT_CALLS, -1);  // collision_step counts this pair's first call itself
         int moved = collision_step(e, op, s0, s1, true);
         if (moved) {
-#ifdef MOOG_FULL_REFRESH  // diagnostic build: every listed pair re-evaluated after a contact
-          refresh_candidates(e, n_cmask_words);
-#else
           refresh_candidates_moved(e, n_cmask_words, s0, s1, moved);
-#endif
           // continue after (i, w, l) with the refreshed matrix
           m = M[wi] & ~((2u << l) - 1u);
           nz = __ballot_sync(FULL, widx < nwords && M[widx] != 0u) & ~((2u << t) - 1u);
@@ -3537,7 +3529,7 @@ __device__ __forceinline__ void owner_warp(const StepArgs &a, unsigned char *sme
   // CTAs are dispatched in blockIdx order: with `order` the envs that were the most
   // expensive on the previous call go first, so the longest-running env does not
   // start in the last wave (longest-processing-time-first)
-  const int n = a.order ? a.order[a.first + blockIdx.x] : a.first + (int)blockIdx.x;
+  const int n = a.order ? a.order[blockIdx.x] : (int)blockIdx.x;
   const long long t_begin = clock64();
   unsigned long long trace_t0 = 0;
   if (a.trace) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(trace_t0));
@@ -3734,7 +3726,6 @@ __global__ void __launch_bounds__(64) moog_step_kernel(const StepArgs a) {
   // kernel, moog_render.cu) may start as soon as every CTA of this grid has got here, i.e. once
   // no env is waiting for an SM any more; it consumes the envs in the order they finish (a.done).
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  if ((int)blockIdx.x >= a.count) return;
   if (threadIdx.x >= 32) {
     // Helper warp (launched when the step is bound by its longest-running env and the SMs
     // have registers to spare): sleeps on a named barrier until the owner posts a request,
@@ -3753,10 +3744,7 @@ __global__ void __launch_bounds__(64) moog_step_kernel(const StepArgs a) {
   } else {
     owner_warp(a, smem_raw, lane);
   }
-#ifdef MOOG_NO_FUSED_RENDER  // diagnostic build: the step kernel without the renderer's code
-  return;
-#else
-  if (!a.fused_render) return;
+  if (!a.frames) return;
   // PILRenderer.__call__ (pil_renderer.py:88-120) of the state the env was left in, by every
   // thread of the CTA, from the record that is still in shared memory: the canvas, edge lists and
   // int vertices go where the step's scratch was, the item spans into the vertex cache once the
@@ -3777,7 +3765,6 @@ __global__ void __launch_bounds__(64) moog_step_kernel(const StepArgs a) {
     render_env(src, lay, smem_raw + a.render_off, (unsigned *)e.vtx, (int)threadIdx.x, T, P, true,
                a.frames + (size_t)e.env_id * OH * OW * 3, [] { __syncthreads(); });
   }
-#endif
 }
 
 // order[] = env indices by decreasing cost[] (bucket sort; the order inside a bucket
@@ -3818,71 +3805,74 @@ cudaError_t launch_order(const int *cost, int *order, int n, cudaStream_t stream
   return cudaGetLastError();
 }
 
-// Shared-memory request of one step CTA and whether the CTA also draws its env's frame.
-StepPlan plan_step(const int32_t *hdr, int resident_envs_per_sm, bool helper, int frames_mode, const LaunchOptions &opt) {
-  StepPlan plan;
-  size_t smem = (size_t)env_smem_bytes(hdr, helper);
-  {
-    // Resident CTAs (= envs) per SM.  The step is bound by its longest-running env, and a
-    // warp runs ~2.4x slower next to 11 others than alone (profiles/README.md), so beyond
-    // the point where every SM has work, fewer co-resident envs finish the step sooner.  The
-    // dynamic shared-memory request is padded to cap the residency (option "ctas_per_sm"
-    // overrides; "smem_pad" = <bytes> pads directly).
-    const int target = opt.ctas_per_sm > 0 ? opt.ctas_per_sm : resident_envs_per_sm;
-    if (opt.smem_pad > 0) {
-      smem += (size_t)opt.smem_pad;
-    } else if (target > 0 && (size_t)233472 / (smem + 1024) > (size_t)target) {
-      // (when the records alone allow exactly `target` envs nothing is padded, and the SM keeps
-      // the shared memory it does not need as L1: launch_step sets the carve-out)
-      size_t per_cta = (size_t)233472 / (size_t)target;  // 228 KB per SM, 1 KB of it reserved per CTA
-      if (per_cta > 1024 + smem) smem = ((per_cta - 1024) & ~(size_t)127);
-      if (smem > 227 * 1024) smem = 227 * 1024;
-    }
+// How a step call launches a batch of n_envs on a device with `sms` multiprocessors.
+StepPlan plan_step(const int32_t *hdr, int mode, int n_envs, bool frames, int sms, const LaunchOptions &opt) {
+  StepPlan p = {};
+  // Longest-processing-time-first dispatch from the costs of the previous call (moog_order_kernel):
+  // a large batch runs in waves, and the env that was the most expensive must not start in the last one.
+  p.ordered = (mode == MODE_ENV_STEP || mode == MODE_PHYSICS) && n_envs >= 1024;
+  // The step ends when its longest-running env does, and a warp runs ~2.4x slower next to 11
+  // others than alone (profiles/README.md): with the envs dispatched longest-first, capping
+  // the envs resident per SM at about n_envs / (5.5 .. 7 x SMs) finishes the step sooner than filling
+  // the SMs (4096 envs on 148 SMs: 5 per SM; measured with the frames drawn behind the step, step
+  // + render per 4096 envs: 3: 5.33 ms, 4: 4.66 ms, 5: 4.46 ms, and 5.6 ms at 12 with one warp per env).
+  // In that regime the SMs have registers to spare, and every env gets a helper warp that
+  // computes one of the two directions of _get_collision_vectors (option "helper" overrides).
+  if (sms > 0) {
+    int resident = (n_envs + 7 * sms / 2) / (7 * sms);  // n_envs / (7 x SMs), rounded
+    // helper-warp regime (few envs per SM): one more env per SM pays once the frames are drawn
+    // behind the step (4096 envs: 4 -> 5 per SM, 4.66 -> 4.46 ms); larger batches keep 7 waves
+    // (8192 / 32768 envs measured slower at 10 / 40 per SM than at 8 / 32)
+    if (resident <= 4) resident = (2 * n_envs + 11 * sms / 2) / (11 * sms);
+    if (resident < 2) resident = 2;
+    p.helper = resident <= 6;
+    if (p.ordered) p.resident = resident;
+  }
+  if (opt.helper >= 0) p.helper = opt.helper != 0;
+  if (opt.ctas_per_sm > 0) p.resident = opt.ctas_per_sm;
+  // The residency cap is a padded dynamic shared-memory request (option "ctas_per_sm" sets the cap).
+  size_t smem = (size_t)env_smem_bytes(hdr, p.helper);
+  if (p.resident > 0 && (size_t)233472 / (smem + 1024) > (size_t)p.resident) {
+    // (when the records alone allow exactly `resident` envs nothing is padded, and the SM keeps
+    // the shared memory it does not need as L1: launch_step sets the carve-out)
+    size_t per_cta = (size_t)233472 / (size_t)p.resident;  // 228 KB per SM, 1 KB of it reserved per CTA
+    if (per_cta > 1024 + smem) smem = ((per_cta - 1024) & ~(size_t)127);
+    if (smem > 227 * 1024) smem = 227 * 1024;
   }
   // The frame of the state the env is left in (io.frames), drawn by the env's own CTA right after
-  // its step: the renderer reads the record where it lies in shared memory and builds its canvas
-  // where the step's scratch was.  frames_mode 2 = the caller prefers it (small batches: one
-  // launch, no second pass over the state), 1 = frames wanted but the render kernel is the better
-  // choice: measured on 4096 falling_balls20 envs, two warps per env drawing between the steps of
-  // their neighbours cost more (6.0 ms) than the render kernel behind the step (4.3 + 0.55 ms).
-  // Option "fused_render" = 0 never fuses, = 1 fuses whenever one CTA can hold a canvas.
-  plan.render_off = 0;
-  plan.fuse = false;
-  if (frames_mode > 0 && hdr[MOOG_H_R_ENABLED] && hdr[MOOG_H_R_AA] == 1) {
+  // its step when one CTA can hold the canvas: the renderer reads the record where it lies in shared
+  // memory and builds its canvas where the step's scratch was.  Small batches (every env has an SM
+  // to itself) gain one launch and no second pass over the state; for large ones the render kernel is
+  // the better choice: measured on 4096 falling_balls20 envs, two warps per env drawing between the
+  // steps of their neighbours cost more (6.0 ms) than the render kernel behind the step (4.3 + 0.55 ms).
+  if (frames && n_envs <= 2 * sms && hdr[MOOG_H_R_ENABLED] && hdr[MOOG_H_R_AA] == 1) {
     const int VTr = hdr[MOOG_H_N_VTX] > 0 ? hdr[MOOG_H_N_VTX] : 1;
     const SmemLayout sl = smem_layout(hdr[MOOG_H_N_SLOTS], VTr, hdr[MOOG_H_N_ENVF], hdr[MOOG_H_CMASK_WORDS],
-                                      helper ? 2 : 1, helper ? DCV_TILE_MAX : DCV_TILE_MIN);
+                                      p.helper ? 2 : 1, p.helper ? DCV_TILE_MAX : DCV_TILE_MIN);
     const int C = hdr[MOOG_H_R_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
     const RenderLayout rl = render_layout(hdr[MOOG_H_R_HEIGHT], hdr[MOOG_H_R_WIDTH], hdr[MOOG_H_N_SLOTS] * C, VTr * C,
                                           hdr[MOOG_H_R_WIDTH], 16 * VTr);
-    plan.render_off = (sl.scratch + 15) & ~15;  // everything from the warps' scratch on is dead after the step
-    const size_t need = (size_t)plan.render_off + (size_t)rl.total;
-    bool want = frames_mode == 2;
-    if (opt.fused_render >= 0) want = opt.fused_render != 0;
-#ifdef MOOG_NO_FUSED_RENDER
-    want = false;
-#endif
-    if (want && need <= 227 * 1024) {
-      plan.fuse = true;
+    const int render_off = (sl.scratch + 15) & ~15;  // everything from the warps' scratch on is dead after the step
+    const size_t need = (size_t)render_off + (size_t)rl.total;
+    if (need <= 227 * 1024) {
+      p.fuse = true;
+      p.render_off = render_off;
       if (smem < need) smem = need;
     }
   }
-  plan.smem = smem;
-  return plan;
+  p.smem = smem;
+  // Frames of a large batch: the step ends when its longest-running env does, and long before
+  // that most SMs have no env left to step.  The render kernel is launched behind the step kernel
+  // with programmatic stream serialization, starts as soon as the last env has got an SM, and
+  // draws the envs in the order they finish (the `done` list) on the SMs the step left idle.
+  p.tail = frames && p.ordered && !p.fuse;
+  return p;
 }
 
-cudaError_t launch_step(const StepArgs &a, const int32_t *hdr, cudaStream_t stream, int *n_launches, int first,
-                        int count, int resident_envs_per_sm, bool helper, int frames_mode, bool *fused,
-                        const LaunchOptions &opt) {
-  if (fused) *fused = false;
-  if (count < 0) count = a.n_envs - first;
-  if (a.n_envs <= 0 || count <= 0) return cudaSuccess;
-  const StepPlan plan = plan_step(hdr, resident_envs_per_sm, helper,
-                                  a.io.frames != nullptr && a.mode == MODE_ENV_STEP ? frames_mode : 0, opt);
+cudaError_t launch_step(const StepArgs &a, const int32_t *hdr, const StepPlan &plan, cudaStream_t stream,
+                        int *n_launches) {
+  if (a.n_envs <= 0) return cudaSuccess;
   const size_t smem = plan.smem;
-  const bool fuse = plan.fuse;
-  const int render_off = plan.render_off;
-  if (fused) *fused = fuse;
   static size_t configured = 0;
   if (smem > configured) {
     cudaError_t err = cudaFuncSetAttribute(moog_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -3905,21 +3895,17 @@ cudaError_t launch_step(const StepArgs &a, const int32_t *hdr, cudaStream_t stre
       carve_set = pct;
     }
   }
-  int blocks = count;
   StepArgs b = a;
-  b.first = first;
-  b.count = count;
   b.S = hdr[MOOG_H_N_SLOTS];
   b.L = hdr[MOOG_H_N_LAYERS];
   b.K = hdr[MOOG_H_K];
   b.VT = hdr[MOOG_H_N_VTX];
   b.NF = hdr[MOOG_H_N_ENVF];
   b.CMW = hdr[MOOG_H_CMASK_WORDS];
-  b.dcv_tile = helper ? DCV_TILE_MAX : DCV_TILE_MIN;
-  b.fused_render = fuse ? 1 : 0;
-  b.render_off = render_off;
-  b.frames = fuse ? a.io.frames : nullptr;
-  moog_step_kernel<<<blocks, helper ? 64 : 32, smem, stream>>>(b);
+  b.dcv_tile = plan.helper ? DCV_TILE_MAX : DCV_TILE_MIN;
+  b.render_off = plan.render_off;
+  b.frames = plan.fuse ? a.io.frames : nullptr;
+  moog_step_kernel<<<a.n_envs, plan.helper ? 64 : 32, smem, stream>>>(b);
   if (n_launches) *n_launches += 1;
   return cudaGetLastError();
 }

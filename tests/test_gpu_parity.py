@@ -576,19 +576,18 @@ def test_step_kernel_draws_the_same_frames_as_the_render_kernel(scene, helper, m
     env in from the record in shared memory (owner + helper warp, or the owner alone).  Along
     the golden trajectory the frames must equal what `moog_render` draws from the stored state
     afterwards -- which the tests above pin to PILRenderer's output -- and the state must not
-    notice.  MOOG_FUSED_RENDER=1 forces the fused path wherever one CTA can hold a canvas; where
-    it cannot (big canvases, TorusGeometry's 9 copies, anti-aliasing) the call falls back to the
-    render kernel, and the frames must be the same as well."""
+    notice.  A batch of 5 envs draws inside the step kernel wherever one CTA can hold the canvas,
+    which every scene here does."""
     g = util.load_golden(scene)
     prog = g['program']
     if prog.render is None:
         pytest.skip('scene has no renderer')
-    monkeypatch.setenv('MOOG_FUSED_RENDER', '1')
     monkeypatch.setenv('MOOG_HELPER', helper)
     T = min(len(g['reward']), 30)
     n = 5
     arrays = {k: np.concatenate([util.state_at(g, None, prefix='init')[k]] * n, axis=0) for k in util.STATE_KEYS}
     engines = [_engine(prog, arrays), _engine(prog, arrays)]
+    assert engines[0].dev_program.step_draws_frames(n), (scene, helper)
     for eng in engines:
         eng.post_reset()
     host = torch.zeros(tuple(engines[0].frames.shape), dtype=torch.uint8).pin_memory()

@@ -85,6 +85,29 @@ def test_device_path_has_no_cpu_fallback():
         Engine(g['program'], 4, 'cuda:0')
 
 
+@pytest.mark.gpu
+def test_set_option_takes_the_launch_options_and_refuses_other_names():
+    """moog_program_set_option changes "helper", "ctas_per_sm", "trace_times" and "seed" of a live
+    program and returns MOOG_E_INVAL for any other name, such as the launch options that used to
+    select a code path or a size the library picks itself."""
+    import moog_b200  # noqa: F401
+    from moog_b200 import capi
+    prog = capi.DeviceProgram(util.load_golden('falling_balls20')['program'].blob)
+    L = capi.lib()
+
+    def set_option(name, value):
+        return L.moog_program_set_option(prog.handle, name.encode(), value)
+
+    for name, value in (('helper', 0), ('ctas_per_sm', 3), ('trace_times', 1), ('seed', 7)):
+        assert set_option(name, value) == 0, name
+    assert prog.step_launch_info(4096)[:2] == (3, 1)
+    for name, value in (('helper', -1), ('ctas_per_sm', 0), ('trace_times', 0), ('seed', 0)):
+        assert set_option(name, value) == 0, name
+    for name in ('tail_render', 'fused_render', 'smem_pad', 'render_epb', 'tail_ctas_per_sm', 'tail_busy_thr'):
+        assert set_option(name, 1) == capi.E_INVAL, name
+    prog.close()
+
+
 def test_product_package_never_touches_the_oracle():
     pkg = os.path.join(ROOT, 'moog.github.io_b200')
     for dirpath, _, files in os.walk(pkg):

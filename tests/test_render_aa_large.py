@@ -273,26 +273,25 @@ def _oracle_frames(prog, arrays):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize('tail', [1, 2])
+@pytest.mark.parametrize('n', [1024, 6])
 @pytest.mark.parametrize('scene', util.AA_SCENES)
-def test_step_call_frames(scene, tail):
-    """moog_env_step with frames at 1024 envs (the render behind the step, tail_render 1 / 2) and at 6
-    envs, at every listed size: the frames are the oracle's render of the state each env was left in."""
+def test_step_call_frames(scene, n):
+    """moog_env_step with frames at 1024 envs (the persistent render kernel behind the step) and at 6
+    envs (the render kernel after it), at every listed size: the frames are the oracle's render of the
+    state each env was left in."""
     import torch
     g = util.load_golden(scene)
     steps = _steps(g, 8)
     one = _states(g, steps)
     for w, h, aa in SIZES + [(75, 50, 3)]:
         prog = _program(g, w, h, aa)
-        for n in (1024, 6):
-            idx = np.arange(n) % len(steps)
-            eng = _engine(prog, {k: v[idx] for k, v in one.items()})
-            eng.dev_program.set_option('tail_render', tail)
-            eng.env_step(np.zeros((n, max(prog.action_dim, 1))), auto_reset=False, frames=True)
-            got = eng.frames.cpu().numpy()
-            torch.cuda.synchronize()
-            want = _oracle_frames(prog, eng.state.download())
-            assert int((got != want).sum()) == 0, (scene, w, h, aa, n, tail)
+        idx = np.arange(n) % len(steps)
+        eng = _engine(prog, {k: v[idx] for k, v in one.items()})
+        eng.env_step(np.zeros((n, max(prog.action_dim, 1))), auto_reset=False, frames=True)
+        got = eng.frames.cpu().numpy()
+        torch.cuda.synchronize()
+        want = _oracle_frames(prog, eng.state.download())
+        assert int((got != want).sum()) == 0, (scene, w, h, aa, n)
 
 
 @pytest.mark.gpu
