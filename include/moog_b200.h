@@ -145,6 +145,23 @@ int moog_render_view(moog_program *p, const moog_state *st, int n_envs, int view
  * before launching anything). */
 int moog_render_plan(const void *blob, size_t nbytes, int view, int *chunk_rows, int *smem_bytes);
 
+/* SpriteMask `mask` of N envs (no reference counterpart; moog_b200_program.h MOOG_H_MASKS): out[N][H][W] int16,
+ * row 0 = top as in the frames, each pixel the slot of the last sprite in draw order whose Pillow polygon
+ * fill covers it (the fill the frames use, at the mask's image size and polygon modifier; sprites whose
+ * ink alpha byte is 0 are left out), -1 where none does.  A launch of its own on `stream`, like
+ * moog_render_view: call it after moog_env_step to draw the masks of the state that call left.  `out` is
+ * any device-accessible address aligned to 16 bytes: HBM, or pinned host memory.  MOOG_E_INVAL for a NULL
+ * program / state / out, n_envs < 0, a misaligned out or a mask outside [0, hdr[MOOG_H_N_MASKS]);
+ * MOOG_E_UNSUPPORTED for a mask no band holds (moog_mask_plan). */
+int moog_render_mask(moog_program *p, const moog_state *st, int n_envs, int mask, int16_t *out, void *stream);
+
+/* How the mask kernel draws mask `mask` of a program blob, without touching the GPU (like
+ * moog_render_plan): *band_rows rows at a time, *smem_bytes of shared memory per env; either pointer
+ * may be NULL.  0; MOOG_E_INVAL for a malformed blob or a mask outside [0, hdr[MOOG_H_N_MASKS]);
+ * MOOG_E_UNSUPPORTED for a mask no band can hold in one CTA's shared memory (TorusGeometry over outlines
+ * as large as cleanup's). */
+int moog_mask_plan(const void *blob, size_t nbytes, int mask, int *band_rows, int *smem_bytes);
+
 /* RawState.__call__ (moog/observers/raw_state.py:17-19) for N envs: every sprite slot's state as
  * out[N][S][MOOG_OBS_COLS] float32 (layout and columns: moog_b200_program.h MOOG_OBS_*).  A launch of its
  * own on `stream`, so call it after moog_env_step to observe the state that call left.  `out` is any

@@ -130,6 +130,8 @@ enum {
   MOOG_H_METAVAR_INIT = 59, /* dpool index of their values after meta_state_initializer() (environment.py:86) */
   MOOG_H_VIEWS = 60,      /* index in ipool of the view table: MOOG_H_N_VIEWS rows of MOOG_VIEW_WORDS */
   MOOG_H_N_VIEWS = 61,    /* PILRenderer observers after the first (views 1..); 0 = one renderer or none */
+  MOOG_H_MASKS = 62,      /* index in ipool of the mask table: MOOG_H_N_MASKS rows of MOOG_VIEW_WORDS */
+  MOOG_H_N_MASKS = 63,    /* SpriteMask observers (0 = none, and no table) */
   MOOG_H_META_OFF = 56,   /* envf offset of column 0; column k of slot s is envf[off + k * S + s], NaN = no such key.
                              Read as attribute MOOG_AT_META0 + k; travels with the sprite when slots are compacted */
   MOOG_H_CMASK_WORDS = 50 /* 32-bit words of the per-env broad-phase candidate matrices of all
@@ -161,6 +163,14 @@ MOOG_STATIC_ASSERT_(MOOG_H_R_WIDTH - MOOG_H_R_HEIGHT == MOOG_V_WIDTH && MOOG_H_R
                         MOOG_H_R_ENABLED - MOOG_H_R_HEIGHT == MOOG_V_ENABLED && MOOG_V_ENABLED + 1 == MOOG_VIEW_WORDS,
                     "the header's renderer words are a view row");
 #undef MOOG_STATIC_ASSERT_
+
+/* Masks: one per SpriteMask observer, in the order of the config's observers dict, independent of the
+ * views (a program may have masks and no renderer).  Mask k is row k of the mask table,
+ * ipool[hdr[MOOG_H_MASKS] + MOOG_VIEW_WORDS * k ...], in view-row order: MOOG_V_AA = 1, MOOG_V_BG = 0,
+ * MOOG_V_COLORMAP = 0, MOOG_V_MODIFIER / MOOG_V_MOD_LAYER as for a renderer, MOOG_V_ENABLED = 1.  At most
+ * MOOG_MAX_VIEWS masks.  A mask is int16 mask[N][H][W]: the slot of the last sprite in draw order whose
+ * Pillow polygon fill covers the pixel (row 0 = top, as the frames), -1 where none does; sprites whose
+ * ink alpha byte is 0 are not drawn. */
 
 enum { MOOG_CMAP_NONE = 0, MOOG_CMAP_HSV = 1 };
 enum { MOOG_PMOD_NONE = 0, MOOG_PMOD_FIRST_PERSON = 1, MOOG_PMOD_TORUS = 2 };

@@ -12,6 +12,8 @@ num_envs=N)` works on an unchanged MOOG config -- and the same `reset()` /
                                                            PILRenderers under its own key)
                 {key: float32 [N, S, 16]}                 (RawState: every sprite slot, see
                                                            include/moog_b200_program.h MOOG_OBS_*)
+                {key: int16 [N, H, W]}                    (SpriteMask: the slot each pixel shows,
+                                                           -1 for none)
 
 An env whose previous step returned LAST is reset by the next `step()` call and
 ignores that call's action (environment.py:100-101).  Initial states come from
@@ -158,6 +160,9 @@ class Engine(object):
                   for r in views]
         self.frames = frames[0] if frames else None
         self.view_frames = frames[1:]
+        # one int16 [N, H, W] buffer per SpriteMask, in mask order
+        self.masks = [torch.full((self.n, m['height'], m['width']), -1, dtype=torch.int16, device=self.device)
+                      for _, m in getattr(program, 'masks', ())]
         self.sprites = None
         if getattr(program, 'state_key', None) is not None:
             self.sprites = torch.zeros((self.n, program.n_slots, compiler.OBS_COLS), **f32)
@@ -179,6 +184,14 @@ class Engine(object):
                     'observer {!r}: PILRenderer(image_size=({}, {}), anti_aliasing={}) draws a {} x {} canvas, '
                     'and no chunk of it fits the shared memory of one CTA'.format(
                         key, r['width'], r['height'], r['aa'], r['aa'] * r['width'], r['aa'] * r['height']))
+            capi.check(code)
+        for k, (key, m) in enumerate(getattr(program, 'masks', ())):
+            code, _, _ = capi.mask_plan(program.blob, k)
+            if code == capi.E_UNSUPPORTED:
+                raise capi.MoogError(
+                    'observer {!r}: SpriteMask(image_size=({}, {})) cannot be drawn: no band of its rows fits '
+                    'the shared memory of one CTA next to the edge lists of its sprites'.format(
+                        key, m['width'], m['height']))
             capi.check(code)
 
     def call_seed(self):
@@ -329,6 +342,27 @@ class Engine(object):
                     self.dev_program.handle, ctypes.byref(st), count, view, dst, self._stream()))
         return out
 
+    def render_mask(self, out=None, first=0, count=None, mask=0):
+        """SpriteMask `mask` of the envs [first, first + count) into out[first:first + count] (`out` None:
+        the mask's own buffer in `masks`), drawn by `moog_render_mask`: a contiguous int16 [N, H, W]
+        tensor on this device or in pinned host memory, whose range starts 16-byte aligned."""
+        if not 0 <= mask < len(self.masks):
+            raise ValueError('mask {} is outside [0, {})'.format(mask, len(self.masks)))
+        own = self.masks[mask]
+        out = own if out is None else out
+        count = self.n - first if count is None else count
+        if first < 0 or count < 0 or first + count > self.n:
+            raise ValueError('env range [{}, {}) is outside [0, {})'.format(first, first + count, self.n))
+        if out.dtype != torch.int16 or tuple(out.shape) != tuple(own.shape) or not out.is_contiguous():
+            raise ValueError('mask {} must be a contiguous int16 tensor of shape {}'.format(mask, tuple(own.shape)))
+        self._check_reachable(out, 'masks')
+        st = self.state.struct(first)
+        dst = ctypes.c_void_p(out.data_ptr() + first * out.stride(0) * out.element_size())
+        with self._on_device():
+            capi.check(capi.lib().moog_render_mask(
+                self.dev_program.handle, ctypes.byref(st), count, mask, dst, self._stream()))
+        return out
+
     def observe_sprites(self, out=None):
         """`moog_observe_sprites`: RawState (raw_state.py:17-19) of every env as float32 [N, S, 16]
         (columns: include/moog_b200_program.h MOOG_OBS_*), into `self.sprites` or `out` -- a
@@ -383,6 +417,7 @@ class BatchedEnvironment(object):
         self._image_keys = [k for k, _ in self.program.views]
         self._image_key = self._image_keys[0] if self._image_keys else None
         self._state_key = self.program.state_key
+        self._mask_keys = [k for k, _ in self.program.masks]   # SpriteMask observers in mask order
         self._rng = np.random.RandomState(seed)
         self._started = False
         self._copy_stream = None
@@ -449,11 +484,12 @@ class BatchedEnvironment(object):
         `host` is a TimeStep of CPU tensors (step_type int32[N], reward float32[N],
         discount float32[N] or None, observation {'image': uint8[N,H,W,3]} -- one such image per
         PILRenderer, under its key -- and, with a RawState observer, its key -> pinned
-        float32[N,S,16]).  Returns `host` once everything has arrived (the caller owns the
-        TimeStep).  The other views and the sprite observation travel like the frames of view 0:
+        float32[N,S,16], and with SpriteMask observers, each key -> pinned int16[N,H,W]).  Returns `host`
+        once everything has arrived (the caller owns the TimeStep).  The other views, the masks and the
+        sprite observation travel like the frames of view 0:
         stored by their kernels straight into the pinned tensors with 'mapped', computed in device
-        memory and copied after it otherwise (with 'chunked': range by range, a view whose frame
-        is not a multiple of 16 bytes in one range).
+        memory and copied after it otherwise (with 'chunked': range by range, a view or mask whose
+        per-env bytes are not a multiple of 16 in one range).
 
         frames = 'mapped': the step call draws every env's frame straight into the pinned host
         image (the kernels' stores cross PCIe while other envs are still being stepped; no
@@ -467,6 +503,7 @@ class BatchedEnvironment(object):
         img = host.observation[self._image_key] if self._image_key is not None else None
         more = [host.observation[k] for k in self._image_keys[1:]]  # views 1..
         spr = host.observation.get(self._state_key) if self._state_key is not None else None
+        masks = [host.observation[k] for k in self._mask_keys]
         auto = frames == 'auto'
         if auto:
             frames = self._auto_frames(img)
@@ -484,6 +521,8 @@ class BatchedEnvironment(object):
                     dst.copy_(src, non_blocking=True)
                 if spr is not None:
                     spr.copy_(e.sprites, non_blocking=True)
+                for dst, src in zip(masks, e.masks):
+                    dst.copy_(src, non_blocking=True)
             else:
                 dst = None if img is None else (img if frames == 'mapped' else True)
                 e.env_step(self._flatten_action(action), sample_resets=(self.reset_mode == 'device'), frames=dst)
@@ -494,6 +533,11 @@ class BatchedEnvironment(object):
                         e.render(out=dst, view=v)
                     else:
                         dst.copy_(e.render(view=v), non_blocking=True)
+                for m, dst in enumerate(masks):
+                    if frames == 'mapped':
+                        e.render_mask(out=dst, mask=m)
+                    else:
+                        dst.copy_(e.render_mask(mask=m), non_blocking=True)
                 if spr is not None:
                     if frames == 'mapped':
                         e.observe_sprites(out=spr)
@@ -518,11 +562,13 @@ class BatchedEnvironment(object):
         host.reward.copy_(e.reward, non_blocking=True)
         if host.discount is not None:
             host.discount.copy_(e.discount, non_blocking=True)
-        if self._image_key is not None:
+        if self._image_key is not None or masks:
             dsts = [host.observation[k] for k in self._image_keys]
-            # a range of a view other than 0 must start 16-byte aligned (moog_render_view): a view
-            # whose frame is not a multiple of 16 bytes is drawn and copied whole with the first range
+            # a range of a view other than 0 or of a mask must start 16-byte aligned (moog_render_view,
+            # moog_render_mask): one whose per-env bytes are not a multiple of 16 is drawn and copied
+            # whole with the first range
             ranged = [v == 0 or e.view_buffer(v)[0].numel() % 16 == 0 for v in range(len(dsts))]
+            mranged = [e.masks[m][0].numel() * 2 % 16 == 0 for m in range(len(masks))]
             chunks = max(1, min(int(chunks), len(self._copy_events), self.num_envs))
             # equal ranges: measured on B200 / PCIe 5 with 4096 64x64 frames, 4 equal ranges beat
             # 1, 2, 8 or 16 ranges and growing / shrinking ones (each render launch has a fixed
@@ -540,12 +586,20 @@ class BatchedEnvironment(object):
                     if span is not None:
                         e.render(first=span[0], count=span[1] - span[0], view=v)
                         spans.append((v, span))
+                mspans = []
+                for m in range(len(masks)):
+                    span = (first, first + count) if mranged[m] else ((0, self.num_envs) if c == 0 else None)
+                    if span is not None:
+                        e.render_mask(first=span[0], count=span[1] - span[0], mask=m)
+                        mspans.append((m, span))
                 ev = self._copy_events[c]
                 ev.record(main)
                 copy.wait_event(ev)
                 with torch.cuda.stream(copy):
                     for v, (a, b) in spans:
                         dsts[v][a:b].copy_(e.view_buffer(v)[a:b], non_blocking=True)
+                    for m, (a, b) in mspans:
+                        masks[m][a:b].copy_(e.masks[m][a:b], non_blocking=True)
                 first += count
         copy.synchronize()
         main.synchronize()
@@ -585,6 +639,8 @@ class BatchedEnvironment(object):
         obs = {}
         for v, key in enumerate(self._image_keys):
             obs[key] = self.engine.render(view=v)
+        for m, key in enumerate(self._mask_keys):
+            obs[key] = self.engine.render_mask(mask=m)
         if self._state_key is not None:
             obs[self._state_key] = self.engine.observe_sprites()
         return obs
@@ -596,6 +652,8 @@ class BatchedEnvironment(object):
             obs = {self._image_key: e.frames} if self._image_key is not None else {}
             for v, key in enumerate(self._image_keys[1:], 1):
                 obs[key] = e.render(view=v)
+            for m, key in enumerate(self._mask_keys):
+                obs[key] = e.render_mask(mask=m)
             if self._state_key is not None:
                 obs[self._state_key] = e.observe_sprites()
         else:
@@ -679,8 +737,8 @@ class HostPipeline(object):
     i.e. the policy acts on an observation that is one step old (the usual actor pipeline); with
     depth 1 it is `step_to_host`.  Every submit copies that step's actions host -> device and
     every collect returns step_type / reward / discount / frames of every PILRenderer (and the
-    RawState observation when the config has one) in pinned host memory, valid until `depth`
-    further submits.  frames = 'mapped': the kernels store the frames and the sprite observation
+    RawState observation and the SpriteMasks when the config has them) in pinned host memory, valid
+    until `depth` further submits.  frames = 'mapped': the kernels store the frames, masks and sprite observation
     straight into the slot's pinned buffers over PCIe; 'device': they are written to HBM and copied
     by a copy engine on a second stream while the next step runs.
     Reference protocol: moog/environment.py:98-126 (one `step` per submit, auto-reset included).
@@ -707,9 +765,14 @@ class HostPipeline(object):
                 obs[key] = imgs[-1]
             if env._state_key is not None:  # pylint: disable=protected-access
                 spr = obs[env._state_key] = pin(*e.sprites.shape, dtype=torch.float32)  # pylint: disable=protected-access
+            masks = []  # one pinned mask per SpriteMask, in mask order
+            for m, key in enumerate(env._mask_keys):  # pylint: disable=protected-access
+                masks.append(pin(*e.masks[m].shape, dtype=torch.int16))
+                obs[key] = masks[-1]
             self._slots.append(dict(
                 ts=TimeStep(pin(n, dtype=torch.int32), pin(n, dtype=torch.float32), pin(n, dtype=torch.float32), obs),
-                imgs=imgs, spr=spr,
+                imgs=imgs, spr=spr, masks=masks,
+                dev_masks=[torch.empty_like(d) for d in e.masks] if frames == 'device' else None,
                 dev_imgs=[torch.empty_like(e.view_buffer(v)) for v in range(len(imgs))] if frames == 'device' else None,
                 dev_sprites=(torch.empty_like(e.sprites) if (spr is not None and frames == 'device') else None),
                 host_act=pin(n, ad, dtype=torch.float64),
@@ -733,6 +796,8 @@ class HostPipeline(object):
                     img.copy_(e.view_buffer(v), non_blocking=True)
                 if slot['spr'] is not None:
                     slot['spr'].copy_(e.sprites, non_blocking=True)
+                for host_mask, dev in zip(slot['masks'], e.masks):
+                    host_mask.copy_(dev, non_blocking=True)
             else:
                 act = None
                 if action is not None:
@@ -748,18 +813,22 @@ class HostPipeline(object):
                 e.env_step(act, sample_resets=(env.reset_mode == 'device'), frames=dsts[0] if dsts else None)
                 for v in range(1, len(dsts)):
                     e.render(out=dsts[v], view=v)
+                for m, dst in enumerate(slot['masks'] if self.frames == 'mapped' else slot['dev_masks']):
+                    e.render_mask(out=dst, mask=m)
                 if slot['spr'] is not None:
                     e.observe_sprites(out=slot['spr'] if self.frames == 'mapped' else slot['dev_sprites'])
             ts = slot['ts']
             ts.step_type.copy_(e.step_type, non_blocking=True)
             ts.reward.copy_(e.reward, non_blocking=True)
             ts.discount.copy_(e.discount, non_blocking=True)
-            if self.frames == 'device' and (slot['imgs'] or slot['spr'] is not None) and not was_reset:
+            if self.frames == 'device' and (slot['imgs'] or slot['masks'] or slot['spr'] is not None) and not was_reset:
                 slot['stepped'].record(self._main)
                 self._copy.wait_event(slot['stepped'])
                 with torch.cuda.stream(self._copy):
                     for img, dev in zip(slot['imgs'], slot['dev_imgs']):
                         img.copy_(dev, non_blocking=True)
+                    for host_mask, dev in zip(slot['masks'], slot['dev_masks']):
+                        host_mask.copy_(dev, non_blocking=True)
                     if slot['spr'] is not None:
                         slot['spr'].copy_(slot['dev_sprites'], non_blocking=True)
                     slot['done'].record(self._copy)

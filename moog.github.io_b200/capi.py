@@ -42,7 +42,7 @@ SYMBOLS = ('moog_program_create', 'moog_program_destroy',
            'moog_host_points_in_path', 'moog_step_launch_info',
            'moog_step_draws_frames', 'moog_program_set_option',
            'moog_program_validate', 'moog_observe_sprites', 'moog_render_view',
-           'moog_render_plan')
+           'moog_render_plan', 'moog_render_mask', 'moog_mask_plan')
 
 
 # include/moog_b200.h return codes
@@ -112,6 +112,10 @@ def lib():
     L.moog_program_validate.restype = ci
     L.moog_render_plan.argtypes = [vp, ctypes.c_size_t, ci, ctypes.POINTER(ci), ctypes.POINTER(ci)]
     L.moog_render_plan.restype = ci
+    L.moog_render_mask.argtypes = [vp, ctypes.POINTER(MoogState), ci, ci, vp, vp]
+    L.moog_render_mask.restype = ci
+    L.moog_mask_plan.argtypes = [vp, ctypes.c_size_t, ci, ctypes.POINTER(ci), ctypes.POINTER(ci)]
+    L.moog_mask_plan.restype = ci
     L.moog_launch_count.argtypes = []
     L.moog_launch_count.restype = ctypes.c_int64
     _lib = L
@@ -138,6 +142,16 @@ def render_plan(blob, view=0):
     buf = ctypes.create_string_buffer(bytes(blob), len(blob))
     rows, smem = ctypes.c_int(), ctypes.c_int()
     code = int(lib().moog_render_plan(buf, len(blob), int(view), ctypes.byref(rows), ctypes.byref(smem)))
+    return code, rows.value, smem.value
+
+
+def mask_plan(blob, mask=0):
+    """How the mask kernel draws mask `mask` of a program blob, without a device
+    (include/moog_b200.h moog_mask_plan): (code, band_rows, smem_bytes); code 0, or
+    E_UNSUPPORTED for a mask no band can hold, or E_INVAL."""
+    buf = ctypes.create_string_buffer(bytes(blob), len(blob))
+    rows, smem = ctypes.c_int(), ctypes.c_int()
+    code = int(lib().moog_mask_plan(buf, len(blob), int(mask), ctypes.byref(rows), ctypes.byref(smem)))
     return code, rows.value, smem.value
 
 

@@ -57,8 +57,9 @@ H_RESET, H_N_RESET, H_N_DPOOL, H_SHAPE_TAB = 51, 52, 53, 54
 H_N_META, H_META_OFF = 55, 56
 H_N_METAVAR, H_METAVAR_OFF, H_METAVAR_INIT = 57, 58, 59
 H_VIEWS, H_N_VIEWS = 60, 61
+H_MASKS, H_N_MASKS = 62, 63
 VIEW_WORDS = 8           # MOOG_VIEW_WORDS: a view table row, the words H_R_HEIGHT .. H_R_ENABLED
-MAX_VIEWS = 8            # MOOG_MAX_VIEWS: PILRenderer observers per program
+MAX_VIEWS = 8            # MOOG_MAX_VIEWS: PILRenderer observers per program, and SpriteMask observers
 MAX_META_VARS = 16
 
 F_DRAG, F_KINETIC_FRICTION, F_DOWN_GRAVITY, F_GRAVITY, F_RANDOM, \
@@ -152,6 +153,7 @@ class Program(object):
         self.voff = [0]          # first cached vertex of each slot
         self.render = None       # settings of view 0 (the first PILRenderer), or None
         self.views = []          # (observers key, render dict) of every PILRenderer, in observers order
+        self.masks = []          # (observers key, mask dict) of every SpriteMask, in observers order
         self.state_key = None    # observers key of the RawState observer, or None
         self.blob = b''
 
@@ -247,6 +249,10 @@ class Program(object):
             # has no table, and its blob is what it was before views existed)
             hdr[H_VIEWS] = self.add_ints(w for _, r in self.views[1:] for w in _view_words(r))
             hdr[H_N_VIEWS] = len(self.views) - 1
+        if self.masks:
+            # the mask table behind the view table (a program without a mask has none)
+            hdr[H_MASKS] = self.add_ints(w for _, m in self.masks for w in _view_words(m))
+            hdr[H_N_MASKS] = len(self.masks)
         ops = np.zeros(len(self.ops), dtype=OP_DTYPE)
         for k, o in enumerate(self.ops):
             ops[k]['kind'] = o['kind']
@@ -783,11 +789,16 @@ def _view_words(r):
 def _compile_render(prog, observers):
     prog.state_key = None
     prog.views = []
+    prog.masks = []
     for key, obs in (observers or {}).items():
         if _kind(obs) == 'PILRenderer':
             if len(prog.views) >= MAX_VIEWS:
                 raise CompileError('at most {} PILRenderer observers are supported'.format(MAX_VIEWS))
             prog.views.append((key, _lower_renderer(prog, obs)))
+        elif _kind(obs) == 'SpriteMask':
+            if len(prog.masks) >= MAX_VIEWS:
+                raise CompileError('at most {} SpriteMask observers are supported'.format(MAX_VIEWS))
+            prog.masks.append((key, _lower_mask(prog, obs)))
         elif _kind(obs) == 'RawState':
             if prog.state_key is not None:
                 raise CompileError('only one RawState observer is supported')
@@ -821,22 +832,35 @@ def _lower_renderer(prog, renderer):
             raise CompileError(
                 'color_to_rgb must be None or "hsv_to_rgb" on the device path')
         cmap = CMAP_NONE
-    pm = renderer._polygon_modifier
-    pk = _kind(pm)
-    modifier, mod_layer = PMOD_NONE, 0
-    if pk == 'FirstPersonAgent':
-        modifier, mod_layer = PMOD_FIRST_PERSON, prog.layer_index(
-            pm._agent_layer)
-    elif pk == 'TorusGeometry':
-        modifier = PMOD_TORUS
-    elif pk != 'DoNothing':
-        raise CompileError('unsupported polygon modifier {}'.format(pk))
+    modifier, mod_layer = _lower_modifier(prog, renderer._polygon_modifier)
     # pil_renderer.py:46,65-66: canvas = (aa*size[0], aa*size[1]) is handed to
     # PIL as (width, height) while the array that comes back is [height, width].
     return dict(height=int(size[1]), width=int(size[0]),
                 aa=int(renderer._anti_aliasing), bg=tuple(bg)[:3],
                 colormap=cmap, modifier=modifier,
                 modifier_layer=mod_layer)
+
+
+def _lower_modifier(prog, pm):
+    """(MOOG_PMOD_*, agent layer) of a polygon modifier."""
+    pk = _kind(pm)
+    if pk == 'FirstPersonAgent':
+        return PMOD_FIRST_PERSON, prog.layer_index(pm._agent_layer)
+    if pk == 'TorusGeometry':
+        return PMOD_TORUS, 0
+    if pk != 'DoNothing':
+        raise CompileError('unsupported polygon modifier {}'.format(pk))
+    return PMOD_NONE, 0
+
+
+def _lower_mask(prog, mask):
+    """A SpriteMask as a view row: anti_aliasing 1, no background, no colour map."""
+    size = tuple(mask._image_size)
+    if len(size) != 2:
+        raise CompileError('image_size must be (width, height)')
+    modifier, mod_layer = _lower_modifier(prog, mask._polygon_modifier)
+    return dict(height=int(size[1]), width=int(size[0]), aa=1, bg=(0, 0, 0), colormap=CMAP_NONE,
+                modifier=modifier, modifier_layer=mod_layer)
 
 
 # ---------------------------------------------------------------------------

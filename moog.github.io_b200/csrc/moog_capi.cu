@@ -28,6 +28,10 @@ struct moog_program {
   int *resample[MOOG_MAX_VIEWS];
   moog::RenderPlan plan[MOOG_MAX_VIEWS];  // how the render kernels draw each view (render_plan)
   int ksize_h[MOOG_MAX_VIEWS], ksize_v[MOOG_MAX_VIEWS];
+  // masks (one per SpriteMask): where their rows lie in the blob, and how the mask kernel draws them
+  int n_masks;
+  int mask_off[MOOG_MAX_VIEWS];
+  moog::RenderPlan mask_plan[MOOG_MAX_VIEWS];
   // largest outline a slot of each layer can hold (from the blob's voff table)
   int layer_vcap[MOOG_MAX_LAYERS];
   // cached vertex -> (slot << 8 | index within the slot's outline), [VT]: the Euler pass of the step
@@ -268,6 +272,35 @@ int moog_program_validate(const void *blob, size_t nbytes) {
       if (v[MOOG_V_MODIFIER] == MOOG_PMOD_FIRST_PERSON && !layer_ok(v[MOOG_V_MOD_LAYER])) return MOOG_E_INVAL;
     }
   }
+  // masks: rows of the mask table, with a renderer row's bounds and the words a mask fixes
+  const int nm = hdr[MOOG_H_N_MASKS], mt = hdr[MOOG_H_MASKS];
+  if (nm < 0 || nm > MOOG_MAX_VIEWS) return MOOG_E_INVAL;
+  if (nm > 0) {
+    if (mt < 0 || (long long)mt + (long long)MOOG_VIEW_WORDS * nm > NI) return MOOG_E_INVAL;
+    for (int k = 0; k < nm; ++k) {
+      const int32_t *m = pv.ipool + mt + MOOG_VIEW_WORDS * k;
+      if (m[MOOG_V_ENABLED] != 1 || m[MOOG_V_AA] != 1 || m[MOOG_V_BG] != 0 || m[MOOG_V_COLORMAP] != MOOG_CMAP_NONE ||
+          m[MOOG_V_HEIGHT] < 1 || m[MOOG_V_WIDTH] < 1 || m[MOOG_V_HEIGHT] > 8192 || m[MOOG_V_WIDTH] > 8192)
+        return MOOG_E_INVAL;
+      if (m[MOOG_V_MODIFIER] != MOOG_PMOD_NONE && m[MOOG_V_MODIFIER] != MOOG_PMOD_FIRST_PERSON &&
+          m[MOOG_V_MODIFIER] != MOOG_PMOD_TORUS)
+        return MOOG_E_INVAL;
+      if (m[MOOG_V_MODIFIER] == MOOG_PMOD_FIRST_PERSON && !layer_ok(m[MOOG_V_MOD_LAYER])) return MOOG_E_INVAL;
+    }
+  }
+  return 0;
+}
+
+int moog_mask_plan(const void *blob, size_t nbytes, int mask, int *band_rows, int *smem_bytes) {
+  const int bad = moog_program_validate(blob, nbytes);
+  if (bad) return bad;
+  const int32_t *hdr = (const int32_t *)blob;
+  if (mask < 0 || mask >= hdr[MOOG_H_N_MASKS]) return MOOG_E_INVAL;
+  const int32_t *m = moog::view_of(blob).ipool + hdr[MOOG_H_MASKS] + MOOG_VIEW_WORDS * mask;
+  const moog::RenderPlan plan = moog::render_plan(hdr, m);
+  if (!plan.ok) return MOOG_E_UNSUPPORTED;
+  if (band_rows) *band_rows = plan.rows;
+  if (smem_bytes) *smem_bytes = plan.env_bytes;
   return 0;
 }
 
@@ -310,6 +343,12 @@ int moog_program_create(const void *blob, size_t nbytes, moog_program **out) {
         p->view_off[k] = (int)(v - hdr);
         p->plan[k] = moog::render_plan(p->hdr, p->view[k]);
       }
+    }
+    p->n_masks = hdr[MOOG_H_N_MASKS];
+    for (int k = 0; k < p->n_masks; ++k) {
+      const int32_t *m = pv.ipool + hdr[MOOG_H_MASKS] + MOOG_VIEW_WORDS * k;
+      p->mask_off[k] = (int)(m - hdr);
+      p->mask_plan[k] = moog::render_plan(p->hdr, m);
     }
   }
   if (moog::env_smem_bytes(p->hdr) > 220 * 1024 || p->hdr[MOOG_H_CMASK_WORDS] > 2048) {
@@ -537,6 +576,23 @@ static int render_impl(moog_program *p, const moog_state *st, int n_envs, int vi
   }
   int launches = 0;
   cudaError_t err = moog::launch_render(a, p->plan[view], v, (cudaStream_t)stream, &launches, done, n_envs);
+  g_launches += launches;
+  return err == cudaSuccess ? 0 : cuda_fail(err);
+}
+
+int moog_render_mask(moog_program *p, const moog_state *st, int n_envs, int mask, int16_t *out, void *stream) {
+  if (!p || !valid_state(st) || !out || n_envs < 0 || ((uintptr_t)out & 15) || mask < 0 || mask >= p->n_masks)
+    return MOOG_E_INVAL;
+  if (!p->mask_plan[mask].ok) return MOOG_E_UNSUPPORTED;
+  moog::RenderArgs a;
+  memset(&a, 0, sizeof(a));
+  a.blob = p->dev_blob;
+  a.view_off = p->mask_off[mask];
+  a.st = *st;
+  a.n_envs = n_envs;
+  a.frames = (uint8_t *)out;
+  int launches = 0;
+  cudaError_t err = moog::launch_mask(a, p->mask_plan[mask], (cudaStream_t)stream, &launches);
   g_launches += launches;
   return err == cudaSuccess ? 0 : cuda_fail(err);
 }

@@ -122,6 +122,9 @@ RenderPlan render_plan(const int32_t *host_hdr, const int32_t *host_view);
 // words at a.view_off (the view's settings)
 cudaError_t launch_render(const RenderArgs &a, const RenderPlan &plan, const int32_t *host_view, cudaStream_t stream,
                           int *n_launches, int *done = nullptr, int n_done = 0);
+// moog_render_mask: a.view_off locates the mask row, a.frames is the int16 [n_envs][H][W] destination;
+// plan: render_plan of the mask row (anti_aliasing 1: its bands are an anti_aliasing 1 frame's)
+cudaError_t launch_mask(const RenderArgs &a, const RenderPlan &plan, cudaStream_t stream, int *n_launches);
 // moog_observe_sprites (moog_observe.cu): one warp per env
 cudaError_t launch_observe(const ObserveArgs &a, cudaStream_t stream, int *n_launches);
 // ints behind the finished list that launch_render's tail kernel uses: a ticket counter and the

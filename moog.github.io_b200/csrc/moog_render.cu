@@ -63,6 +63,23 @@ __global__ void moog_render_kernel(RenderArgs a, int T, int envs_per_block, int 
   draw_env<AA>(a, src, smem_raw + (size_t)g * env_bytes, t, T, P, live, a.frames + row * OH * OW * 3, rows, ring);
 }
 
+// SpriteMask: one env's mask per T threads, as moog_render_kernel<false> draws a frame (a.frames holds
+// the int16 masks)
+__global__ void moog_render_mask_kernel(RenderArgs a, int T, int envs_per_block, int P, int rows) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  ProgramView pv = view_of(a.blob);
+  const int32_t *mask = pv.hdr + a.view_off;
+  const int OH = mask[MOOG_V_HEIGHT], OW = mask[MOOG_V_WIDTH];
+  const int g = threadIdx.x / T, t = threadIdx.x - g * T;
+  const int n = blockIdx.x * envs_per_block + g;
+  const bool live = n < a.n_envs;
+  const size_t row = live ? (size_t)n : 0;
+  const RenderSrc src = env_src(a, pv, mask, row);
+  const RenderLayout lay = view_layout(pv.hdr, mask, rows, 0);
+  mask_env(src, lay, smem_raw + (size_t)g * lay.total, t, T, P, live, (int16_t *)a.frames + row * OH * OW,
+           [] { __syncthreads(); }, rows);
+}
+
 // The same for the envs of a step kernel that is still running (launched behind it with
 // programmatic stream serialization: this grid starts once every step CTA is resident or done, so
 // its CTAs land on the SMs the step has no more envs for).  A few CTAs per SM take tickets for the
@@ -253,23 +270,25 @@ static cudaError_t allow_smem(K kernel, size_t smem, size_t &configured) {
   return err;
 }
 
+// envs per CTA: the split that keeps the most envs resident per SM (228 KB of shared
+// memory, 1 KB of it reserved per CTA); ties go to the larger CTA
+static int envs_per_block(int T, size_t env_bytes) {
+  int epb = 1, best = 0;
+  for (int c = 1; c * T <= 256 || c == 1; ++c) {
+    const size_t per_cta = env_bytes * c + 1024;
+    if (per_cta > 228 * 1024) break;
+    const int envs = (int)(233472 / per_cta) * c;
+    if (envs >= best) { best = envs; epb = c; }
+  }
+  return epb;
+}
+
 template <bool AA>
 static cudaError_t launch_render_t(const RenderArgs &a, const RenderPlan &plan, cudaStream_t stream, int *n_launches,
                                    int *done, int n_done) {
   const int T = plan.T, P = plan.P, rows = plan.rows, ring = plan.ring;
   const size_t env_bytes = (size_t)plan.env_bytes;
-  // envs per CTA: the split that keeps the most envs resident per SM (228 KB of shared
-  // memory, 1 KB of it reserved per CTA); ties go to the larger CTA
-  int epb = 1;
-  {
-    int best = 0;
-    for (int c = 1; c * T <= 256 || c == 1; ++c) {
-      const size_t per_cta = env_bytes * c + 1024;
-      if (per_cta > 228 * 1024) break;
-      const int envs = (int)(233472 / per_cta) * c;
-      if (envs >= best) { best = envs; epb = c; }
-    }
-  }
+  const int epb = envs_per_block(T, env_bytes);
   size_t smem = env_bytes * epb;
   if (smem > 224 * 1024) return cudaErrorInvalidConfiguration;
   static size_t configured = 0;
@@ -319,6 +338,21 @@ cudaError_t launch_render(const RenderArgs &a, const RenderPlan &plan, const int
   if (!plan.ok) return cudaErrorInvalidConfiguration;  // render_impl refuses such a view before
   return view[MOOG_V_AA] > 1 ? launch_render_t<true>(a, plan, stream, n_launches, done, n_done)
                              : launch_render_t<false>(a, plan, stream, n_launches, done, n_done);
+}
+
+cudaError_t launch_mask(const RenderArgs &a, const RenderPlan &plan, cudaStream_t stream, int *n_launches) {
+  if (a.n_envs <= 0) return cudaSuccess;
+  if (!plan.ok) return cudaErrorInvalidConfiguration;  // mask_impl refuses such a mask before
+  const int epb = envs_per_block(plan.T, (size_t)plan.env_bytes);
+  const size_t smem = (size_t)plan.env_bytes * epb;
+  if (smem > 224 * 1024) return cudaErrorInvalidConfiguration;
+  static size_t configured = 0;
+  cudaError_t err = allow_smem(moog_render_mask_kernel, smem, configured);
+  if (err != cudaSuccess) return err;
+  const int blocks = (a.n_envs + epb - 1) / epb;
+  moog_render_mask_kernel<<<blocks, epb * plan.T, smem, stream>>>(a, plan.T, epb, plan.P, plan.rows);
+  if (n_launches) *n_launches += 1;
+  return cudaGetLastError();
 }
 
 }  // namespace moog

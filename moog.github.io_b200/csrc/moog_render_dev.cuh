@@ -115,6 +115,21 @@ struct BlendSink {
   }
 };
 
+// BlendSink's counterpart for a sprite mask: the covered pixels of the row take the sprite's slot
+struct SlotSink {
+  unsigned *row;
+  int W;
+  unsigned slot;
+  int xlo, xhi;
+  __device__ __forceinline__ void hline(int x0, int x1) {
+    if (x0 < 0) x0 = 0; else if (x0 >= W) return;   // hline32rgba's clipping
+    if (x1 < 0) return; else if (x1 >= W) x1 = W - 1;
+    x0 = max(x0, xlo);
+    x1 = min(x1, xhi);
+    for (int x = x0; x <= x1; ++x) row[x] = slot;
+  }
+};
+
 #define ITEM_SPANS 3          /* spans stored per item; more -> the item is redone directly */
 #define ITEM_OVERFLOW 0xffu
 struct SpanSink {
@@ -399,14 +414,18 @@ __device__ __forceinline__ void render_prepare(const RenderSrc &src, const Rende
 // render_draw_rows: the canvas rows [y0, y1) into the layout's canvas (its row 0 = canvas row y0):
 // background, (sprite, row) item spans, then P threads per row fill the sprites in z-order.
 // Returns after a barrier: the canvas rows are complete.
-template <class Sync>
+// SLOTS (the fill policy): false, the frames: the ink is blended into RGBX words over the view's
+// background.  true, a sprite mask: every pixel a sprite with a non-zero ink alpha covers takes its
+// slot, over a background of MASK_NONE; the scan conversion is the same.
+#define MASK_NONE 0xffffu /* int16 -1 */
+template <class Sync, bool SLOTS = false>
 __device__ __forceinline__ void render_draw_rows(const RenderSrc &src, const RenderLayout &lay, unsigned char *base,
                                                  unsigned *ext_items, int t, int T, int P, bool live, int y0, int y1,
                                                  Sync sync) {
   const int32_t *view = src.view;
   const int S = src.hdr[MOOG_H_N_SLOTS], VT = src.hdr[MOOG_H_N_VTX];
   const int aa = view[MOOG_V_AA], H = aa * view[MOOG_V_HEIGHT], W = aa * view[MOOG_V_WIDTH];
-  const unsigned bgc = (unsigned)view[MOOG_V_BG] & 0xffffffu;
+  const unsigned bgc = SLOTS ? MASK_NONE : (unsigned)view[MOOG_V_BG] & 0xffffffu;
   const int C = view[MOOG_V_MODIFIER] == MOOG_PMOD_TORUS ? 9 : 1;
   unsigned *canvas = (unsigned *)(base + lay.canvas);
   unsigned *ink = (unsigned *)(base + lay.ink);
@@ -495,6 +514,7 @@ __device__ __forceinline__ void render_draw_rows(const RenderSrc &src, const Ren
         if (y < ymin_c || y > ymax_c) continue;
         const int s0 = C == 1 ? s : s / C;
         const unsigned color = ink[s0];
+        if (SLOTS && (color >> 24) == 0u) continue;  // alpha 0: not in the frame, not in the mask
         const int b0 = sibase[s];
         unsigned cntw = ITEM_OVERFLOW;
         const unsigned *item = nullptr;
@@ -506,12 +526,22 @@ __device__ __forceinline__ void render_draw_rows(const RenderSrc &src, const Ren
           for (unsigned q = 0; q < cntw; ++q) {
             unsigned sp = item[1 + q];
             int x0 = max((int)(sp & 0xffffu), xlo), x1 = min((int)(sp >> 16), xhi);
-            if ((color >> 24) == 255u) {  // DIV255(fg * 255) == fg: opaque ink overwrites
+            if (SLOTS) {
+              for (int x = x0; x <= x1; ++x) row[x] = (unsigned)s0;
+            } else if ((color >> 24) == 255u) {  // DIV255(fg * 255) == fg: opaque ink overwrites
               for (int x = x0; x <= x1; ++x) row[x] = color & 0xffffffu;
             } else {
               for (int x = x0; x <= x1; ++x) row[x] = blend_px(row[x], color);
             }
           }
+        } else if (SLOTS) {
+          SlotSink sink;
+          sink.row = row;
+          sink.W = W;
+          sink.slot = (unsigned)s0;
+          sink.xlo = xlo;
+          sink.xhi = xhi;
+          polygon_row_rec(erec + (s - s0 * C) * VT + src.voff[s0], snedge[s], y, ymax_c, shoriz[s] != 0, sink);
         } else {
           BlendSink sink;
           sink.row = row;
@@ -584,6 +614,50 @@ __device__ __forceinline__ void render_env(const RenderSrc &src, const RenderLay
     render_draw_rows(src, lay, base, ext_items, t, T, P, live, y0, y1, sync);
     if (live) render_store_rows((const unsigned *)(base + lay.canvas), OW + 1, out, OH, OW, y0, y1, t, T);
     if (y0 + HB < H) sync();  // the next band reuses the canvas and the item spans
+  }
+}
+
+// render_store_rows for a mask: the low 16 bits of the canvas words [r1 - r0][img_stride] of the image
+// rows [r0, r1), flipped, into out ([OH][OW] int16).  16-byte stores when a row is a multiple of 16
+// bytes (OW % 8 == 0; `out` is then 16-byte aligned wherever an env starts), else one pixel per store.
+__device__ __forceinline__ void mask_store_rows(const unsigned *img, int img_stride, int16_t *out, int OH, int OW,
+                                                int r0, int r1, int t, int T) {
+  if ((OW & 7) == 0) {
+    uint4 *out4 = (uint4 *)out;
+    const int cpr = OW >> 3;
+    for (int q0 = t; q0 < (r1 - r0) * cpr; q0 += T) {
+      const int q = q0 + (OH - r1) * cpr;
+      const int j = q / cpr, c = q - j * cpr;
+      const unsigned *srcp = img + (OH - 1 - j - r0) * img_stride + 8 * c;
+      unsigned w[4];
+#pragma unroll
+      for (int i = 0; i < 4; ++i) w[i] = (srcp[2 * i] & 0xffffu) | (srcp[2 * i + 1] << 16);
+      out4[q] = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+  } else {
+    const int n = (r1 - r0) * OW;
+    for (int i0 = t; i0 < n; i0 += T) {
+      const int i = i0 + (OH - r1) * OW;
+      const int j = i / OW, col = i - j * OW;
+      out[i] = (int16_t)(img[(OH - 1 - j - r0) * img_stride + col] & 0xffffu);
+    }
+  }
+}
+
+// A SpriteMask of ONE env: render_env with the slot fill policy and the int16 store.  The mask row has
+// anti_aliasing 1, so `lay` and HB are those of an anti_aliasing 1 frame of the same size.
+template <class Sync>
+__device__ __forceinline__ void mask_env(const RenderSrc &src, const RenderLayout &lay, unsigned char *base, int t,
+                                         int T, int P, bool live, int16_t *out, Sync sync, int HB) {
+  const int OH = src.view[MOOG_V_HEIGHT], OW = src.view[MOOG_V_WIDTH];
+  if (HB <= 0 || HB > OH) HB = OH;
+  render_prepare(src, lay, base, t, T, live, sync);
+#pragma unroll 1
+  for (int y0 = 0; y0 < OH; y0 += HB) {
+    const int y1 = min(OH, y0 + HB);
+    render_draw_rows<Sync, true>(src, lay, base, nullptr, t, T, P, live, y0, y1, sync);
+    if (live) mask_store_rows((const unsigned *)(base + lay.canvas), OW + 1, out, OH, OW, y0, y1, t, T);
+    if (y0 + HB < OH) sync();
   }
 }
 

@@ -41,6 +41,9 @@ class VectorGymWrapper(object):
         spaces = {}
         for key, r in self._env.program.views:
             spaces[key] = dict(low=0, high=255, shape=(r['height'], r['width'], 3), dtype='uint8')
+        for key, m in self._env.program.masks:  # SpriteMask: a record slot per pixel, -1 for none
+            spaces[key] = dict(low=-1, high=self._env.program.n_slots - 1, shape=(m['height'], m['width']),
+                               dtype='int16')
         key = self._env.program.state_key
         if key is not None:
             spaces[key] = dict(low=-np.inf, high=np.inf, shape=(self._env.program.n_slots, compiler.OBS_COLS),

@@ -53,3 +53,32 @@ class RawState(AbstractObserver):
     column of an empty slot is 0).  `BatchedEnvironment.shape_names()` names the shape ids."""
 
     _observation_spec = None
+
+
+class SpriteMask(AbstractObserver):
+    """Which sprite each pixel shows.  The reference has no such observer; this one is an extension.
+
+    The batched environment returns under this key one int16 tensor [num_envs, H, W] for
+    `image_size=(W, H)` (PILRenderer's order).  For output pixel mask[n, j, x], let y = H - 1 - j
+    (the frames' np.flipud).  The value is the record slot s of the LAST sprite in draw order whose
+    polygon covers canvas pixel (x, y), or -1 where no sprite does.
+    - "Covers" means covered by the fill the frames use: Pillow's ImageDraw.Draw(canvas, 'RGBA')
+      .polygon (polygon_generic with deferred horizontal edges).  The vertices are the int-truncated
+      world vertices times the image size, after `polygon_modifier`.
+    - Draw order is slot order over the live slots (layer order, then list order).
+    - Only sprites whose ink alpha byte uint8(int64(opacity)) is non-zero count: a sprite with alpha
+      0 is invisible in the frames and absent from the mask.
+    - Every TorusGeometry copy of slot s writes s.
+    The slot is the RawState row, so state[n, mask[n, j, x]] is the sprite shown at that pixel.  A
+    mask is scan-converted at image_size: no anti-aliasing, no colours, no background."""
+
+    def __init__(self, image_size=(64, 64), polygon_modifier=None):
+        self._image_size = tuple(image_size)
+        if polygon_modifier is None:
+            polygon_modifier = polygon_modifiers.DoNothing()
+        self._polygon_modifier = polygon_modifier
+        self._observation_spec = None
+
+    @property
+    def polygon_modifier(self):
+        return self._polygon_modifier
