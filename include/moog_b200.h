@@ -170,6 +170,35 @@ int moog_mask_plan(const void *blob, size_t nbytes, int mask, int *band_rows, in
  * nothing. */
 int moog_observe_sprites(moog_program *p, const moog_state *st, int n_envs, float *out, void *stream);
 
+/* One RaySensor (no reference counterpart; moog/observers/pil_renderer.py RaySensor): n_rays rays from the
+ * position of slot layer_off[agent_layer] + agent_index.  Target slots: the live slots of the layers whose
+ * bit is set in `layers`, except the agent's own.  dirs is a DEVICE pointer to [n_rays][2] float64
+ * directions (cos phi_k, sin phi_k), computed by the host. */
+typedef struct {
+  int32_t agent_layer;
+  int32_t agent_index;
+  uint32_t layers;     /* bit l: layer l holds targets */
+  int32_t n_rays;      /* 1 .. 256 */
+  double max_range;    /* finite, > 0 */
+  const double *dirs;  /* [n_rays][2], 8-byte aligned */
+} moog_ray_spec;
+
+/* RaySensor readings of N envs: out[N][n_rays][2] float32.  For ray k with direction d from origin o, every
+ * edge (a, b) of a target slot's closed outline (its MOOG_M_NV cached world vertices, vertex j joined to
+ * vertex (j + 1) mod nv) is tested in float64, formulas as written: e = b - a, w = a - o, den = d x e,
+ * t = (w x e) / den, u = (w x d) / den, a hit when den != 0, 0 <= u <= 1 and t >= 0 (a x b = a.x b.y - a.y b.x).
+ * A slot whose outline holds o by the even-odd rule (edges with (a.y > o.y) != (b.y > o.y) and
+ * o.x < a.x + (o.y - a.y)(b.x - a.x) / (b.y - a.y)) reads t = 0.  The reading is (float(t / max_range), slot)
+ * for the smallest t <= max_range over the target slots, a tie going to the later slot, and (1, -1) when
+ * there is none or the agent layer holds no sprite at agent_index.  No wrapping under TorusGeometry.  A
+ * launch of its own on `stream`, like moog_observe_sprites: call it after moog_env_step.  `out` is any
+ * device-accessible address aligned to 16 bytes: HBM, or pinned host memory.  MOOG_E_INVAL for a NULL
+ * program / state / spec / dirs / out, n_envs < 0, n_rays outside [1, 256], a max_range that is not finite
+ * and > 0, an agent layer, an agent index < 0 or a target layer outside the program, a misaligned out or
+ * dirs; nothing is launched then, nor for n_envs == 0. */
+int moog_ray_sensor(moog_program *p, const moog_state *st, int n_envs, const moog_ray_spec *spec, float *out,
+                    void *stream);
+
 /* Host-side (CPU) polygon predicates for the HOST Sprite class only: the state
  * initializer's rejection sampling calls Sprite.overlaps_sprite /
  * contains_points (moog/state_initialization/sprite_generators.py:69-105,

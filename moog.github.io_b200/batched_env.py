@@ -14,6 +14,8 @@ num_envs=N)` works on an unchanged MOOG config -- and the same `reset()` /
                                                            include/moog_b200_program.h MOOG_OBS_*)
                 {key: int16 [N, H, W]}                    (SpriteMask: the slot each pixel shows,
                                                            -1 for none)
+                {key: float32 [N, R, 2]}                  (RaySensor: t / max_range and the slot
+                                                           each ray meets first, (1, -1) for none)
 
 An env whose previous step returned LAST is reset by the next `step()` call and
 ignores that call's action (environment.py:100-101).  Initial states come from
@@ -163,6 +165,16 @@ class Engine(object):
         # one int16 [N, H, W] buffer per SpriteMask, in mask order
         self.masks = [torch.full((self.n, m['height'], m['width']), -1, dtype=torch.int16, device=self.device)
                       for _, m in getattr(program, 'masks', ())]
+        # one float32 [N, R, 2] buffer per RaySensor, in sensor order, and the moog_ray_spec of each, whose
+        # direction table is uploaded once here
+        self.rays = []
+        self._ray_specs = []
+        for _, r in getattr(program, 'rays', ()):
+            self.rays.append(torch.empty((self.n, r['num_rays'], 2), **f32))
+            dirs = torch.from_numpy(r['dirs']).to(self.device, dtype=torch.float64).contiguous()
+            spec = capi.MoogRaySpec(r['agent_layer'], r['agent_index'], r['layers'], r['num_rays'],
+                                    r['max_range'], dirs.data_ptr())
+            self._ray_specs.append((spec, dirs))
         self.sprites = None
         if getattr(program, 'state_key', None) is not None:
             self.sprites = torch.zeros((self.n, program.n_slots, compiler.OBS_COLS), **f32)
@@ -363,6 +375,29 @@ class Engine(object):
                 self.dev_program.handle, ctypes.byref(st), count, mask, dst, self._stream()))
         return out
 
+    def sense_rays(self, out=None, first=0, count=None, sensor=0):
+        """RaySensor `sensor` of the envs [first, first + count) into out[first:first + count] (`out` None:
+        the sensor's own buffer in `rays`), cast by `moog_ray_sensor`: a contiguous float32 [N, R, 2]
+        tensor on this device or in pinned host memory, whose range starts 16-byte aligned."""
+        if not 0 <= sensor < len(self.rays):
+            raise ValueError('sensor {} is outside [0, {})'.format(sensor, len(self.rays)))
+        own = self.rays[sensor]
+        out = own if out is None else out
+        count = self.n - first if count is None else count
+        if first < 0 or count < 0 or first + count > self.n:
+            raise ValueError('env range [{}, {}) is outside [0, {})'.format(first, first + count, self.n))
+        if out.dtype != torch.float32 or tuple(out.shape) != tuple(own.shape) or not out.is_contiguous():
+            raise ValueError('rays of sensor {} must be a contiguous float32 tensor of shape {}'.format(
+                sensor, tuple(own.shape)))
+        self._check_reachable(out, 'rays')
+        st = self.state.struct(first)
+        dst = ctypes.c_void_p(out.data_ptr() + first * out.stride(0) * out.element_size())
+        with self._on_device():
+            capi.check(capi.lib().moog_ray_sensor(
+                self.dev_program.handle, ctypes.byref(st), count, ctypes.byref(self._ray_specs[sensor][0]), dst,
+                self._stream()))
+        return out
+
     def observe_sprites(self, out=None):
         """`moog_observe_sprites`: RawState (raw_state.py:17-19) of every env as float32 [N, S, 16]
         (columns: include/moog_b200_program.h MOOG_OBS_*), into `self.sprites` or `out` -- a
@@ -418,6 +453,7 @@ class BatchedEnvironment(object):
         self._image_key = self._image_keys[0] if self._image_keys else None
         self._state_key = self.program.state_key
         self._mask_keys = [k for k, _ in self.program.masks]   # SpriteMask observers in mask order
+        self._ray_keys = [k for k, _ in self.program.rays]     # RaySensor observers in sensor order
         self._rng = np.random.RandomState(seed)
         self._started = False
         self._copy_stream = None
@@ -484,11 +520,12 @@ class BatchedEnvironment(object):
         `host` is a TimeStep of CPU tensors (step_type int32[N], reward float32[N],
         discount float32[N] or None, observation {'image': uint8[N,H,W,3]} -- one such image per
         PILRenderer, under its key -- and, with a RawState observer, its key -> pinned
-        float32[N,S,16], and with SpriteMask observers, each key -> pinned int16[N,H,W]).  Returns `host`
-        once everything has arrived (the caller owns the TimeStep).  The other views, the masks and the
-        sprite observation travel like the frames of view 0:
+        float32[N,S,16], with SpriteMask observers, each key -> pinned int16[N,H,W], and with RaySensor
+        observers, each key -> pinned float32[N,R,2]).  Returns `host` once everything has arrived (the
+        caller owns the TimeStep).  The other views, the masks, the rays and the sprite observation travel
+        like the frames of view 0:
         stored by their kernels straight into the pinned tensors with 'mapped', computed in device
-        memory and copied after it otherwise (with 'chunked': range by range, a view or mask whose
+        memory and copied after it otherwise (with 'chunked': range by range, a view, mask or sensor whose
         per-env bytes are not a multiple of 16 in one range).
 
         frames = 'mapped': the step call draws every env's frame straight into the pinned host
@@ -504,6 +541,7 @@ class BatchedEnvironment(object):
         more = [host.observation[k] for k in self._image_keys[1:]]  # views 1..
         spr = host.observation.get(self._state_key) if self._state_key is not None else None
         masks = [host.observation[k] for k in self._mask_keys]
+        rays = [host.observation[k] for k in self._ray_keys]
         auto = frames == 'auto'
         if auto:
             frames = self._auto_frames(img)
@@ -523,6 +561,8 @@ class BatchedEnvironment(object):
                     spr.copy_(e.sprites, non_blocking=True)
                 for dst, src in zip(masks, e.masks):
                     dst.copy_(src, non_blocking=True)
+                for dst, src in zip(rays, e.rays):
+                    dst.copy_(src, non_blocking=True)
             else:
                 dst = None if img is None else (img if frames == 'mapped' else True)
                 e.env_step(self._flatten_action(action), sample_resets=(self.reset_mode == 'device'), frames=dst)
@@ -538,6 +578,11 @@ class BatchedEnvironment(object):
                         e.render_mask(out=dst, mask=m)
                     else:
                         dst.copy_(e.render_mask(mask=m), non_blocking=True)
+                for r, dst in enumerate(rays):
+                    if frames == 'mapped':
+                        e.sense_rays(out=dst, sensor=r)
+                    else:
+                        dst.copy_(e.sense_rays(sensor=r), non_blocking=True)
                 if spr is not None:
                     if frames == 'mapped':
                         e.observe_sprites(out=spr)
@@ -562,13 +607,14 @@ class BatchedEnvironment(object):
         host.reward.copy_(e.reward, non_blocking=True)
         if host.discount is not None:
             host.discount.copy_(e.discount, non_blocking=True)
-        if self._image_key is not None or masks:
+        if self._image_key is not None or masks or rays:
             dsts = [host.observation[k] for k in self._image_keys]
             # a range of a view other than 0 or of a mask must start 16-byte aligned (moog_render_view,
             # moog_render_mask): one whose per-env bytes are not a multiple of 16 is drawn and copied
             # whole with the first range
             ranged = [v == 0 or e.view_buffer(v)[0].numel() % 16 == 0 for v in range(len(dsts))]
             mranged = [e.masks[m][0].numel() * 2 % 16 == 0 for m in range(len(masks))]
+            rranged = [e.rays[r][0].numel() * 4 % 16 == 0 for r in range(len(rays))]
             chunks = max(1, min(int(chunks), len(self._copy_events), self.num_envs))
             # equal ranges: measured on B200 / PCIe 5 with 4096 64x64 frames, 4 equal ranges beat
             # 1, 2, 8 or 16 ranges and growing / shrinking ones (each render launch has a fixed
@@ -592,6 +638,12 @@ class BatchedEnvironment(object):
                     if span is not None:
                         e.render_mask(first=span[0], count=span[1] - span[0], mask=m)
                         mspans.append((m, span))
+                rspans = []
+                for r in range(len(rays)):
+                    span = (first, first + count) if rranged[r] else ((0, self.num_envs) if c == 0 else None)
+                    if span is not None:
+                        e.sense_rays(first=span[0], count=span[1] - span[0], sensor=r)
+                        rspans.append((r, span))
                 ev = self._copy_events[c]
                 ev.record(main)
                 copy.wait_event(ev)
@@ -600,6 +652,8 @@ class BatchedEnvironment(object):
                         dsts[v][a:b].copy_(e.view_buffer(v)[a:b], non_blocking=True)
                     for m, (a, b) in mspans:
                         masks[m][a:b].copy_(e.masks[m][a:b], non_blocking=True)
+                    for r, (a, b) in rspans:
+                        rays[r][a:b].copy_(e.rays[r][a:b], non_blocking=True)
                 first += count
         copy.synchronize()
         main.synchronize()
@@ -641,6 +695,8 @@ class BatchedEnvironment(object):
             obs[key] = self.engine.render(view=v)
         for m, key in enumerate(self._mask_keys):
             obs[key] = self.engine.render_mask(mask=m)
+        for r, key in enumerate(self._ray_keys):
+            obs[key] = self.engine.sense_rays(sensor=r)
         if self._state_key is not None:
             obs[self._state_key] = self.engine.observe_sprites()
         return obs
@@ -654,6 +710,8 @@ class BatchedEnvironment(object):
                 obs[key] = e.render(view=v)
             for m, key in enumerate(self._mask_keys):
                 obs[key] = e.render_mask(mask=m)
+            for r, key in enumerate(self._ray_keys):
+                obs[key] = e.sense_rays(sensor=r)
             if self._state_key is not None:
                 obs[self._state_key] = e.observe_sprites()
         else:
@@ -737,8 +795,9 @@ class HostPipeline(object):
     i.e. the policy acts on an observation that is one step old (the usual actor pipeline); with
     depth 1 it is `step_to_host`.  Every submit copies that step's actions host -> device and
     every collect returns step_type / reward / discount / frames of every PILRenderer (and the
-    RawState observation and the SpriteMasks when the config has them) in pinned host memory, valid
-    until `depth` further submits.  frames = 'mapped': the kernels store the frames, masks and sprite observation
+    RawState observation, the SpriteMasks and the RaySensors when the config has them) in pinned host
+    memory, valid until `depth` further submits.  frames = 'mapped': the kernels store the frames, masks,
+    rays and sprite observation
     straight into the slot's pinned buffers over PCIe; 'device': they are written to HBM and copied
     by a copy engine on a second stream while the next step runs.
     Reference protocol: moog/environment.py:98-126 (one `step` per submit, auto-reset included).
@@ -769,10 +828,15 @@ class HostPipeline(object):
             for m, key in enumerate(env._mask_keys):  # pylint: disable=protected-access
                 masks.append(pin(*e.masks[m].shape, dtype=torch.int16))
                 obs[key] = masks[-1]
+            rays = []  # one pinned reading per RaySensor, in sensor order
+            for r, key in enumerate(env._ray_keys):  # pylint: disable=protected-access
+                rays.append(pin(*e.rays[r].shape, dtype=torch.float32))
+                obs[key] = rays[-1]
             self._slots.append(dict(
                 ts=TimeStep(pin(n, dtype=torch.int32), pin(n, dtype=torch.float32), pin(n, dtype=torch.float32), obs),
-                imgs=imgs, spr=spr, masks=masks,
+                imgs=imgs, spr=spr, masks=masks, rays=rays,
                 dev_masks=[torch.empty_like(d) for d in e.masks] if frames == 'device' else None,
+                dev_rays=[torch.empty_like(d) for d in e.rays] if frames == 'device' else None,
                 dev_imgs=[torch.empty_like(e.view_buffer(v)) for v in range(len(imgs))] if frames == 'device' else None,
                 dev_sprites=(torch.empty_like(e.sprites) if (spr is not None and frames == 'device') else None),
                 host_act=pin(n, ad, dtype=torch.float64),
@@ -798,6 +862,8 @@ class HostPipeline(object):
                     slot['spr'].copy_(e.sprites, non_blocking=True)
                 for host_mask, dev in zip(slot['masks'], e.masks):
                     host_mask.copy_(dev, non_blocking=True)
+                for host_rays, dev in zip(slot['rays'], e.rays):
+                    host_rays.copy_(dev, non_blocking=True)
             else:
                 act = None
                 if action is not None:
@@ -815,13 +881,16 @@ class HostPipeline(object):
                     e.render(out=dsts[v], view=v)
                 for m, dst in enumerate(slot['masks'] if self.frames == 'mapped' else slot['dev_masks']):
                     e.render_mask(out=dst, mask=m)
+                for r, dst in enumerate(slot['rays'] if self.frames == 'mapped' else slot['dev_rays']):
+                    e.sense_rays(out=dst, sensor=r)
                 if slot['spr'] is not None:
                     e.observe_sprites(out=slot['spr'] if self.frames == 'mapped' else slot['dev_sprites'])
             ts = slot['ts']
             ts.step_type.copy_(e.step_type, non_blocking=True)
             ts.reward.copy_(e.reward, non_blocking=True)
             ts.discount.copy_(e.discount, non_blocking=True)
-            if self.frames == 'device' and (slot['imgs'] or slot['masks'] or slot['spr'] is not None) and not was_reset:
+            if self.frames == 'device' and (slot['imgs'] or slot['masks'] or slot['rays'] or slot['spr'] is not None) \
+                    and not was_reset:
                 slot['stepped'].record(self._main)
                 self._copy.wait_event(slot['stepped'])
                 with torch.cuda.stream(self._copy):
@@ -829,6 +898,8 @@ class HostPipeline(object):
                         img.copy_(dev, non_blocking=True)
                     for host_mask, dev in zip(slot['masks'], slot['dev_masks']):
                         host_mask.copy_(dev, non_blocking=True)
+                    for host_rays, dev in zip(slot['rays'], slot['dev_rays']):
+                        host_rays.copy_(dev, non_blocking=True)
                     if slot['spr'] is not None:
                         slot['spr'].copy_(slot['dev_sprites'], non_blocking=True)
                     slot['done'].record(self._copy)

@@ -14,7 +14,7 @@ import sys
 _PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_PKG, 'csrc')
 LIB = os.environ.get('MOOG_B200_LIB') or os.path.join(_PKG, 'lib', 'libmoog_b200.so')   # override: A/B runs
-SOURCES = ['moog_step.cu', 'moog_render.cu', 'moog_observe.cu', 'moog_capi.cu', 'moog_host_geom.cpp']
+SOURCES = ['moog_step.cu', 'moog_render.cu', 'moog_observe.cu', 'moog_rays.cu', 'moog_capi.cu', 'moog_host_geom.cpp']
 HEADERS = [os.path.join(CSRC, 'moog_common.cuh'), os.path.join(CSRC, 'moog_render_dev.cuh'),
            os.path.join(CSRC, 'moog_dcv_argmin.cuh'), os.path.join(CSRC, 'moog_seg_cross.cuh'),
            os.path.join(_PKG, '..', 'include', 'moog_b200.h'),

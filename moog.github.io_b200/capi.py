@@ -33,6 +33,13 @@ class MoogStepIO(ctypes.Structure):
                 ('frames', ctypes.c_void_p)]
 
 
+class MoogRaySpec(ctypes.Structure):
+    """`moog_ray_spec`."""
+    _fields_ = [('agent_layer', ctypes.c_int32), ('agent_index', ctypes.c_int32),
+                ('layers', ctypes.c_uint32), ('n_rays', ctypes.c_int32),
+                ('max_range', ctypes.c_double), ('dirs', ctypes.c_void_p)]
+
+
 # every symbol include/moog_b200.h declares
 SYMBOLS = ('moog_program_create', 'moog_program_destroy',
            'moog_program_env_smem_bytes', 'moog_env_step',
@@ -42,7 +49,7 @@ SYMBOLS = ('moog_program_create', 'moog_program_destroy',
            'moog_host_points_in_path', 'moog_step_launch_info',
            'moog_step_draws_frames', 'moog_program_set_option',
            'moog_program_validate', 'moog_observe_sprites', 'moog_render_view',
-           'moog_render_plan', 'moog_render_mask', 'moog_mask_plan')
+           'moog_render_plan', 'moog_render_mask', 'moog_mask_plan', 'moog_ray_sensor')
 
 
 # include/moog_b200.h return codes
@@ -116,6 +123,8 @@ def lib():
     L.moog_render_mask.restype = ci
     L.moog_mask_plan.argtypes = [vp, ctypes.c_size_t, ci, ctypes.POINTER(ci), ctypes.POINTER(ci)]
     L.moog_mask_plan.restype = ci
+    L.moog_ray_sensor.argtypes = [vp, ctypes.POINTER(MoogState), ci, ctypes.POINTER(MoogRaySpec), vp, vp]
+    L.moog_ray_sensor.restype = ci
     L.moog_launch_count.argtypes = []
     L.moog_launch_count.restype = ctypes.c_int64
     _lib = L

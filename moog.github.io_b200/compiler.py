@@ -61,6 +61,8 @@ H_MASKS, H_N_MASKS = 62, 63
 VIEW_WORDS = 8           # MOOG_VIEW_WORDS: a view table row, the words H_R_HEIGHT .. H_R_ENABLED
 MAX_VIEWS = 8            # MOOG_MAX_VIEWS: PILRenderer observers per program, and SpriteMask observers
 MAX_META_VARS = 16
+MAX_RAY_SENSORS = 8      # RaySensor observers per program
+MAX_RAYS = 256           # rays per RaySensor (include/moog_b200.h moog_ray_spec)
 
 F_DRAG, F_KINETIC_FRICTION, F_DOWN_GRAVITY, F_GRAVITY, F_RANDOM, \
     F_DIST_LINEAR, F_DIST_SPRING, F_COLLISION, F_MAZE_WALK = range(1, 10)
@@ -154,6 +156,7 @@ class Program(object):
         self.render = None       # settings of view 0 (the first PILRenderer), or None
         self.views = []          # (observers key, render dict) of every PILRenderer, in observers order
         self.masks = []          # (observers key, mask dict) of every SpriteMask, in observers order
+        self.rays = []           # (observers key, ray dict) of every RaySensor, in observers order (not in the blob)
         self.state_key = None    # observers key of the RawState observer, or None
         self.blob = b''
 
@@ -790,6 +793,7 @@ def _compile_render(prog, observers):
     prog.state_key = None
     prog.views = []
     prog.masks = []
+    prog.rays = []
     for key, obs in (observers or {}).items():
         if _kind(obs) == 'PILRenderer':
             if len(prog.views) >= MAX_VIEWS:
@@ -799,6 +803,11 @@ def _compile_render(prog, observers):
             if len(prog.masks) >= MAX_VIEWS:
                 raise CompileError('at most {} SpriteMask observers are supported'.format(MAX_VIEWS))
             prog.masks.append((key, _lower_mask(prog, obs)))
+        elif _kind(obs) == 'RaySensor':
+            if len(prog.rays) >= MAX_RAY_SENSORS:
+                raise CompileError('observer {!r}: at most {} RaySensor observers are supported'.format(
+                    key, MAX_RAY_SENSORS))
+            prog.rays.append((key, _lower_rays(prog, key, obs)))
         elif _kind(obs) == 'RawState':
             if prog.state_key is not None:
                 raise CompileError('only one RawState observer is supported')
@@ -861,6 +870,34 @@ def _lower_mask(prog, mask):
     modifier, mod_layer = _lower_modifier(prog, mask._polygon_modifier)
     return dict(height=int(size[1]), width=int(size[0]), aa=1, bg=(0, 0, 0), colormap=CMAP_NONE,
                 modifier=modifier, modifier_layer=mod_layer)
+
+
+def _lower_rays(prog, key, sensor):
+    """A RaySensor as the fields of include/moog_b200.h moog_ray_spec, its direction table included."""
+    def bad(what):
+        return CompileError('observer {!r}: RaySensor {}'.format(key, what))
+    names = [sensor._agent_layer] + list(prog.layer_names if sensor._layers is None else sensor._layers)
+    for name in names:
+        if name not in prog.layer_names:
+            raise bad('names layer {!r}, which is not in the environment state (layers: {})'.format(
+                name, prog.layer_names))
+    R = sensor._num_rays
+    if isinstance(R, bool) or not isinstance(R, (int, np.integer)) or not 1 <= R <= MAX_RAYS:
+        raise bad('num_rays must be an integer in [1, {}], not {!r}'.format(MAX_RAYS, R))
+    max_range, fov = float(sensor._max_range), float(sensor._fov)
+    if not (np.isfinite(max_range) and max_range > 0):
+        raise bad('max_range must be finite and > 0, not {!r}'.format(sensor._max_range))
+    if not 0 < fov <= 2 * np.pi:
+        raise bad('fov must be in (0, 2 pi], not {!r}'.format(sensor._fov))
+    index = sensor._agent_index
+    if isinstance(index, bool) or not isinstance(index, (int, np.integer)) or index < 0:
+        raise bad('agent_index must be an integer >= 0, not {!r}'.format(index))
+    layers = 0
+    for name in names[1:]:
+        layers |= 1 << prog.layer_index(name)
+    return dict(agent_layer=prog.layer_index(names[0]), agent_index=int(index), layers=layers,
+                num_rays=int(R), max_range=max_range,
+                dirs=np.ascontiguousarray(sensor.directions(), dtype=np.float64))
 
 
 # ---------------------------------------------------------------------------

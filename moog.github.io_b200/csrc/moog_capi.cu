@@ -614,6 +614,39 @@ int moog_observe_sprites(moog_program *p, const moog_state *st, int n_envs, floa
   return err == cudaSuccess ? 0 : cuda_fail(err);
 }
 
+int moog_ray_sensor(moog_program *p, const moog_state *st, int n_envs, const moog_ray_spec *spec, float *out,
+                    void *stream) {
+  if (!p || !valid_state(st) || !spec || !spec->dirs || !out || n_envs < 0 || ((uintptr_t)out & 15) ||
+      ((uintptr_t)spec->dirs & 7))
+    return MOOG_E_INVAL;
+  const int L = p->hdr[MOOG_H_N_LAYERS];
+  if (spec->n_rays < 1 || spec->n_rays > 256 || !isfinite(spec->max_range) || !(spec->max_range > 0.0) ||
+      spec->agent_layer < 0 || spec->agent_layer >= L || spec->agent_index < 0 ||
+      (L < 32 && (spec->layers >> L) != 0))
+    return MOOG_E_INVAL;
+  if (n_envs == 0) return 0;
+  moog::RayArgs a;
+  memset(&a, 0, sizeof(a));
+  a.blob = p->dev_blob;
+  a.st = *st;
+  a.out = out;
+  a.dirs = spec->dirs;
+  a.max_range = spec->max_range;
+  a.n_envs = n_envs;
+  a.S = p->hdr[MOOG_H_N_SLOTS];
+  a.L = L;
+  a.VT = p->hdr[MOOG_H_N_VTX];
+  a.n_rays = spec->n_rays;
+  a.agent_layer = spec->agent_layer;
+  a.agent_index = spec->agent_index;
+  a.layers = spec->layers;
+  memcpy(a.layer_off, &p->hdr[MOOG_H_LAYER_OFF], sizeof(a.layer_off));
+  int launches = 0;
+  cudaError_t err = moog::launch_ray_sensor(a, (cudaStream_t)stream, &launches);
+  g_launches += launches;
+  return err == cudaSuccess ? 0 : cuda_fail(err);
+}
+
 const char *moog_strerror(int code) {
   switch (code) {
     case 0: return "ok";

@@ -75,6 +75,18 @@ struct ObserveArgs {
   int layer_off[MOOG_MAX_LAYERS + 1];
 };
 
+struct RayArgs {
+  const void *blob;     // device copy of the program (its voff table)
+  moog_state st;
+  float *out;           // [n_envs][n_rays][2]
+  const double *dirs;   // [n_rays][2]
+  double max_range;
+  int n_envs, S, L, VT, n_rays;
+  int agent_layer, agent_index;
+  unsigned layers;      // bit l: layer l holds targets
+  int layer_off[MOOG_MAX_LAYERS + 1];
+};
+
 // Launch options of one program (moog_program_set_option / the MOOG_* environment variables, which
 // are read ONCE, when the program is created).  -1 / 0 = decided by the library.
 struct LaunchOptions {
@@ -127,6 +139,8 @@ cudaError_t launch_render(const RenderArgs &a, const RenderPlan &plan, const int
 cudaError_t launch_mask(const RenderArgs &a, const RenderPlan &plan, cudaStream_t stream, int *n_launches);
 // moog_observe_sprites (moog_observe.cu): one warp per env
 cudaError_t launch_observe(const ObserveArgs &a, cudaStream_t stream, int *n_launches);
+// moog_ray_sensor (moog_rays.cu): one CTA per env, one thread per ray
+cudaError_t launch_ray_sensor(const RayArgs &a, cudaStream_t stream, int *n_launches);
 // ints behind the finished list that launch_render's tail kernel uses: a ticket counter and the
 // per-SM count of envs being stepped
 constexpr int kTailExtraInts = 1 + 256;

@@ -44,6 +44,9 @@ class VectorGymWrapper(object):
         for key, m in self._env.program.masks:  # SpriteMask: a record slot per pixel, -1 for none
             spaces[key] = dict(low=-1, high=self._env.program.n_slots - 1, shape=(m['height'], m['width']),
                                dtype='int16')
+        for key, r in self._env.program.rays:  # RaySensor: (t / max_range, slot) per ray, (1, -1) for none
+            spaces[key] = dict(low=-1, high=max(1, self._env.program.n_slots - 1), shape=(r['num_rays'], 2),
+                               dtype='float32')
         key = self._env.program.state_key
         if key is not None:
             spaces[key] = dict(low=-np.inf, high=np.inf, shape=(self._env.program.n_slots, compiler.OBS_COLS),

@@ -6,6 +6,7 @@ is not used on this path.
 """
 
 import abc
+import math
 
 from . import color_maps
 from . import polygon_modifiers
@@ -82,3 +83,47 @@ class SpriteMask(AbstractObserver):
     @property
     def polygon_modifier(self):
         return self._polygon_modifier
+
+
+class RaySensor(AbstractObserver):
+    """Range finder: rays from an agent sprite to the first outline they cross.  The reference has no such
+    observer; this one is an extension.
+
+    The batched environment returns under this key one float32 tensor [num_envs, num_rays, 2].
+    - Origin o: the position (x, y) of sprite `agent_index` of layer `agent_layer`.  When that layer holds
+      fewer live sprites, every ray reads "no hit".
+    - Ray k points along phi_k = direction - fov / 2 + fov * (k + 0.5) / num_rays, counter-clockwise from +x
+      in the world frame: the rays do not turn with the agent (FirstPersonAgent only translates either).
+      The host computes d_k = (np.cos(phi_k), np.sin(phi_k)) once, in float64 (`directions()`); the device
+      evaluates no trigonometric function.
+    - Targets: every live sprite of `layers` (None: all layers) except the agent itself, whatever its
+      opacity.  A sprite's outline is the closed polygon through its cached world vertices; vertex j is
+      joined to vertex (j + 1) mod nv, and a degenerate edge never hits.
+    - Hit distance, float64, evaluated as written (a x b = a.x * b.y - a.y * b.x): for an edge (a, b),
+      e = b - a, w = a - o, den = d x e; when den != 0, t = (w x e) / den and u = (w x d) / den, and the
+      edge is hit when 0 <= u <= 1 and t >= 0.  A sprite's t is its smallest edge t, or 0 when o lies
+      inside its outline by the even-odd rule (edges with (a.y > o.y) != (b.y > o.y) and
+      o.x < a.x + (o.y - a.y) * (b.x - a.x) / (b.y - a.y)).
+    - Reading of ray k: the smallest t over the targets, a tie going to the later sprite in draw order.
+      When t <= max_range it is (float32(t / max_range), float32(slot)), the slot being the RawState row
+      (`program.layer_off` maps it to its layer); otherwise (1.0, -1.0).
+    Rays do not wrap under TorusGeometry.  Limits: 1 <= num_rays <= 256, a finite max_range > 0,
+    0 < fov <= 2 pi, at most 8 RaySensors per config."""
+
+    def __init__(self, agent_layer, num_rays=32, max_range=0.5, fov=2 * math.pi, direction=math.pi / 2,
+                 layers=None, agent_index=0):
+        self._agent_layer = agent_layer
+        self._num_rays = num_rays
+        self._max_range = max_range
+        self._fov = fov
+        self._direction = direction
+        self._layers = None if layers is None else list(layers)
+        self._agent_index = agent_index
+        self._observation_spec = None
+
+    def directions(self):
+        """[num_rays, 2] float64: (cos phi_k, sin phi_k) of every ray."""
+        import numpy as np
+        k = np.arange(int(self._num_rays), dtype=np.float64)
+        phi = self._direction - self._fov / 2 + self._fov * (k + 0.5) / self._num_rays
+        return np.stack([np.cos(phi), np.sin(phi)], axis=1)
